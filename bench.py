@@ -22,6 +22,7 @@ with one NCCL all-gather + N-1 point additions.  The one JSON line also carries
     python bench.py --gpus 1 --steps 10 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference        # CPU port of the reference path, same metric
+    python bench.py --dump-outputs DIR      # also write the last timed step's outputs to DIR/*.npy
 
 `--workload encode | hash | fixed_base | pipeline | decompress | compress` times one of the
 other configs alone with the same harness.
@@ -118,7 +119,39 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config block of the MSM line")
     ap.add_argument("--no-single-process", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed call returned in its last step to DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm; --impl reference has none")
+    return a
+
+
+DUMP_BUDGET = 64_000_000     # bytes written by --dump-outputs, .npy headers included
+
+
+def dump_outputs(path: str, outputs: dict) -> None:
+    """Write every output of the last timed step as <path>/<name>.npy in float32 (every value
+    is a byte, so the conversion is exact).  When the outputs together would exceed 64 MB,
+    all of them keep the same rows, a sample drawn with a fixed seed, and rows.npy (float64)
+    lists the row indices kept.  `outputs` maps names to torch tensors on any device."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    total = sum(4 * t.numel() for t in outputs.values())
+    if total > DUMP_BUDGET - (1 << 16):          # room for the .npy headers
+        n = {t.shape[0] for t in outputs.values()}
+        assert len(n) == 1, "sampled outputs must share their first dimension"
+        n = n.pop()
+        row_bytes = sum(4 * t[0].numel() for t in outputs.values()) + 8
+        m = (DUMP_BUDGET - (1 << 16)) // row_bytes
+        rows = np.sort(np.random.default_rng(377).choice(n, m, replace=False))
+        np.save(os.path.join(path, "rows.npy"), rows.astype(np.float64))
+        outputs = {k: t[torch.from_numpy(rows).to(t.device)] for k, t in outputs.items()}
+    for k, t in outputs.items():
+        np.save(os.path.join(path, k + ".npy"), t.cpu().numpy().astype(np.float32))
 
 
 # ---------------------------------------------------------------------------
@@ -522,9 +555,9 @@ def bench_msm(cx: Ctx, logn: int, steps: int, warmup: int, e2e: bool, extras: bo
         cnt[0] += 1
         if world == 1:
             dev.msm_async(sc, pts, d.PT_ELEMENT, out_element=oe[i], out_encoding=oc[i], inputs_ready=True)
-            last[0] = oc[i]
+            last[0] = (oe[i], oc[i])
         else:
-            last[0] = ddist.msm_sharded_async(sc, pts, d.PT_ELEMENT, inputs_ready=True)[1]
+            last[0] = ddist.msm_sharded_async(sc, pts, d.PT_ELEMENT, inputs_ready=True)
 
     sampler = ClockSampler(cx.local_rank)
     if rank == 0:
@@ -532,11 +565,14 @@ def bench_msm(cx: Ctx, logn: int, steps: int, warmup: int, e2e: bool, extras: bo
     ms_step, launches = cx.time_device(step_dev, steps, warmup)
     clocks = sampler.stop() if rank == 0 else None
     value = world * n / (ms_step * 1e-3) / 1e6
-    got = bytes(last[0].cpu().numpy().tobytes())
+    got = bytes(last[0][1].cpu().numpy().tobytes())
     verified = got == want
     out = {"value": value, "unit": "Mpoints/s", "ms_per_step": ms_step, "gpu_launches": launches,
            "clocks": clocks, "verified_known_answer": verified, "h2d": n * (32 + 128), "d2h": 160,
-           "steps": steps, "l2": "inputs (%.0f MiB per GPU) exceed the 126 MB L2" % (n * 160 / 2**20)}
+           "steps": steps, "l2": "inputs (%.0f MiB per GPU) exceed the 126 MB L2" % (n * 160 / 2**20),
+           # the projective (X : Y : Z : T) of the sum depends on the order in which the counting
+           # sort's atomic slot claims put each bucket's points; its affine (x, y) does not
+           "outputs": {"element_xy": dev.normalize(last[0][0].reshape(1, 128))[0], "encoding": last[0][1]}}
     imad_peak = d.imad_peak()
     peaks = measured_peaks()
     out["roofline"], out["roofline_hbm"], out["stages"] = msm_roofline(cx, n, logn, ms_step, imad_peak, peaks)
@@ -795,18 +831,25 @@ def bench_elementwise(cx: Ctx, wl: str, logn: int, steps: int, warmup: int, e2e:
         make_out = lambda: (d.pinned_empty((n, 32)), d.pinned_empty((n,)))
         step_e2e = lambda h, o: d.batch_scalar_mul(h[0], h[1], d.PT_ENCODING, d.OUT_ENCODING,
                                                    return_ok=True, out=o[0], ok=o[1])
+    last = [None]
+
+    def step_last():
+        last[0] = step_dev()
+
     # inputs + outputs below the 126 MB L2: flush it between the timed iterations
     small = (h2d + d2h) < (126 << 20)
     sampler = ClockSampler(cx.local_rank)
     if cx.rank == 0:
         sampler.start()
-    ms_step, launches = cx.time_device(step_dev, steps, warmup, flush_l2=small)
+    ms_step, launches = cx.time_device(step_last, steps, warmup, flush_l2=small)
     clocks = sampler.stop() if cx.rank == 0 else None
     unit = "Melem/s"
     out = {"value": cx.world * n / (ms_step * 1e-3) / 1e6, "unit": unit, "ms_per_step": ms_step,
            "gpu_launches": launches, "h2d": h2d, "d2h": d2h, "units": n, "clocks": clocks, "steps": steps,
            "l2": ("flushed between timed iterations (256 MiB write outside the event pairs)" if small else
-                  "inputs + outputs (%.0f MiB) exceed the 126 MB L2" % ((h2d + d2h) / 2**20))}
+                  "inputs + outputs (%.0f MiB) exceed the 126 MB L2" % ((h2d + d2h) / 2**20)),
+           "outputs": (dict(zip(("elements", "ok"), last[0])) if wl == "decompress"
+                       else {"encodings": last[0]})}
     imad_peak = d.imad_peak()
     peaks = measured_peaks()
     ach = n * OPS_OF[wl] * IMAD_PER_FQ_OP / (ms_step * 1e-3) / 1e9
@@ -901,6 +944,9 @@ def main_ours(args):
         res = bench_msm(cx, logn, steps, warmup, not args.no_e2e, extras=True)
     else:
         res = bench_elementwise(cx, wl, logn, steps, warmup, not args.no_e2e)
+    outputs = res.pop("outputs")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
     cpu = None
     if want_cpu:
         cpu = cpu_baseline_of(wl, args.ref_logn or CPU_SAMPLE_LOGN[wl], 3)
@@ -918,6 +964,7 @@ def main_ours(args):
             c = cpu_baseline_of(w, CPU_SAMPLE_LOGN[w]) if want_cpu else None
             configs[name] = config_entry(r, c)
             configs[name]["workload"] = WORKLOAD_NAME[w].format(logn=ln)
+            del r
             cx.torch.cuda.empty_cache()
         r = bench_msm(cx, 20, max(10, csteps), 3, not args.no_e2e, extras=False)
         c = cpu_baseline_of("msm", 20) if want_cpu else None

@@ -1,5 +1,5 @@
 """CPU-side checks of bench.py's host logic: the known-answer arithmetic that verifies the
-timed MSMs, the reference arm's JSON line and its step / budget handling."""
+timed MSMs, the reference arm's JSON line and its step / budget handling, the output dump."""
 import json
 import os
 import random
@@ -58,3 +58,34 @@ def test_reference_arm_line_and_budget():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--logn", "10"],
                        capture_output=True, text=True, timeout=600, cwd=ROOT, env=dict(os.environ, RANK="1"))
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_steps_below_one_are_refused():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                       capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
+def test_dump_outputs_float32_and_seeded_row_sample(tmp_path):
+    small = {"element_xy": torch.arange(64, dtype=torch.uint8), "encoding": torch.arange(32, dtype=torch.uint8)}
+    bench.dump_outputs(str(tmp_path / "small"), small)
+    for name, t in small.items():
+        got = np.load(tmp_path / "small" / (name + ".npy"))
+        assert got.dtype == np.float32 and np.array_equal(got, t.numpy())
+    assert not (tmp_path / "small" / "rows.npy").exists()
+    # larger than the budget: every output keeps the same seeded sample of rows
+    n = 600000
+    g = torch.Generator().manual_seed(1)
+    big = {"elements": torch.randint(0, 256, (n, 128), dtype=torch.uint8, generator=g),
+           "ok": torch.randint(0, 2, (n,), dtype=torch.uint8, generator=g)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), big)
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= bench.DUMP_BUDGET
+    rows = np.load(tmp_path / "a" / "rows.npy")
+    assert rows.dtype == np.float64 and 0 < len(rows) < n and np.all(np.diff(rows) > 0)
+    rows = rows.astype(np.int64)
+    for name, t in big.items():
+        got = np.load(tmp_path / "a" / (name + ".npy"))
+        assert got.dtype == np.float32 and np.array_equal(got, t.numpy()[rows])
+    for f in ("rows.npy", "elements.npy", "ok.npy"):
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f))
