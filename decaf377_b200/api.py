@@ -165,14 +165,16 @@ MSM_STAGES = ("points", "count", "scan", "scatter", "accumulate", "stitch", "buc
 
 
 def msm_stage_info() -> dict:
-    """Per-stage device times (ms) and geometry of the most recent MSM."""
+    """Per-stage device times (ms) and geometry of the most recent MSM ("windowed": it ran
+    over a windowed MsmBases set; c and W are then the set's)."""
     ms = (C.c_float * 8)()
     c, w, n = C.c_int(0), C.c_int(0), C.c_uint64(0)
     check(_lib.load().d377_msm_stage_info(ms, C.byref(c), C.byref(w), C.byref(n)))
-    mixed = C.c_int(0)
+    mixed, windowed = C.c_int(0), C.c_int(0)
     check(_lib.load().d377_msm_last_mode(C.byref(mixed)))
+    check(_lib.load().d377_msm_last_windowed(C.byref(windowed)))
     return {"ms": dict(zip(MSM_STAGES, [float(x) for x in ms])), "c": c.value, "W": w.value,
-            "n": int(n.value), "mixed": bool(mixed.value)}
+            "n": int(n.value), "mixed": bool(mixed.value), "windowed": bool(windowed.value)}
 
 
 def msm_timeline() -> list:
@@ -438,19 +440,38 @@ class MsmBases:
     """Long-lived MSM bases (d377_msm_bases_create): ScalarMul::batch_convert_to_mul_base once
     (ark_curve/element.rs:27-34), then VariableBaseMSM::msm(&bases, &scalars) many times.
     Pass the object as `points` to vartime_multiscalar_mul / msm_submit / device.msm: only
-    the scalars cross the link and the normalisation is skipped."""
+    the scalars cross the link and the normalisation is skipped.
 
-    def __init__(self, points=None, point_format: int = PT_ELEMENT, *, device_ptr: int = 0, n: int = 0):
+    ``windowed=True`` (d377_msm_bases_create_windowed) also stores 2^(c j) * P_i for every
+    window j: n * W * 128 bytes of device memory, and every MSM over the set adds all windows
+    into one bucket set and skips the Horner tail.  ``c`` is the window width of such a set
+    (0: chosen from n; 4..22 otherwise).  ``.c``, ``.windows`` and ``.nbytes`` describe the
+    set (c = 0 and windows = 1 for a plain one)."""
+
+    def __init__(self, points=None, point_format: int = PT_ELEMENT, *, device_ptr: int = 0, n: int = 0,
+                 windowed: bool = False, c: int = 0):
         _ensure_init()
+        lib = _lib.load()
         out = C.c_void_p(0)
         if points is not None:
             pts = _arr(points, _PT_WIDTH[point_format], "points")
             n = pts.shape[0]
-            check(_lib.load().d377_msm_bases_create(_ptr(pts), point_format, n, C.byref(out)))
+            if windowed:
+                check(lib.d377_msm_bases_create_windowed(_ptr(pts), point_format, n, int(c), C.byref(out)))
+            else:
+                check(lib.d377_msm_bases_create(_ptr(pts), point_format, n, C.byref(out)))
+        elif windowed:
+            check(lib.d377_msm_bases_create_windowed_dev(C.c_void_p(device_ptr), point_format, n, int(c),
+                                                         C.byref(out)))
         else:
-            check(_lib.load().d377_msm_bases_create_dev(C.c_void_p(device_ptr), point_format, n, C.byref(out)))
+            check(lib.d377_msm_bases_create_dev(C.c_void_p(device_ptr), point_format, n, C.byref(out)))
         self.ptr = out.value or 0
         self.n = n
+        nn, cc, ww, nb = C.c_size_t(0), C.c_int(0), C.c_int(0), C.c_size_t(0)
+        check(lib.d377_msm_bases_info(C.c_void_p(self.ptr), C.byref(nn), C.byref(cc), C.byref(ww), C.byref(nb)))
+        self.c = int(cc.value)
+        self.windows = int(ww.value)
+        self.nbytes = int(nb.value)
 
     def close(self) -> None:
         if self.ptr:

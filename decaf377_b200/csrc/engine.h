@@ -34,6 +34,15 @@ struct MsmGeomInfo {
   int c = 0, W = 0;
 };
 
+// Layout of a set of prepared bases (d377_msm_bases_create*).  Plain sets: c = 0, W = 1, one
+// bucket operand per base.  Windowed sets (d377_msm_bases_create_windowed*): W slabs of n
+// operands, window-major with stride n; record j*n + i holds 2^(c*j) * P_i.
+struct BasesLayout {
+  size_t n = 0;
+  int c = 0, W = 1;
+  size_t bytes = 0;
+};
+
 // Per-device state of the Pippenger pipeline (msm.cu).
 struct MsmState {
   bool ready = false;
@@ -60,6 +69,7 @@ struct MsmState {
   DevBuf tail_ws[2];
   MsmGeomInfo last_geom;
   bool last_affine = false;
+  bool last_windowed = false;
   int last_groups = 1;
   size_t last_n = 0;
   bool stage_valid = false;
@@ -123,8 +133,8 @@ struct Engine {
   cudaStream_t out_stream = nullptr;
   cudaEvent_t pe_in[2] = {nullptr, nullptr}, pe_k[2] = {nullptr, nullptr}, pe_out[2] = {nullptr, nullptr};
   DevBuf st_in[2][3], st_out[2][2];
-  // prepared MSM bases handed out by d377_msm_bases_create: device pointer -> number of bases
-  std::unordered_map<const void*, size_t> bases;
+  // prepared MSM bases handed out by d377_msm_bases_create*: device pointer -> layout
+  std::unordered_map<const void*, BasesLayout> bases;
   // asynchronous MSMs (d377_msm_dev_async): sticky status word, reported by d377_sync
   bool async_status_dirty = false;
   MsmState msm;
@@ -255,8 +265,13 @@ int msm_enqueue(const uint8_t* scalars, const uint8_t* points, int point_format,
                 const cudaEvent_t* scalars_ready_ev = nullptr);
 cudaStream_t result_stream(Engine& e);
 int msm_check_flags(uint32_t flags);
-int check_bases(Engine& e, const uint8_t* points, size_t n);   // kernels.cu
+// kernels.cu; *layout (may be null) receives the set's layout
+int check_bases(Engine& e, const uint8_t* points, size_t n, BasesLayout* layout = nullptr);
 int msm_bases_prepare(const uint8_t* points, int point_format, size_t n, uint8_t* records);
+// the W - 1 upper slabs of a windowed set whose slab 0 msm_bases_prepare has written
+int msm_bases_fill_windows(uint8_t* table, size_t n, int c, int W);
+int msm_windowed_c(size_t n);    // window width of a windowed set when the caller passes c = 0
+bool msm_last_windowed();
 int msm_stage_info(float* ms, int* c, int* W, uint64_t* n);
 int msm_timeline(float* ms, int cap, int* ngroups);
 bool msm_last_mixed();

@@ -1254,7 +1254,10 @@ int d377_msm_bases_create_dev(const uint8_t* points, int point_format, size_t n,
   D377_CUDA(cudaMalloc(&rec, n * 128 + 128));
   int rc = msm_bases_prepare(points, point_format, n, rec);
   if (rc) { cudaFree(rec); return rc; }
-  _eng.bases[rec] = n;
+  BasesLayout bl;
+  bl.n = n;
+  bl.bytes = n * 128 + 128;
+  _eng.bases[rec] = bl;
   *bases = rec;
   return D377_OK;
 }
@@ -1273,6 +1276,84 @@ int d377_msm_bases_create(const uint8_t* points, int point_format, size_t n, uin
   if (rc) cudaStreamSynchronize(e.stream);
   cudaFree(tmp);
   return rc;
+}
+
+// Arguments of the windowed twins, checked before anything is allocated or read: *W receives
+// the number of windows of the width *c (0 = chosen from n).
+static int windowed_args(int point_format, size_t n, int* c, int* W, uint8_t** bases, const uint8_t* points) {
+  if (point_format < 0 || point_format > 3) { set_error("bad point_format %d", point_format); return D377_ERR_INVALID_ARG; }
+  if (!bases || (n && !points)) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
+  if (*c != 0 && (*c < 4 || *c > 22)) { set_error("window width %d out of range [4, 22]", *c); return D377_ERR_INVALID_ARG; }
+  if (*c == 0) *c = msm_windowed_c(n);
+  *W = (252 + *c - 1) / *c;
+  // the scatter stores a record index and a sign bit in 32 bits
+  if ((double)n * (double)*W >= 2147483648.0) {
+    set_error("windowed bases: n * W = %zu * %d records reach 2^31", n, *W);
+    return D377_ERR_INVALID_ARG;
+  }
+  return D377_OK;
+}
+
+int d377_msm_bases_create_windowed_dev(const uint8_t* points, int point_format, size_t n, int c, uint8_t** bases) {
+  D377_REQUIRE_READY();
+  int W = 0;
+  TRY(windowed_args(point_format, n, &c, &W, bases, points));
+  const size_t bytes = n * (size_t)W * 128 + 128;
+  uint8_t* tab = nullptr;
+  cudaError_t ce = cudaMalloc(&tab, bytes);
+  if (ce != cudaSuccess) {
+    cudaGetLastError();
+    set_error("windowed bases: cannot allocate %zu bytes of device memory (%s)", bytes, cudaGetErrorString(ce));
+    return D377_ERR_CUDA;
+  }
+  int rc = msm_bases_prepare(points, point_format, n, tab);   // slab 0 = the plain set
+  if (!rc) rc = msm_bases_fill_windows(tab, n, c, W);
+  if (rc) { cudaStreamSynchronize(_eng.stream); cudaFree(tab); return rc; }
+  BasesLayout bl;
+  bl.n = n;
+  bl.c = c;
+  bl.W = W;
+  bl.bytes = bytes;
+  _eng.bases[tab] = bl;
+  *bases = tab;
+  return D377_OK;
+}
+
+int d377_msm_bases_create_windowed(const uint8_t* points, int point_format, size_t n, int c, uint8_t** bases) {
+  D377_REQUIRE_READY();
+  int W = 0, cc = c;
+  TRY(windowed_args(point_format, n, &cc, &W, bases, points));
+  Engine& e = _eng;
+  const size_t pb = pt_bytes(point_format);
+  uint8_t* tmp = nullptr;
+  D377_CUDA(cudaMalloc(&tmp, n * pb + 128));
+  cudaError_t ce = cudaMemcpyAsync(tmp, points, n * pb, cudaMemcpyHostToDevice, e.stream);
+  if (ce != cudaSuccess) { cudaStreamSynchronize(e.stream); cudaFree(tmp); return cuda_fail(ce, "upload of the bases", __FILE__, __LINE__); }
+  int rc = d377_msm_bases_create_windowed_dev(tmp, point_format, n, c, bases);   // synchronises the stream
+  if (rc) cudaStreamSynchronize(e.stream);
+  cudaFree(tmp);
+  return rc;
+}
+
+int d377_msm_bases_info(const uint8_t* bases, size_t* n, int* c, int* windows, size_t* bytes) {
+  D377_REQUIRE_READY_NOJOIN();
+  auto it = _eng.bases.find(bases);
+  if (it == _eng.bases.end()) {
+    set_error("d377_msm_bases_info: %p is not a live set of prepared bases of device %d", (const void*)bases, _eng.device);
+    return D377_ERR_INVALID_ARG;
+  }
+  if (n) *n = it->second.n;
+  if (c) *c = it->second.c;
+  if (windows) *windows = it->second.W;
+  if (bytes) *bytes = it->second.bytes;
+  return D377_OK;
+}
+
+int d377_msm_last_windowed(int* windowed) {
+  D377_REQUIRE_READY();
+  if (!windowed) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
+  *windowed = msm_last_windowed() ? 1 : 0;
+  return D377_OK;
 }
 
 int d377_msm_bases_destroy(uint8_t* bases) {
@@ -1294,16 +1375,17 @@ int d377_msm_bases_destroy(uint8_t* bases) {
 
 namespace d377 {
 // D377_PT_BASES: `points` must be a live handle of this engine holding at least n bases
-int check_bases(Engine& e, const uint8_t* points, size_t n) {
+int check_bases(Engine& e, const uint8_t* points, size_t n, BasesLayout* layout) {
   auto it = e.bases.find(points);
   if (it == e.bases.end()) {
     set_error("msm: D377_PT_BASES needs the pointer d377_msm_bases_create returned (on device %d)", e.device);
     return D377_ERR_INVALID_ARG;
   }
-  if (n > it->second) {
-    set_error("msm: %zu scalars for %zu prepared bases", n, it->second);
+  if (n > it->second.n) {
+    set_error("msm: %zu scalars for %zu prepared bases", n, it->second.n);
     return D377_ERR_INVALID_ARG;
   }
+  if (layout) *layout = it->second;
   return D377_OK;
 }
 }  // namespace d377

@@ -228,6 +228,33 @@ void launch_normalize(const uint8_t* el, size_t n, uint8_t* scratch, uint8_t* ou
                                                                           e.tune_gcd_inv != 0);
 }
 
+// Windowed bases: the running points 2^(c j) * P_i, projective in `run` (n x 128 B), move on
+// to the next window: c doublings in place, one base per thread.  With `first` (slab 0 of
+// the table, the bucket operands (y-x, y+x, ...) of P_i) the running point is taken from
+// there instead: (X' : Y' : Z) = (2x : 2y : 2), in extended coordinates (2X' : 2Y' : 4 : X'Y').
+__global__ void __launch_bounds__(kBlk)
+k_msm_bases_double(uint8_t* __restrict__ run, const aff4_t* __restrict__ first, size_t n, int c) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  pt_t p;
+  if (first) {
+    const uint8_t* rec = reinterpret_cast<const uint8_t*>(first + i);
+    const fq_r ymx = fq_assume<1000>(fq_load(rec)), ypx = fq_assume<1000>(fq_load(rec + 32));
+    const fq_t x2 = fq_sub(ypx, ymx), y2 = fq_add(ypx, ymx);
+    p.x = fq_fold(fq_dbl(x2));
+    p.y = fq_fold(fq_dbl(y2));
+    p.z = fq_fold(fq_dbl(fq_dbl(fq_one())));
+    p.t = fq_mul(x2, y2);
+  } else {
+    p = pt_load(run + 128 * i);
+  }
+#pragma unroll 1
+  for (int k = 1; k < c; k++) p = pt_dbl<false>(p);
+  p = pt_dbl<true>(p);
+  D377_DBG_POINT(p);
+  pt_store(run + 128 * i, p);
+}
+
 // ---- 2./4. signed-digit recoding ------------------------------------------
 struct MsmGeom {
   int c;        // window width
@@ -252,8 +279,10 @@ D377_DI uint32_t scalar_window(const fq_raw_t& s, int w, int c) {
 // The kernel handles the windows [wa, wb) of one window group (`counts` and `dig` are the
 // group's own arrays, bucket ids are local to the group); the signed-digit carry into
 // window wa is recomputed from the windows below it.
+// `wstride`: bucket ids of consecutive windows lie this far apart -- g.K (one bucket set per
+// window) or 0 (windowed bases: every window of the group adds into ONE set of K buckets).
 __global__ void __launch_bounds__(256, 8)   // <= 32 registers: fits beside 4 accumulation CTAs
-k_msm_count(const uint8_t* __restrict__ scalars, size_t n, MsmGeom g, int wa, int wb,
+k_msm_count(const uint8_t* __restrict__ scalars, size_t n, MsmGeom g, int wa, int wb, uint32_t wstride,
             uint32_t* __restrict__ counts, uint32_t* __restrict__ dig, uint32_t* __restrict__ flags) {
   // grid-stride: when the kernel shares the SMs with an accumulation it is launched with
   // one CTA per SM (the registers an accumulation CTA set leaves over) and walks the batch
@@ -274,7 +303,7 @@ k_msm_count(const uint8_t* __restrict__ scalars, size_t n, MsmGeom g, int wa, in
       uint32_t e = 0xffffffffu;
       if (d != 0 && ok) {
         uint32_t mag = d < 0 ? (uint32_t)(-d) : (uint32_t)d;
-        uint32_t id = (uint32_t)(w - wa) * g.K + (mag - 1);
+        uint32_t id = (uint32_t)(w - wa) * wstride + (mag - 1);
         atomicAdd(&counts[id], 1u);   // result unused: compiles to RED.E.ADD
         e = id | (d < 0 ? 0x80000000u : 0u);
       }
@@ -289,11 +318,14 @@ k_msm_count(const uint8_t* __restrict__ scalars, size_t n, MsmGeom g, int wa, in
 // (n * 4 B) and its cursors resident in L2, so the random 4-byte stores merge there instead
 // of becoming DRAM read-modify-writes.  Every thread moves kScatterIlp entries so that as
 // many (digit -> atomic -> store) chains are in flight.
+// The stored index of entry i in row r is rec_base + r * rec_stride + i: the point index
+// (both 0), or the record (w, i) = w * N + i of a windowed set (rec_base = wa * N,
+// rec_stride = N).
 constexpr int kScatterIlp = 4;
 
 __global__ void __launch_bounds__(256, 8)
 k_msm_scatter(const uint32_t* __restrict__ dig, size_t n, uint32_t rows, uint32_t* __restrict__ cursor,
-              uint32_t* __restrict__ sorted) {
+              uint32_t* __restrict__ sorted, uint32_t rec_base, uint32_t rec_stride) {
   const size_t tiles_per_row = (n + 256 * kScatterIlp - 1) / (256 * kScatterIlp);
   const size_t total = tiles_per_row * rows;
   // row-major walk: all CTAs work on the same window at (almost) the same time
@@ -302,6 +334,7 @@ k_msm_scatter(const uint32_t* __restrict__ dig, size_t n, uint32_t rows, uint32_
     const size_t r = tile / tiles_per_row;
     const size_t base = (tile - r * tiles_per_row) * (256 * kScatterIlp) + threadIdx.x;
     const uint32_t* row = dig + r * n;
+    const uint32_t rec0 = rec_base + (uint32_t)r * rec_stride;
     uint32_t e[kScatterIlp], pos[kScatterIlp];
 #pragma unroll
     for (int k = 0; k < kScatterIlp; k++) {
@@ -314,7 +347,7 @@ k_msm_scatter(const uint32_t* __restrict__ dig, size_t n, uint32_t rows, uint32_
 #pragma unroll
     for (int k = 0; k < kScatterIlp; k++) {
       const size_t i = base + (size_t)k * 256;
-      if (e[k] != 0xffffffffu) sorted[pos[k]] = (uint32_t)i | (e[k] & 0x80000000u);
+      if (e[k] != 0xffffffffu) sorted[pos[k]] = (rec0 + (uint32_t)i) | (e[k] & 0x80000000u);
     }
   }
 }
@@ -1278,6 +1311,60 @@ int msm_bases_prepare(const uint8_t* points, int point_format, size_t n, uint8_t
   return msm_check_flags(*hflags);
 }
 
+// Windowed bases: slab j of `table` (n records at table + j * n * 128) gets the bucket
+// operands of 2^(c j) * P_i.  Slab 0 (P_i itself) has been written by msm_bases_prepare; the
+// running points are kept projective in a scratch of n x 128 B and every slab is one
+// k_msm_bases_double (c doublings) plus one batch normalisation (k_msm_normalize<128>).
+int msm_bases_fill_windows(uint8_t* table, size_t n, int c, int W) {
+  Engine& e = engine();
+  if (n == 0 || W <= 1) return D377_OK;
+  int rc = ensure(e.scratch, n * 32);
+  if (rc) return rc;
+  uint8_t* run = nullptr;
+  D377_CUDA(cudaMalloc(&run, n * 128));
+  size_t per = n >> 17;
+  per = per < 1 ? 1 : per;
+  size_t T = ((n + per - 1) / per + kNormBlk - 1) / kNormBlk * kNormBlk;
+  T = std::min(T, (size_t)e.sm_count * 3 * kNormBlk);
+  cudaError_t ce = cudaSuccess;
+  for (int j = 1; j < W && ce == cudaSuccess; j++) {
+    k_msm_bases_double<<<grid_for(n, kBlk), kBlk, 0, e.stream>>>(run, j == 1 ? (const aff4_t*)table : nullptr, n, c);
+    D377_LAUNCHED();
+    k_msm_normalize<128><<<(unsigned)(T / kNormBlk), kNormBlk, 0, e.stream>>>(
+        run, n, T, (uint8_t*)e.scratch.p, table + (size_t)j * n * 128, e.tune_gcd_inv != 0);
+    D377_LAUNCHED();
+    ce = cudaGetLastError();
+  }
+  if (ce == cudaSuccess) ce = cudaStreamSynchronize(e.stream);
+  else cudaStreamSynchronize(e.stream);
+  cudaFree(run);
+  if (ce != cudaSuccess) return cuda_fail(ce, "windowed bases", __FILE__, __LINE__);
+  return D377_OK;
+}
+
+// Window width of a windowed set created with c = 0.  Cost model as in choose_geom, with one
+// set of K buckets per MSM and no Horner tail: n W mixed additions (7 M) + the reduction of K
+// buckets (two additions each, ~32 M with the tree).  From 2^20 bases the choice is the
+// measured one (tools/msm_windowed_bench.py --c 16,18,20,21,22 on B200,
+// profiles/r3_msm_windowed_bench.json): c = 21 (W = 12) wins there -- back to back 2.01 /
+// 6.26 / 23.6 ms at 2^20 / 2^22 / 2^24 against 2.03 / 6.57 / 26.7 for c = 18 and 2.58 / 7.69 /
+// 27.2 for c = 22 -- where the model would still take 18 at 2^20.  Below 2^20 the model
+// decides (11 at 2^10, 15 at 2^16); at 2^16 the sweep measured c = 16 a little faster (blocking
+// 0.70 against 0.72 ms, back to back 0.47 against 0.55 ms), a point not swept densely enough yet
+// to change the model for.
+int msm_windowed_c(size_t n) {
+  if (n >= ((size_t)1 << 20)) return 21;
+  int best_c = 4;
+  double best = 1e300;
+  for (int c = 4; c <= 22; c++) {
+    const int W = (252 + c - 1) / c;
+    const double K = std::ldexp(1.0, c - 1);
+    const double cost = (double)W * (double)n * 7.0 + K * 32.0;
+    if (cost < best) { best = cost; best_c = c; }
+  }
+  return best_c;
+}
+
 // One Pippenger.  Head (point conversion, sort, bucket accumulation) on the engine and sort
 // streams; tail (stitch, bucket reduction, weighted tree, Horner, compress) on the tail
 // stream, over one of two tail-side workspace sets: the head of the next MSM starts right
@@ -1288,9 +1375,16 @@ int msm_bases_prepare(const uint8_t* points, int point_format, size_t n, uint8_t
 // event (or on nothing at all if *scalars_ready is null), and the scalar side of this MSM
 // is NOT ordered behind the engine stream: it starts as soon as its workspace set is free,
 // i.e. under the bucket accumulation of the previous MSM.
+//
+// `bases` (D377_PT_BASES only): the layout of the set `points` points into.  A windowed set
+// fixes c and W, and every window group then owns ONE set of K buckets: window w of the group
+// adds the record w * N + i (= 2^(c w) P_i, N = the set's stride) into bucket |d| - 1, the
+// groups' bucket sets are reduced like windows, and the tail sums the group results without
+// any doubling.
 static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_format, size_t n,
                     uint8_t* out_element, uint8_t* out_encoding, uint32_t* flags /* device, OR-ed */,
-                    const cudaEvent_t* scalars_ready = nullptr, const cudaEvent_t* points_ready = nullptr) {
+                    const cudaEvent_t* scalars_ready = nullptr, const cudaEvent_t* points_ready = nullptr,
+                    const BasesLayout* bases = nullptr) {
   Engine& e = engine();
   // scalars as the reference holds them in memory (Montgomery limbs): converted on the sort
   // stream into the workspace set before the digits are cut
@@ -1299,8 +1393,15 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   int rc = msm_state_init(e);
   if (rc) return rc;
   MsmState& ms = e.msm;
-  MsmGeom g = choose_geom(e, n);
-  const size_t nb = (size_t)g.W * g.K;
+  const bool windowed = point_format == D377_PT_BASES && bases && bases->c > 0;
+  MsmGeom g;
+  if (windowed) {
+    g.c = bases->c;
+    g.W = bases->W;
+    g.K = 1u << (g.c - 1);
+  } else {
+    g = choose_geom(e, n);
+  }
   const size_t max_entries = n * (size_t)g.W;
   // Run length per accumulate thread.  Every run boundary splits a bucket into pieces
   // that k_msm_seg_reduce has to stitch (one extra addition each), so runs are as long
@@ -1379,15 +1480,24 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   const unsigned sort_cap = ngroups > 1 || may_prefetch
                                 ? (unsigned)e.sm_count * (unsigned)std::max(1, e.tune_sort_ctas) : 0u;
   auto capped = [&](size_t want) { return (unsigned)(sort_cap ? std::min<size_t>(want, sort_cap) : want); };
+  // Buckets of group k: one set per window, or one merged set (windowed bases).  g_bucket[k]
+  // is the group's first bucket in `bsum`; rg is the geometry the bucket reduction sees (a
+  // merged set is reduced like one window).
   size_t g_nthreads[kMaxGroups], g_tbase[kMaxGroups + 1], g_ntiles[kMaxGroups];
+  size_t g_nb[kMaxGroups], g_bucket[kMaxGroups];
   g_tbase[0] = 0;
   for (int k = 0; k < ngroups; k++) {
     size_t ent_k = (size_t)(whi[k] - wlo[k]) * n;
     g_nthreads[k] = (ent_k + L - 1) / L;
     g_tbase[k + 1] = g_tbase[k] + g_nthreads[k];
-    g_ntiles[k] = ((size_t)(whi[k] - wlo[k]) * g.K + 1 + kScanTile - 1) / kScanTile;
+    g_nb[k] = windowed ? (size_t)g.K : (size_t)(whi[k] - wlo[k]) * g.K;
+    g_bucket[k] = windowed ? (size_t)k * g.K : (size_t)wlo[k] * g.K;
+    g_ntiles[k] = (g_nb[k] + 1 + kScanTile - 1) / kScanTile;
   }
   const size_t nthreads = g_tbase[ngroups];
+  MsmGeom rg = g;
+  if (windowed) rg.W = ngroups;
+  const size_t nb = (size_t)rg.W * g.K;
 
   // Bucket additions against affine records cost 7 M instead of 8: free when the input
   // already has Z = 1; Element inputs are normalised first when the batch is large enough
@@ -1432,8 +1542,8 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   size_t o_sc = carve(sc_mont ? n * 32 : 0);
   size_t o_counts[kMaxGroups], o_cursor[kMaxGroups], o_tiles[kMaxGroups];
   for (int k = 0; k < ngroups; k++) {
-    o_counts[k] = carve(((size_t)(whi[k] - wlo[k]) * g.K + 1) * 4);
-    o_cursor[k] = carve(((size_t)(whi[k] - wlo[k]) * g.K + 1) * 4);
+    o_counts[k] = carve((g_nb[k] + 1) * 4);
+    o_cursor[k] = carve((g_nb[k] + 1) * 4);
     o_tiles[k] = carve(g_ntiles[k] * 4 + 4);
   }
   size_t o_bsum = carve(nb * sizeof(pt_t));
@@ -1446,7 +1556,7 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   size_t o_pb2 = carve(2 * nthreads2 * 4);
   size_t o_part3 = carve(2 * nthreads3 * sizeof(pt_t));
   size_t o_pb3 = carve(2 * nthreads3 * 4);
-  const size_t seg_n = (size_t)g.W * S, seg_n2 = (size_t)g.W * ((S + kWT - 1) / kWT);
+  const size_t seg_n = (size_t)rg.W * S, seg_n2 = (size_t)rg.W * ((S + kWT - 1) / kWT);
   size_t o_seg_a = carve(seg_n * sizeof(pt_t));
   size_t o_seg_p = carve(seg_n * sizeof(pt_t));
   size_t o_seg_a2 = carve(seg_n2 * sizeof(pt_t));
@@ -1484,6 +1594,7 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   ms.last_geom.W = g.W;
   ms.last_n = n;
   ms.last_affine = affine;
+  ms.last_windowed = windowed;
   ms.last_groups = ngroups;
   ms.stage_valid = true;
   auto stage_mark = [&](int i, cudaStream_t s) { return cudaEventRecord(ms.ev_stage[i], s); };
@@ -1519,12 +1630,13 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   // ---- scalar side, all groups, on the sort stream (2, 3, 4) ----
   for (int k = 0; k < ngroups; k++) {
     const int wa = wlo[k], wb = whi[k];
-    const size_t nbk = (size_t)(wb - wa) * g.K;
+    const size_t nbk = g_nb[k];
     uint32_t* counts = (uint32_t*)(tw + o_counts[k]);
     uint32_t* tiles = (uint32_t*)(tw + o_tiles[k]);
     uint32_t* cursor = (uint32_t*)(tw + o_cursor[k]);
     D377_CUDA(cudaMemsetAsync(counts, 0, (nbk + 1) * 4, ss));
-    k_msm_count<<<capped(grid_for(n, 256)), 256, 0, ss>>>(scalars, n, g, wa, wb, counts, dig + (size_t)wa * n, flags);
+    k_msm_count<<<capped(grid_for(n, 256)), 256, 0, ss>>>(scalars, n, g, wa, wb, windowed ? 0u : g.K, counts,
+                                                          dig + (size_t)wa * n, flags);
     D377_LAUNCHED();
     k_scan_tiles<<<(unsigned)g_ntiles[k], kScanBlock, 0, ss>>>(counts, nbk + 1, tiles);
     D377_LAUNCHED();
@@ -1533,7 +1645,8 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
     k_scan_apply<<<(unsigned)g_ntiles[k], kScanBlock, 0, ss>>>(counts, nbk + 1, tiles, cursor);
     D377_LAUNCHED();
     k_msm_scatter<<<capped((size_t)grid_for(n, 256 * kScatterIlp) * (size_t)(wb - wa)), 256, 0, ss>>>(
-        dig + (size_t)wa * n, n, (uint32_t)(wb - wa), cursor, sorted + (size_t)wa * n);
+        dig + (size_t)wa * n, n, (uint32_t)(wb - wa), cursor, sorted + (size_t)wa * n,
+        windowed ? (uint32_t)((size_t)wa * bases->n) : 0u, windowed ? (uint32_t)bases->n : 0u);
     D377_LAUNCHED();
     D377_CUDA(cudaEventRecord(ms.ev_sorted[k], ss));
   }
@@ -1567,23 +1680,23 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   // 128 threads, ~106 registers, 4 CTAs/SM: measured flat from 4 to 7 CTAs/SM (the
   // fmaheavy pipe, not latency, is the limiter), slower at 8 (spills).
   for (int k = 0; k < ngroups; k++) {
-    const int wa = wlo[k], wb = whi[k];
-    const size_t nbk = (size_t)(wb - wa) * g.K;
+    const int wa = wlo[k];
+    const size_t nbk = g_nb[k], b0 = g_bucket[k];
     const uint32_t* counts = (const uint32_t*)(tw + o_counts[k]);
     D377_CUDA(cudaStreamWaitEvent(st, ms.ev_sorted[k], 0));
     D377_CUDA(cudaEventRecord(ms.ev_acc0[k], st));
     if (affine && e.tune_acc_tma)
       k_msm_accumulate_tma<<<grid_for(g_nthreads[k], kBlk), kBlk, 2 * kBlk * kTmaSlot + (kBlk / 32) * 16, st>>>(
-          aff_in, sorted + (size_t)wa * n, counts, (uint32_t)nbk, L, bsum + (size_t)wa * g.K,
-          part + 2 * g_tbase[k], pb + 2 * g_tbase[k], (int32_t)((size_t)wa * g.K));
+          aff_in, sorted + (size_t)wa * n, counts, (uint32_t)nbk, L, bsum + b0,
+          part + 2 * g_tbase[k], pb + 2 * g_tbase[k], (int32_t)b0);
     else if (affine)
       k_msm_accumulate<true><<<grid_for(g_nthreads[k], kBlk), kBlk, 0, st>>>(
-          aff_in, sorted + (size_t)wa * n, counts, (uint32_t)nbk, L, bsum + (size_t)wa * g.K,
-          part + 2 * g_tbase[k], pb + 2 * g_tbase[k], (int32_t)((size_t)wa * g.K));
+          aff_in, sorted + (size_t)wa * n, counts, (uint32_t)nbk, L, bsum + b0,
+          part + 2 * g_tbase[k], pb + 2 * g_tbase[k], (int32_t)b0);
     else
       k_msm_accumulate<false><<<grid_for(g_nthreads[k], kBlk), kBlk, 0, st>>>(
-          cached, sorted + (size_t)wa * n, counts, (uint32_t)nbk, L, bsum + (size_t)wa * g.K,
-          part + 2 * g_tbase[k], pb + 2 * g_tbase[k], (int32_t)((size_t)wa * g.K));
+          cached, sorted + (size_t)wa * n, counts, (uint32_t)nbk, L, bsum + b0,
+          part + 2 * g_tbase[k], pb + 2 * g_tbase[k], (int32_t)b0);
     D377_LAUNCHED();
     D377_CUDA(cudaEventRecord(ms.ev_acc[k], st));
   }
@@ -1623,11 +1736,11 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
     GroupTab gt;
     gt.ng = ngroups;
     for (int k = 0; k < ngroups; k++) {
-      gt.wlo[k] = wlo[k];
-      gt.whi[k] = whi[k];
+      gt.wlo[k] = windowed ? k : wlo[k];
+      gt.whi[k] = windowed ? k + 1 : whi[k];
       gt.offs[k] = (const uint32_t*)(tw + o_counts[k]);
     }
-    k_msm_bucket_reduce_ap<<<grid_for((size_t)g.W * S, kBlk), kBlk, 0, ts>>>(bsum, gt, g, Lseg, log_lseg, S, a, p);
+    k_msm_bucket_reduce_ap<<<grid_for((size_t)rg.W * S, kBlk), kBlk, 0, ts>>>(bsum, gt, rg, Lseg, log_lseg, S, a, p);
     D377_LAUNCHED();
   }
   D377_CUDA(cudaGetLastError());
@@ -1635,13 +1748,14 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   // 8: weighted tree -> one sum per window, Horner over the windows, output
   for (uint32_t len = S; len > 1;) {
     const uint32_t olen = (len + kWT - 1) / kWT;
-    k_wsum_tree<<<dim3(olen, (unsigned)g.W), 2 * kWT, 0, ts>>>(a, p, len, a2, p2);
+    k_wsum_tree<<<dim3(olen, (unsigned)rg.W), 2 * kWT, 0, ts>>>(a, p, len, a2, p2);
     D377_LAUNCHED();
     std::swap(a, a2);
     std::swap(p, p2);
     len = olen;
   }
-  rc = finish(ts, a, g.W, g.c, out_element, out_encoding);
+  // windowed: the group sums are already weighted by 2^(c w), k_finish only adds them
+  rc = finish(ts, a, rg.W, windowed ? 0 : g.c, out_element, out_encoding);
   if (rc) return rc;
   D377_CUDA(stage_mark(8, ts));
   D377_CUDA(cudaEventRecord(ms.ev_tail_done[set], ts));
@@ -1666,6 +1780,14 @@ int msm_enqueue(const uint8_t* scalars, const uint8_t* points, int point_format,
   if (chunk == 0 || chunk > kMax) chunk = kMax;
   size_t nchunks = (n + chunk - 1) / chunk;
   if (nchunks > 16) { set_error("msm: too many chunks (n = %zu, chunk = %zu)", n, chunk); return D377_ERR_INVALID_ARG; }
+  // prepared bases: the set's layout (a windowed set keeps its stride N in every chunk, whose
+  // records start at points + 128 * lo)
+  BasesLayout layout;
+  if (pf == D377_PT_BASES) {
+    int rc = check_bases(e, points, n, &layout);
+    if (rc) return rc;
+  }
+  const BasesLayout* bl = pf == D377_PT_BASES ? &layout : nullptr;
   // inputs_ready: the inputs depend on nothing but chunk_ready[k] (or on nothing)
   auto ready_of = [&](size_t k) -> const cudaEvent_t* {
     return !inputs_ready ? nullptr : chunk_ready ? &chunk_ready[k] : &no_event;
@@ -1677,14 +1799,15 @@ int msm_enqueue(const uint8_t* scalars, const uint8_t* points, int point_format,
   };
   if (nchunks == 1) {
     if (chunk_ready) D377_CUDA(cudaStreamWaitEvent(e.stream, chunk_ready[0], 0));
-    return msm_once(scalars, points, point_format, n, out_element, out_encoding, flags, sc_ready_of(0), ready_of(0));
+    return msm_once(scalars, points, point_format, n, out_element, out_encoding, flags, sc_ready_of(0), ready_of(0),
+                    bl);
   }
   pt_t* partials = (pt_t*)(e.d_small + kSmallPartials);  // up to 16 chunk results
   for (size_t k = 0; k < nchunks; k++) {
     size_t lo = k * chunk, len = std::min(chunk, n - lo);
     if (chunk_ready) D377_CUDA(cudaStreamWaitEvent(e.stream, chunk_ready[k], 0));
     int rc = msm_once(scalars + 32 * lo, points + pbytes * lo, point_format, len,
-                      (uint8_t*)(partials + k), nullptr, flags, sc_ready_of(k), ready_of(k));
+                      (uint8_t*)(partials + k), nullptr, flags, sc_ready_of(k), ready_of(k), bl);
     if (rc) return rc;
   }
   cudaStream_t rs = result_stream(e);
@@ -1746,6 +1869,7 @@ int msm_dev_async(const uint8_t* scalars, const uint8_t* points, int point_forma
 }
 
 bool msm_last_mixed() { return engine().msm.last_affine; }
+bool msm_last_windowed() { return engine().msm.last_windowed; }
 
 // d377_shutdown: the streams and events above belong to the device being released
 void msm_shutdown(Engine& e) {

@@ -66,7 +66,7 @@ extern "C" {
                             * out moves 128 instead of 160 bytes per (scalar, point) pair over
                             * PCIe, which is the bound of a host-buffer MSM. */
 #define D377_PT_BASES 4    /* prepared bases: `points` is the DEVICE pointer d377_msm_bases_create
-                            * returned (128 B per base).  d377_msm* only, host-buffer entry points
+                            * (128 B per base) or d377_msm_bases_create_windowed returned.  d377_msm* only, host-buffer entry points
                             * included: only the scalars cross the link. */
 
 /* Scalars as the reference keeps them in memory.  `Fr` is stored in Montgomery form
@@ -317,7 +317,8 @@ int d377_multi_sync(void);
 int d377_msm_submit(const uint8_t* scalars, const uint8_t* points, int point_format, size_t n,
                     int slot);
 int d377_msm_wait(int slot, uint8_t out_element[128], uint8_t out_encoding[32]);
-/* Override the Pippenger window width c (0 = choose from n; otherwise 4..22). */
+/* Override the Pippenger window width c (0 = choose from n; otherwise 4..22).  MSMs over
+ * windowed bases (d377_msm_bases_create_windowed) always use the width of the set. */
 int d377_msm_set_window(int c);
 /* 1 (default): run MSM tails on the result stream, overlapped with the next MSM's head;
  * 0: everything on the engine stream (A/B measurements). */
@@ -346,6 +347,28 @@ int d377_msm_set_host_chunks(int k);
  * fail with D377_ERR_INVALID_ENCODING. */
 int d377_msm_bases_create(const uint8_t* points, int point_format, size_t n, uint8_t** bases);
 int d377_msm_bases_create_dev(const uint8_t* points, int point_format, size_t n, uint8_t** bases);
+/* Prepared bases with precomputed window multiples: the table holds 2^(c*j) * P_i for
+ * j = 0 .. W-1, W = ceil(252 / c), 128 B per entry (n * W * 128 B of device memory), laid out
+ * window-major (entry (i, j) is record j*n + i).  Every MSM over such a set adds all its
+ * windows into ONE set of 2^(c-1) buckets per window group and has no Horner tail.
+ * c = 0: chosen from n; otherwise 4 <= c <= 22.  The handle is used exactly like the one
+ * d377_msm_bases_create returns: d377_msm* with D377_PT_BASES, any prefix n' <= n,
+ * d377_msm_bases_destroy, released by d377_shutdown.  The MSM always uses the set's c
+ * (d377_msm_set_window does not apply), so a small prefix of a large set still pays for
+ * the reduction of the large set's 2^(c-1) buckets.
+ * Refused with D377_ERR_INVALID_ARG before anything is allocated or read: c outside [4, 22]
+ * (other than 0) and n * W >= 2^31.  If the table cannot be allocated the call returns
+ * D377_ERR_CUDA and d377_last_error names the byte count.  Invalid encodings among the
+ * bases give D377_ERR_INVALID_ENCODING.
+ * Measured on one B200 (1000 W; DESIGN.md 3.5): creation ~0.45 s for 2^24 bases at c = 21
+ * (27 ms for 2^20), 1536 B of device memory per base at c = 21 (W = 12); per MSM against a
+ * plain set, back to back 23.6 against 25.2 ms at 2^24, blocking 0.72 against 1.12 ms at 2^16. */
+int d377_msm_bases_create_windowed(const uint8_t* points, int point_format, size_t n, int c, uint8_t** bases);
+int d377_msm_bases_create_windowed_dev(const uint8_t* points, int point_format, size_t n, int c, uint8_t** bases);
+/* n, c, W and device bytes of a live handle (W = 1 and c = 0 for a plain prepared set) */
+int d377_msm_bases_info(const uint8_t* bases, size_t* n, int* c, int* windows, size_t* bytes);
+/* *windowed = 1 if the most recent single-chunk MSM ran over a windowed set of bases */
+int d377_msm_last_windowed(int* windowed);
 int d377_msm_bases_destroy(uint8_t* bases);
 int d377_msm_stage_info(float ms[8], int* c, int* W, uint64_t* n);
 /* Timeline of the most recent single-chunk MSM, four floats per window group in the order

@@ -94,6 +94,12 @@ extern "C" {
                       out: *mut u8, out_format: c_int, ok: *mut u8) -> c_int;
     fn d377_msm_bases_create(points: *const u8, point_format: c_int, n: usize, bases: *mut *mut u8) -> c_int;
     fn d377_msm_bases_destroy(bases: *mut u8) -> c_int;
+    fn d377_msm_bases_create_windowed(points: *const u8, point_format: c_int, n: usize, c: c_int,
+                                      bases: *mut *mut u8) -> c_int;
+    fn d377_msm_bases_create_windowed_dev(points: *const u8, point_format: c_int, n: usize, c: c_int,
+                                          bases: *mut *mut u8) -> c_int;
+    fn d377_msm_bases_info(bases: *const u8, n: *mut usize, c: *mut c_int, windows: *mut c_int,
+                           bytes: *mut usize) -> c_int;
     fn d377_host_alloc(bytes: usize) -> *mut c_void;
     fn d377_host_free(p: *mut c_void) -> c_int;
 }
@@ -548,6 +554,23 @@ impl GpuBases {
         Ok(GpuBases { ptr, len: points.len() })
     }
 
+    /// The same bases with the window multiples 2^(c j) * P_i precomputed
+    /// (d377_msm_bases_create_windowed: n * ceil(252 / c) * 128 bytes of device memory, and
+    /// every `msm` skips the Horner tail).  `c` = 0 lets the library choose from n.
+    pub fn new_windowed(points: &[Element], c: i32) -> Result<Self, GpuError> {
+        let w = elements_to_wire(points);
+        let mut ptr: *mut u8 = core::ptr::null_mut();
+        check(unsafe { d377_msm_bases_create_windowed(w.as_ptr(), PT_ELEMENT, points.len(), c as c_int, &mut ptr) })?;
+        Ok(GpuBases { ptr, len: points.len() })
+    }
+
+    /// (window width c, windows W, device bytes) of the set: (0, 1, _) for `new`.
+    pub fn layout(&self) -> Result<(i32, i32, usize), GpuError> {
+        let (mut n, mut c, mut w, mut bytes) = (0usize, 0 as c_int, 0 as c_int, 0usize);
+        check(unsafe { d377_msm_bases_info(self.ptr as *const u8, &mut n, &mut c, &mut w, &mut bytes) })?;
+        Ok((c as i32, w as i32, bytes))
+    }
+
     pub fn len(&self) -> usize {
         self.len
     }
@@ -654,6 +677,8 @@ mod tests {
         assert_eq!(msm, Element::vartime_multiscalar_mul(s.iter(), p.iter()));
         let bases = GpuBases::new(&p).unwrap();
         assert_eq!(bases.msm(&s).unwrap(), msm);
+        let win = GpuBases::new_windowed(&p, 0).unwrap();
+        assert_eq!(win.msm(&s).unwrap(), msm);
         let g = generator_mul_batch(&s).unwrap();
         for i in 0..s.len() {
             assert_eq!(g[i], Element::GENERATOR * s[i]);
