@@ -81,22 +81,12 @@ struct Engine {
   int sm_count = 148;
   cudaStream_t stream = nullptr;
   std::recursive_mutex mu;
+  // set through the ABI (d377_msm_set_*); the defaults are the library's own choices
   int msm_window_override = 0;
   int msm_host_chunks_override = 0;
-  int tune_acc_run = 0, tune_reduce_seg = 0;  // D377_ACC_RUN / D377_REDUCE_SEG (experiments)
-  int tune_groups = 0;                        // D377_MSM_GROUPS: window groups of the sort/accumulate pipeline
-  int tune_sort_ctas = 1;                     // D377_MSM_SORT_CTAS: sort CTAs per SM while pipelined
-  int tune_normalize = 0;                     // D377_MSM_NORMALIZE: -1 never, 1 always, 0 auto
-  int tune_gcd_inv = 1;                       // D377_GCD_INV: 0 = Fermat inversion in the normalisation (A/B)
-  int tune_norm_wave = 3;                     // D377_MSM_NORM_WAVE: normalisation CTAs per SM (one resident wave); 0 = by batch size
-  int tune_stitch_warp = 1 << 18;             // D377_MSM_STITCH_WARP: stitch levels with at most this many slots use the warp-scan kernel
-  int tune_tail_overlap = 1;                  // D377_MSM_TAIL_OVERLAP: 0 = tails on the engine stream (A/B)
-  int tune_tail_prio = 1;                     // D377_MSM_TAIL_PRIO: 1 = tail stream at the greatest priority
-  int tune_norm_min_per = 8;                  // D377_MSM_NORM_MIN_PER: normalise Element inputs when n / 2^17 >= this
-  int tune_points_prefetch = 1;               // D377_MSM_POINTS_PREFETCH: 0 = point conversion on the engine stream (A/B)
-  int tune_points_prio = 0;                   // D377_MSM_POINTS_PRIO: 1 = points stream at the greatest priority (default: least)
-  int tune_acc_tma = 0;                       // D377_MSM_ACC_TMA: 1 = bucket accumulation with the TMA-staged operand stream (experiment)
-  int tune_sort_prefetch = 1;                 // D377_MSM_SORT_PREFETCH: 0 = the sort always forks from the engine stream (A/B)
+  int msm_groups_override = 0;        // window groups of the sort / accumulate pipeline
+  int msm_normalize_override = 0;     // Element / XYZ inputs: -1 never normalised, 1 always, 0 auto
+  int msm_tail_overlap_override = 1;  // 0 = MSM tails on the engine stream
   // host-API staging
   DevBuf in0, in1, out0, out1;
   // prefix products of k_normalize
@@ -108,8 +98,6 @@ struct Engine {
   // fixed-base table (niels, affine) and its geometry
   void* fb_table = nullptr;
   void* fb_table_jq = nullptr;   // the same multiples on the Jacobi quartic (encoding output)
-  int tune_fb_quartic = 1;       // D377_FB_QUARTIC: 0 = Edwards additions + compress (A/B)
-  size_t fb_quartic_min = (size_t)1 << 18;  // D377_FB_QUARTIC_MIN: smallest batch that builds the 1.6 GB quartic table
   size_t fb_batch_hint = 0;      // size of the host-buffer batch whose chunks are being launched
   // scratch of element_sum_on: [0] engine stream, [1] result stream
   DevBuf sum_ws[2];

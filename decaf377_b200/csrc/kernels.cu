@@ -278,23 +278,6 @@ static int engine_create(int device) {
     D377_CUDA(cudaEventCreateWithFlags(&e.pe_out[b], cudaEventDisableTiming));
   }
   D377_CUDA(cudaEventCreateWithFlags(&e.ev_partial, cudaEventDisableTiming));
-  if (const char* v = getenv("D377_ACC_RUN")) e.tune_acc_run = atoi(v);
-  if (const char* v = getenv("D377_REDUCE_SEG")) e.tune_reduce_seg = atoi(v);
-  if (const char* v = getenv("D377_MSM_NORMALIZE")) e.tune_normalize = atoi(v);
-  if (const char* v = getenv("D377_MSM_GROUPS")) e.tune_groups = atoi(v);
-  if (const char* v = getenv("D377_MSM_SORT_CTAS")) e.tune_sort_ctas = atoi(v);
-  if (const char* v = getenv("D377_MSM_STITCH_WARP")) e.tune_stitch_warp = atoi(v);
-  if (const char* v = getenv("D377_MSM_NORM_WAVE")) e.tune_norm_wave = atoi(v);
-  if (const char* v = getenv("D377_GCD_INV")) e.tune_gcd_inv = atoi(v);
-  if (const char* v = getenv("D377_FB_QUARTIC")) e.tune_fb_quartic = atoi(v);
-  if (const char* v = getenv("D377_FB_QUARTIC_MIN")) e.fb_quartic_min = (size_t)atoll(v);
-  if (const char* v = getenv("D377_MSM_TAIL_OVERLAP")) e.tune_tail_overlap = atoi(v);
-  if (const char* v = getenv("D377_MSM_TAIL_PRIO")) e.tune_tail_prio = atoi(v);
-  if (const char* v = getenv("D377_MSM_SORT_PREFETCH")) e.tune_sort_prefetch = atoi(v);
-  if (const char* v = getenv("D377_MSM_ACC_TMA")) e.tune_acc_tma = atoi(v);
-  if (const char* v = getenv("D377_MSM_POINTS_PREFETCH")) e.tune_points_prefetch = atoi(v);
-  if (const char* v = getenv("D377_MSM_POINTS_PRIO")) e.tune_points_prio = atoi(v);
-  if (const char* v = getenv("D377_MSM_NORM_MIN_PER")) e.tune_norm_min_per = atoi(v);
   e.ready = true;
   bool known = false;
   for (int k = 0; k < g_norder; k++) known = known || g_order[k] == device;
@@ -562,13 +545,13 @@ int d377_msm_last_mode(int* mixed) {
 
 int d377_msm_set_normalize(int mode) {
   if (mode < -1 || mode > 1) { set_error("normalize mode %d out of range [-1, 1]", mode); return D377_ERR_INVALID_ARG; }
-  engine().tune_normalize = mode;
+  engine().msm_normalize_override = mode;
   return D377_OK;
 }
 
 int d377_msm_set_groups(int groups) {
   if (groups < 0 || groups > 8) { set_error("group count %d out of range [0, 8]", groups); return D377_ERR_INVALID_ARG; }
-  engine().tune_groups = groups;
+  engine().msm_groups_override = groups;
   return D377_OK;
 }
 
@@ -593,7 +576,7 @@ int d377_msm_set_host_chunks(int k) {
 
 int d377_msm_set_tail_overlap(int on) {
   D377_REQUIRE_READY();
-  _eng.tune_tail_overlap = on ? 1 : 0;
+  _eng.msm_tail_overlap_override = on ? 1 : 0;
   return D377_OK;
 }
 
@@ -751,9 +734,9 @@ int d377_fixed_base_mul_dev(const uint8_t* scalars, size_t n, uint8_t* out, int 
   // win that back builds it (or finds it built); smaller calls take the Edwards table +
   // compress, whose output is bit-identical.  The host-buffer entry point passes the size of
   // the whole batch through fb_batch_hint so that its chunks agree.
+  constexpr size_t kFbQuarticMin = (size_t)1 << 18;
   const size_t batch = std::max(n, e.fb_batch_hint);
-  bool quartic = out_format == D377_OUT_ENCODING && e.tune_fb_quartic &&
-                 (e.fb_table_jq != nullptr || batch >= e.fb_quartic_min);
+  bool quartic = out_format == D377_OUT_ENCODING && (e.fb_table_jq != nullptr || batch >= kFbQuarticMin);
   if (quartic && ensure_fb_table_jq() != D377_OK) {
     // no room for the quartic table: the Edwards path gives the same bytes
     cudaGetLastError();

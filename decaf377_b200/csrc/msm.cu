@@ -153,7 +153,7 @@ constexpr int kNormBlk = 256;
 template <int kStride, bool kXY = false>
 __global__ void __launch_bounds__(kNormBlk)
 k_msm_normalize(const uint8_t* __restrict__ pts, size_t n, size_t T, uint8_t* __restrict__ scratch,
-                void* __restrict__ out_v, bool gcd_inv) {
+                void* __restrict__ out_v) {
   aff4_t* out = reinterpret_cast<aff4_t*>(out_v);
   uint8_t* out_xy = reinterpret_cast<uint8_t*>(out_v);
   __shared__ fq_t sh[kNormBlk / 32 + 1];
@@ -185,7 +185,7 @@ k_msm_normalize(const uint8_t* __restrict__ pts, size_t n, size_t T, uint8_t* __
     fq_t tot = sh[0];
 #pragma unroll 1
     for (int v = 1; v < kNormBlk / 32; v++) tot = fq_mul(tot, sh[v]);
-    fq_t inv = gcd_inv ? fq_inv_vartime(tot) : fq_inv(tot);
+    fq_t inv = fq_inv_vartime(tot);
     if (lane == 0) sh[kNormBlk / 32] = inv;
   }
   __syncthreads();
@@ -217,15 +217,42 @@ k_msm_normalize(const uint8_t* __restrict__ pts, size_t n, size_t T, uint8_t* __
   }
 }
 
+// Thread count T of a batch normalisation of n points: every thread walks per >= min_per
+// strided points, per = n / 2^17 so that >= 2^17 threads stay busy, and T is capped at one
+// wave: every CTA is resident from the start (3 per SM at <= 80 registers), so the kernel has
+// no ragged last wave and the CTA-wide inversion bubble occurs once.
+constexpr size_t kNormCtasPerSm = 3;
+
+static size_t normalize_threads(size_t n, size_t min_per, int sm_count) {
+  const size_t per = std::max(n >> 17, min_per);
+  const size_t T = ((n + per - 1) / per + kNormBlk - 1) / kNormBlk * kNormBlk;
+  return std::min(T, (size_t)sm_count * kNormCtasPerSm * kNormBlk);
+}
+
 // d377_batch_normalize: same kernel, one resident wave of CTAs (or fewer for small batches).
 void launch_normalize(const uint8_t* el, size_t n, uint8_t* scratch, uint8_t* out, cudaStream_t st) {
-  Engine& e = engine();
-  size_t per = n >> 17;
-  per = per < 1 ? 1 : per;
-  size_t T = ((n + per - 1) / per + kNormBlk - 1) / kNormBlk * kNormBlk;
-  T = std::min(T, (size_t)e.sm_count * 3 * kNormBlk);
-  k_msm_normalize<128, true><<<(unsigned)(T / kNormBlk), kNormBlk, 0, st>>>(el, n, T, scratch, out,
-                                                                          e.tune_gcd_inv != 0);
+  const size_t T = normalize_threads(n, 1, engine().sm_count);
+  k_msm_normalize<128, true><<<(unsigned)(T / kNormBlk), kNormBlk, 0, st>>>(el, n, T, scratch, out);
+}
+
+// Input points of any wire format -> affine bucket operands on `st`: Element / XYZ by batch
+// normalisation (normalize_threads(n, min_per), `scratch` n x 32 B), AffinePoint / Encoding
+// one point per thread (an invalid encoding sets bit 1 of `flags`).
+static void launch_points_affine(const Engine& e, int point_format, const uint8_t* pts, size_t n, size_t min_per,
+                                 uint8_t* scratch, aff4_t* out, uint32_t* flags, cudaStream_t st) {
+  if (point_format == D377_PT_ELEMENT || point_format == D377_PT_XYZ) {
+    const size_t T = normalize_threads(n, min_per, e.sm_count);
+    if (point_format == D377_PT_ELEMENT)
+      k_msm_normalize<128><<<(unsigned)(T / kNormBlk), kNormBlk, 0, st>>>(pts, n, T, scratch, out);
+    else
+      k_msm_normalize<96><<<(unsigned)(T / kNormBlk), kNormBlk, 0, st>>>(pts, n, T, scratch, out);
+  } else if (point_format == D377_PT_AFFINE) {
+    k_msm_points_affine<D377_PT_AFFINE><<<grid_for(n, kBlk), kBlk, 0, st>>>(pts, n, out, flags);
+  } else {
+    k_msm_points_affine<D377_PT_ENCODING><<<grid_for(n, kBlk), kBlk, ISQRT_SMEM_WORDS(kBlk) * 4, st>>>(pts, n, out,
+                                                                                                        flags);
+  }
+  D377_LAUNCHED();
 }
 
 // Windowed bases: the running points 2^(c j) * P_i, projective in `run` (n x 128 B), move on
@@ -552,141 +579,6 @@ k_msm_accumulate(const void* __restrict__ pts_v, const uint32_t* __restrict__ so
   }
 }
 
-// ---- 5b. the same accumulation with a TMA-staged operand stream (experiment) ---------
-// The north star asks for "a TMA-staged point stream".  The stream of a bucket sort is a
-// gather of 128-byte records at random addresses, so the staging unit is one record per
-// lane: every lane issues `cp.async.bulk` (1-D bulk copy, the TMA unit: UBLKCP in SASS) of
-// the NEXT entry's record into its own shared-memory slot while the current entry is added;
-// a warp shares one mbarrier per stage (one lane arms it with the bytes its lanes are about
-// to request, every lane's copy completes on it, every lane waits on its phase).  Two
-// stages of 128 x 144 B (the slots are padded by 16 B so that the 16-byte reads of a quarter
-// warp fall into distinct banks) = 36 KB per CTA.  It frees the 16 registers of the operand
-// prefetch and replaces three LDG.256 per addition by six LDS.128.  Selected with
-// D377_MSM_ACC_TMA=1; measured against the register-staged kernel in DESIGN.md 3.4.
-constexpr int kTmaSlot = 144;
-D377_DI uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-D377_DI fq_r fq_lds(uint32_t addr) {
-  fq_r r;
-  asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r.l[0]), "=r"(r.l[1]), "=r"(r.l[2]), "=r"(r.l[3]) : "r"(addr));
-  asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];"
-               : "=r"(r.l[4]), "=r"(r.l[5]), "=r"(r.l[6]), "=r"(r.l[7]) : "r"(addr + 16));
-  return r;
-}
-
-__global__ void __maxnreg__(112)
-k_msm_accumulate_tma(const void* __restrict__ pts_v, const uint32_t* __restrict__ sorted,
-                     const uint32_t* __restrict__ offsets, uint32_t nb, int L,
-                     pt_t* __restrict__ bsum, pt_t* __restrict__ part, int32_t* __restrict__ part_bucket,
-                     int32_t bucket_base) {
-  extern __shared__ __align__(128) uint8_t tma_smem[];
-  const uint8_t* pts = reinterpret_cast<const uint8_t*>(pts_v);
-  constexpr uint32_t kRec = 128u;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  // [stage][thread] slots, then [warp][stage] barriers
-  const uint32_t slot0 = smem_u32(tma_smem) + threadIdx.x * kTmaSlot;
-  const uint32_t slot_stride = blockDim.x * kTmaSlot;
-  const uint32_t bar0 = smem_u32(tma_smem) + 2 * slot_stride + warp * 16;
-  if (lane == 0) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar0));
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar0 + 8));
-  }
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  __syncwarp();
-  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-  const uint32_t total = offsets[nb];
-  const uint64_t lo64 = (uint64_t)t * (uint64_t)L;
-  // every lane of a warp runs the same L iterations (the barrier protocol is warp-wide);
-  // lanes past the end of the list carry no entries
-  const bool live = lo64 < total;
-  const uint32_t lo = live ? (uint32_t)lo64 : 0u;
-  const uint32_t hi = live ? (uint32_t)min((uint64_t)total, lo64 + (uint64_t)L) : 0u;
-  uint32_t b = 0;
-  if (live) {
-    uint32_t z = nb;
-    while (z - b > 1) {
-      uint32_t m = b + ((z - b) >> 1);
-      if (offsets[m] <= lo) b = m; else z = m;
-    }
-  }
-  bool starts_here = live && offsets[b] >= lo;
-  uint32_t next = live ? offsets[b + 1] : 0u;
-  pt_t acc = pt_identity();
-  uint32_t e_next = live ? sorted[lo] : 0u;
-  uint32_t e_next2 = lo + 1 < hi ? sorted[lo + 1] : 0u;
-  // issue the copy of entry `e` into stage `st` (warp-wide: arm, then every lane with an entry copies)
-  auto issue = [&](uint32_t e, bool has, int st) {
-    const uint32_t nact = __popc(__ballot_sync(0xffffffffu, has));
-    if (nact == 0) return false;
-    const uint32_t bar = bar0 + 8 * st;
-    if (lane == 0)
-      asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(nact * kRec) : "memory");
-    __syncwarp();
-    if (has) {
-      const uint8_t* src = pts + (size_t)(e & 0x7fffffffu) * kRec;
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                   ::"r"(slot0 + st * slot_stride), "l"(src), "r"(kRec), "r"(bar) : "memory");
-    }
-    return true;
-  };
-  uint32_t phase0 = 0, phase1 = 0;
-  bool armed = issue(e_next, lo < hi, 0);
-#pragma unroll 1
-  for (int it = 0; it < L; it++) {
-    const uint32_t pos = lo + (uint32_t)it;
-    const int st = it & 1;
-    const bool valid = pos < hi;
-    const uint32_t e = e_next;
-    e_next = e_next2;
-    if (pos + 2 < hi) e_next2 = sorted[pos + 2];
-    // next entry into the other stage, then wait for this one
-    const bool armed_next = issue(e_next, pos + 1 < hi, st ^ 1);
-    if (!armed) break;   // warp-uniform: no lane has an entry left
-    {
-      const uint32_t bar = bar0 + 8 * st;
-      const uint32_t ph = st ? phase1 : phase0;
-      uint32_t done = 0;
-      while (!done) {
-        asm volatile("{\n\t.reg .pred p;\n\t"
-                     "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-                     "selp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(done) : "r"(bar), "r"(ph) : "memory");
-      }
-      if (st) phase1 ^= 1u; else phase0 ^= 1u;
-    }
-    armed = armed_next;
-    if (valid) {
-      const uint32_t slot = slot0 + st * slot_stride;
-      const uint32_t o = (e >> 31) ? 32u : 0u;
-      const fq_r ymx = fq_lds(slot + o), ypx = fq_lds(slot + (32u - o)), kt = fq_lds(slot + 64u + o);
-      acc = pt_add_affine<true>(acc, ymx, ypx, kt);
-      const bool bucket_ends = (pos + 1 == next);
-      if (bucket_ends || pos + 1 == hi) {
-        uint32_t tt = blockIdx.x * blockDim.x + threadIdx.x;
-        asm volatile("" : "+r"(tt));
-        if (starts_here && bucket_ends) {
-          ptv_store(bsum + b, acc);
-        } else if (!starts_here) {
-          ptv_store(part + 2 * (size_t)tt, acc);
-          part_bucket[2 * (size_t)tt] = bucket_base + (int32_t)b;
-        } else {
-          ptv_store(part + 2 * (size_t)tt + 1, acc);
-          part_bucket[2 * (size_t)tt + 1] = bucket_base + (int32_t)b;
-        }
-        acc = pt_identity();
-        if (bucket_ends && pos + 1 < hi) {
-          do {
-            b++;
-            next = offsets[b + 1];
-          } while (next <= pos + 1);
-          starts_here = true;
-        }
-      }
-    }
-  }
-}
-
 // ---- 6. stitch buckets that straddle accumulation ranges -------------------
 // `keys`/`pts` is a list of slots, each either empty (key < 0) or a partial sum
 // of bucket `key`; all pieces of one bucket are consecutive non-empty slots.
@@ -698,6 +590,8 @@ k_msm_accumulate_tma(const void* __restrict__ pts_v, const uint32_t* __restrict_
 // distribution is.
 constexpr int kSegG = 32;
 constexpr int kSegLook = 64;
+// stitch levels of at most this many slots use the warp-scan kernel below
+constexpr size_t kStitchWarpSlots = (size_t)1 << 18;
 
 __global__ void __launch_bounds__(kBlk)
 k_msm_seg_reduce(const int32_t* __restrict__ keys, const pt_t* __restrict__ pts, size_t nslots,
@@ -1186,12 +1080,11 @@ static int msm_state_init(Engine& e) {
   // The tail kernels are short and latency-bound; at the greatest priority their CTAs take
   // the first slots that the long accumulation CTAs of the next MSM vacate instead of
   // queueing behind them.
-  D377_CUDA(cudaStreamCreateWithPriority(&ms.tail_stream, cudaStreamNonBlocking,
-                                         e.tune_tail_prio ? greatest : least));
+  D377_CUDA(cudaStreamCreateWithPriority(&ms.tail_stream, cudaStreamNonBlocking, greatest));
   // (Measured back to back, greatest against least priority: 2.73 / 3.04 ms at 2^20,
   // 7.9 / 8.2 ms at 2^22, 27.5 / 29.6 ms at 2^24 with the single-group sort prefetch.)
-  D377_CUDA(cudaStreamCreateWithPriority(&ms.points_stream, cudaStreamNonBlocking,
-                                         e.tune_points_prio ? greatest : least));
+  // the points stream at the least priority: see pts_prefetch in msm_once
+  D377_CUDA(cudaStreamCreateWithPriority(&ms.points_stream, cudaStreamNonBlocking, least));
   for (int k = 0; k < 2; k++) D377_CUDA(cudaEventCreateWithFlags(&ms.ev_points_done[k], cudaEventDisableTiming));
   D377_CUDA(cudaEventCreateWithFlags(&ms.ev_fork, cudaEventDisableTiming));
   D377_CUDA(cudaEventCreateWithFlags(&ms.ev_acc_done, cudaEventDisableTiming));
@@ -1213,7 +1106,7 @@ static int msm_state_init(Engine& e) {
 // The stream on which MSM results become complete.  Whoever asks is about to enqueue work
 // there, so the engine stream has to be ordered behind it at the next join.
 cudaStream_t result_stream(Engine& e) {
-  if (!e.tune_tail_overlap || msm_state_init(e) != D377_OK) return e.stream;
+  if (!e.msm_tail_overlap_override || msm_state_init(e) != D377_OK) return e.stream;
   e.msm.tail_pending = true;
   return e.msm.tail_stream;
 }
@@ -1291,20 +1184,8 @@ int msm_bases_prepare(const uint8_t* points, int point_format, size_t n, uint8_t
   if (point_format == D377_PT_ELEMENT || point_format == D377_PT_XYZ) {
     int rc = ensure(e.scratch, n * 32);
     if (rc) return rc;
-    size_t per = n >> 17;
-    per = per < 1 ? 1 : per;
-    size_t T = ((n + per - 1) / per + kNormBlk - 1) / kNormBlk * kNormBlk;
-    T = std::min(T, (size_t)e.sm_count * 3 * kNormBlk);
-    if (point_format == D377_PT_ELEMENT)
-      k_msm_normalize<128><<<(unsigned)(T / kNormBlk), kNormBlk, 0, e.stream>>>(points, n, T, (uint8_t*)e.scratch.p, aff, e.tune_gcd_inv != 0);
-    else
-      k_msm_normalize<96><<<(unsigned)(T / kNormBlk), kNormBlk, 0, e.stream>>>(points, n, T, (uint8_t*)e.scratch.p, aff, e.tune_gcd_inv != 0);
-  } else if (point_format == D377_PT_AFFINE) {
-    k_msm_points_affine<D377_PT_AFFINE><<<grid_for(n, kBlk), kBlk, 0, e.stream>>>(points, n, aff, dflags);
-  } else {
-    k_msm_points_affine<D377_PT_ENCODING><<<grid_for(n, kBlk), kBlk, ISQRT_SMEM_WORDS(kBlk) * 4, e.stream>>>(points, n, aff, dflags);
   }
-  D377_LAUNCHED();
+  launch_points_affine(e, point_format, points, n, 1, (uint8_t*)e.scratch.p, aff, dflags, e.stream);
   D377_CUDA(cudaGetLastError());
   D377_CUDA(cudaMemcpyAsync(hflags, dflags, 4, cudaMemcpyDeviceToHost, e.stream));
   D377_CUDA(cudaStreamSynchronize(e.stream));
@@ -1322,16 +1203,13 @@ int msm_bases_fill_windows(uint8_t* table, size_t n, int c, int W) {
   if (rc) return rc;
   uint8_t* run = nullptr;
   D377_CUDA(cudaMalloc(&run, n * 128));
-  size_t per = n >> 17;
-  per = per < 1 ? 1 : per;
-  size_t T = ((n + per - 1) / per + kNormBlk - 1) / kNormBlk * kNormBlk;
-  T = std::min(T, (size_t)e.sm_count * 3 * kNormBlk);
+  const size_t T = normalize_threads(n, 1, e.sm_count);
   cudaError_t ce = cudaSuccess;
   for (int j = 1; j < W && ce == cudaSuccess; j++) {
     k_msm_bases_double<<<grid_for(n, kBlk), kBlk, 0, e.stream>>>(run, j == 1 ? (const aff4_t*)table : nullptr, n, c);
     D377_LAUNCHED();
     k_msm_normalize<128><<<(unsigned)(T / kNormBlk), kNormBlk, 0, e.stream>>>(
-        run, n, T, (uint8_t*)e.scratch.p, table + (size_t)j * n * 128, e.tune_gcd_inv != 0);
+        run, n, T, (uint8_t*)e.scratch.p, table + (size_t)j * n * 128);
     D377_LAUNCHED();
     ce = cudaGetLastError();
   }
@@ -1363,6 +1241,29 @@ int msm_windowed_c(size_t n) {
     if (cost < best) { best = cost; best_c = c; }
   }
   return best_c;
+}
+
+// Window groups of an MSM over W windows: wlo[k] .. whi[k] are the windows of the k-th group
+// processed, taken from the top down.  Group sizes in processing order, weights 2, 3, 4, ...:
+// the first sort has only the point conversion to hide under, every later one the
+// accumulation of the group before it.
+static void group_windows(int W, int ngroups, int* wlo, int* whi) {
+  int wsum = 0, acc = 0, cut[kMaxGroups + 1];
+  // three groups: 2 : 5 : 7 (measured: the first sort then ends with the normalisation
+  // and every later one just before the accumulation that waits for it)
+  auto weight = [&](int k) { return ngroups == 3 ? (k == 0 ? 2 : k == 1 ? 5 : 7) : k + 2; };
+  for (int k = 0; k < ngroups; k++) wsum += weight(k);
+  cut[0] = 0;
+  for (int k = 0; k < ngroups; k++) {
+    acc += weight(k);
+    cut[k + 1] = std::max(cut[k] + 1, (int)((long long)acc * W / wsum));
+  }
+  cut[ngroups] = W;
+  for (int k = ngroups - 1; k > 0; k--) cut[k] = std::min(cut[k], cut[k + 1] - 1);
+  for (int k = 0; k < ngroups; k++) {
+    whi[k] = W - cut[k];
+    wlo[k] = W - cut[k + 1];
+  }
 }
 
 // One Pippenger.  Head (point conversion, sort, bucket accumulation) on the engine and sort
@@ -1406,8 +1307,7 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   // Run length per accumulate thread.  Every run boundary splits a bucket into pieces
   // that k_msm_seg_reduce has to stitch (one extra addition each), so runs are as long
   // as the thread count allows: >= ~2 full waves of 128-thread CTAs on 148 SMs.
-  int L = max_entries >= ((size_t)1 << 27) ? 128 : max_entries >= ((size_t)1 << 25) ? 64 : 32;
-  if (e.tune_acc_run > 0) L = e.tune_acc_run;
+  const int L = max_entries >= ((size_t)1 << 27) ? 128 : max_entries >= ((size_t)1 << 25) ? 64 : 32;
   if (max_entries >= 0xfffffff0ull) { set_error("msm chunk too large"); return D377_ERR_INVALID_ARG; }
   // Buckets per bucket-reduce thread.  With the weighted tree (k_wsum_tree) a segment
   // costs no scalar multiplication, so segments can be short: many threads, short
@@ -1416,11 +1316,8 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   // more than their latency: longer segments (fewer doublings and tree nodes) win once a
   // window has many buckets -- measured back to back: 2^22 7.64 / 7.49 / 7.42 ms and 2^24
   // 27.08 / 26.97 / 27.00 ms with 16 / 32 / 64, 2^20 (c = 16) 2.43 / 2.48 / 2.64 ms.
-  uint32_t Lseg = g.c >= 18 ? 64 : g.c == 17 ? 32 : 16;
-  if (e.tune_reduce_seg > 0) Lseg = (uint32_t)e.tune_reduce_seg;
-  int log_lseg = 0;
-  while ((2u << log_lseg) <= Lseg) log_lseg++;
-  Lseg = 1u << log_lseg;   // power of two: P_s = Lseg * R_s by doublings
+  const int log_lseg = g.c >= 18 ? 6 : g.c == 17 ? 5 : 4;
+  const uint32_t Lseg = 1u << log_lseg;   // power of two: P_s = Lseg * R_s by doublings
   const uint32_t S = (g.K + Lseg - 1) / Lseg;
 
   // Window groups: group k+1 is sorted (sort stream) while group k is accumulated (engine
@@ -1435,50 +1332,14 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   // When this MSM's sort can run under the accumulation of the MSM before it (its scalars
   // are ready and that accumulation is still in flight), there is nothing left for window
   // groups to hide: one group, a third of the launches (2^24 back to back: 28.14 -> 27.76 ms).
-  const bool may_prefetch = scalars_ready != nullptr && e.tune_tail_overlap && e.tune_sort_prefetch;
+  const bool may_prefetch = scalars_ready != nullptr && e.msm_tail_overlap_override;
   if (may_prefetch && ms.tail_used[0] && cudaEventQuery(ms.ev_acc_done) == cudaErrorNotReady) ngroups = 1;
   cudaGetLastError();
-  if (e.tune_groups > 0) ngroups = std::min(std::min(e.tune_groups, kMaxGroups), g.W);
-  // Group sizes in processing order, weights 2, 3, 4, ...: the first sort has only the
-  // point conversion to hide under, every later one the accumulation of the group before
-  // it.  wlo[k] .. whi[k] are the windows of the k-th group processed.
+  if (e.msm_groups_override > 0) ngroups = std::min(std::min(e.msm_groups_override, kMaxGroups), g.W);
   int wlo[kMaxGroups], whi[kMaxGroups];
-  {
-    int wsum = 0, acc = 0, cut[kMaxGroups + 1];
-    // three groups: 2 : 5 : 7 (measured: the first sort then ends with the normalisation
-    // and every later one just before the accumulation that waits for it)
-    auto weight = [&](int k) { return ngroups == 3 ? (k == 0 ? 2 : k == 1 ? 5 : 7) : k + 2; };
-    for (int k = 0; k < ngroups; k++) wsum += weight(k);
-    cut[0] = 0;
-    for (int k = 0; k < ngroups; k++) {
-      acc += weight(k);
-      cut[k + 1] = std::max(cut[k] + 1, (int)((long long)acc * g.W / wsum));
-    }
-    cut[ngroups] = g.W;
-    for (int k = ngroups - 1; k > 0; k--) cut[k] = std::min(cut[k], cut[k + 1] - 1);
-    // D377_MSM_GW="3,8,3": explicit group sizes in processing order (experiments)
-    if (const char* gwenv = getenv("D377_MSM_GW")) {
-      int sz[kMaxGroups], ng = 0, tot = 0;
-      for (const char* q = gwenv; *q && ng < kMaxGroups;) {
-        sz[ng] = atoi(q);
-        tot += sz[ng++];
-        while (*q && *q != ',') q++;
-        if (*q == ',') q++;
-      }
-      if (tot == g.W) {
-        ngroups = ng;
-        cut[0] = 0;
-        for (int k = 0; k < ng; k++) cut[k + 1] = cut[k] + sz[k];
-      }
-    }
-    for (int k = 0; k < ngroups; k++) {
-      whi[k] = g.W - cut[k];
-      wlo[k] = g.W - cut[k + 1];
-    }
-  }
+  group_windows(g.W, ngroups, wlo, whi);
   // sort kernels beside a resident accumulation: one 256-thread CTA per SM
-  const unsigned sort_cap = ngroups > 1 || may_prefetch
-                                ? (unsigned)e.sm_count * (unsigned)std::max(1, e.tune_sort_ctas) : 0u;
+  const unsigned sort_cap = ngroups > 1 || may_prefetch ? (unsigned)e.sm_count : 0u;
   auto capped = [&](size_t want) { return (unsigned)(sort_cap ? std::min<size_t>(want, sort_cap) : want); };
   // Buckets of group k: one set per window, or one merged set (windowed bases).  g_bucket[k]
   // is the group's first bucket in `bsum`; rg is the geometry the bucket reduction sees (a
@@ -1505,21 +1366,10 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   // multiplications saved).
   const bool projective = point_format == D377_PT_ELEMENT || point_format == D377_PT_XYZ;
   const bool prepared = point_format == D377_PT_BASES;   // `points` already holds the bucket operands
-  bool affine = !projective;
-  size_t norm_per = 0, norm_T = 0;
-  if (projective) {
-    norm_per = n >> 17;                       // >= 2^17 threads stay busy
-    if (norm_per > 64) norm_per = 64;
-    int want = e.tune_normalize;              // D377_MSM_NORMALIZE: -1 off, 1 force, 0 auto
-    if (want > 0 && norm_per < 4) norm_per = 4;
-    if (want >= 0 && norm_per >= (size_t)e.tune_norm_min_per) affine = true;
-    if (want > 0) affine = true;
-    if (affine) norm_T = ((n + norm_per - 1) / norm_per + kNormBlk - 1) / kNormBlk * kNormBlk;
-    // One wave: every CTA is resident from the start (3 per SM at 70 registers), so the
-    // kernel has no ragged last wave and the CTA-wide inversion bubble occurs once.
-    if (affine && e.tune_norm_wave > 0)
-      norm_T = std::min(norm_T, (size_t)e.sm_count * (size_t)e.tune_norm_wave * kNormBlk);
-  }
+  // d377_msm_set_normalize: -1 never, 1 always (at least 4 points per thread), 0 from 2^20 pairs
+  const int want_normalize = e.msm_normalize_override;
+  const bool normalize = projective && (want_normalize > 0 || (want_normalize == 0 && (n >> 17) >= 8));
+  const bool affine = !projective || normalize;
 
   // ---- workspaces -----------------------------------------------------------------
   // Two complete sets (bucket operands, digits, sorted lists, offsets, bucket sums, piece
@@ -1530,13 +1380,13 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   // The other set is only needed while the previous MSM is still in flight: a caller that
   // waits for every result (d377_msm_dev, d377_msm) keeps using set 0 and pays for one.
   int set = 0;
-  if (e.tune_tail_overlap && ms.tail_used[ms.cur_set] &&
+  if (e.msm_tail_overlap_override && ms.tail_used[ms.cur_set] &&
       cudaEventQuery(ms.ev_tail_done[ms.cur_set]) == cudaErrorNotReady)
     set = ms.cur_set ^ 1;
   cudaGetLastError();
   ms.cur_set = set;
   size_t o_cached = carve(prepared ? 0 : n * sizeof(cached_t));
-  size_t o_norm = carve(affine && norm_T ? n * 32 : 0);
+  size_t o_norm = carve(normalize ? n * 32 : 0);
   size_t o_dig = carve(max_entries * 4);
   size_t o_sorted = carve(max_entries * 4);
   size_t o_sc = carve(sc_mont ? n * 32 : 0);
@@ -1585,10 +1435,9 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   // like the accumulation it runs under, so only its bubbles are hidden: ~1 % from 2^21 pairs
   // on one GPU.  In the 8-GPU strong-scaling loop (2^21 pairs per GPU, an all-gather per
   // step) it costs 4 % instead (4.28 -> 4.45 ms), so it is used from 2^22 pairs.
-  const bool pts_prefetch = may_prefetch && e.tune_points_prefetch && !prepared &&
-                            n >= ((size_t)1 << 22);
+  const bool pts_prefetch = may_prefetch && !prepared && n >= ((size_t)1 << 22);
   cudaStream_t ps = pts_prefetch ? ms.points_stream : st;
-  cudaStream_t ts = e.tune_tail_overlap ? ms.tail_stream : e.stream;
+  cudaStream_t ts = e.msm_tail_overlap_override ? ms.tail_stream : e.stream;
 
   ms.last_geom.c = g.c;
   ms.last_geom.W = g.W;
@@ -1656,20 +1505,15 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   D377_CUDA(cudaMemsetAsync(pb, 0xff, 2 * nthreads * 4, st));
   // 1
   if (!prepared) {
-    dim3 gr(grid_for(n, kBlk));
-    if (point_format == D377_PT_ELEMENT && affine)
-      k_msm_normalize<128><<<(unsigned)(norm_T / kNormBlk), kNormBlk, 0, ps>>>(points, n, norm_T, ws + o_norm, aff, e.tune_gcd_inv != 0);
-    else if (point_format == D377_PT_XYZ && affine)
-      k_msm_normalize<96><<<(unsigned)(norm_T / kNormBlk), kNormBlk, 0, ps>>>(points, n, norm_T, ws + o_norm, aff, e.tune_gcd_inv != 0);
-    else if (point_format == D377_PT_ELEMENT)
-      k_msm_points<D377_PT_ELEMENT><<<gr, kBlk, 0, ps>>>(points, n, cached, flags);
-    else if (point_format == D377_PT_XYZ)
-      k_msm_points<D377_PT_XYZ><<<gr, kBlk, 0, ps>>>(points, n, cached, flags);
-    else if (point_format == D377_PT_AFFINE)
-      k_msm_points_affine<D377_PT_AFFINE><<<gr, kBlk, 0, ps>>>(points, n, aff, flags);
-    else
-      k_msm_points_affine<D377_PT_ENCODING><<<gr, kBlk, ISQRT_SMEM_WORDS(kBlk) * 4, ps>>>(points, n, aff, flags);
-    D377_LAUNCHED();
+    if (affine) {
+      launch_points_affine(e, point_format, points, n, want_normalize > 0 ? 4 : 1, ws + o_norm, aff, flags, ps);
+    } else {
+      if (point_format == D377_PT_ELEMENT)
+        k_msm_points<D377_PT_ELEMENT><<<grid_for(n, kBlk), kBlk, 0, ps>>>(points, n, cached, flags);
+      else
+        k_msm_points<D377_PT_XYZ><<<grid_for(n, kBlk), kBlk, 0, ps>>>(points, n, cached, flags);
+      D377_LAUNCHED();
+    }
     if (pts_prefetch) {
       D377_CUDA(cudaEventRecord(ms.ev_points_done[set], ps));
       D377_CUDA(cudaStreamWaitEvent(st, ms.ev_points_done[set], 0));
@@ -1685,11 +1529,7 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
     const uint32_t* counts = (const uint32_t*)(tw + o_counts[k]);
     D377_CUDA(cudaStreamWaitEvent(st, ms.ev_sorted[k], 0));
     D377_CUDA(cudaEventRecord(ms.ev_acc0[k], st));
-    if (affine && e.tune_acc_tma)
-      k_msm_accumulate_tma<<<grid_for(g_nthreads[k], kBlk), kBlk, 2 * kBlk * kTmaSlot + (kBlk / 32) * 16, st>>>(
-          aff_in, sorted + (size_t)wa * n, counts, (uint32_t)nbk, L, bsum + b0,
-          part + 2 * g_tbase[k], pb + 2 * g_tbase[k], (int32_t)b0);
-    else if (affine)
+    if (affine)
       k_msm_accumulate<true><<<grid_for(g_nthreads[k], kBlk), kBlk, 0, st>>>(
           aff_in, sorted + (size_t)wa * n, counts, (uint32_t)nbk, L, bsum + b0,
           part + 2 * g_tbase[k], pb + 2 * g_tbase[k], (int32_t)b0);
@@ -1717,7 +1557,7 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
       int32_t* kout = kbuf[lvl & 1];
       pt_t* pout = pbuf[lvl & 1];
       // work-efficient serial fold while the level is large, warp scan (log depth) below
-      if (e.tune_stitch_warp && nslots <= (size_t)e.tune_stitch_warp)
+      if (nslots <= kStitchWarpSlots)
         k_msm_seg_reduce_warp<<<grid_for(nt * 32, kBlk), kBlk, 0, ts>>>(kin, pin, nslots, bsum, kout, pout, nt);
       else
         k_msm_seg_reduce<<<grid_for(nt, kBlk), kBlk, 0, ts>>>(kin, pin, nslots, bsum, kout, pout, nt);

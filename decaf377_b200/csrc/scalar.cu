@@ -2,8 +2,6 @@
 // fixed-base GENERATOR * s over GPU-built window tables (normalize_batch lives with the
 // MSM normalisation kernel in msm.cu).  Own translation unit so that the
 // heavy kernels of the library compile in parallel.
-#include <cstdlib>
-
 #include "engine.h"
 #include "point.cuh"
 
@@ -323,19 +321,11 @@ void launch_scalar_mul(int point_format, bool encode, const uint8_t* points, con
   // CTA size / residency at 2^16 elements (configuration 1: 512 CTAs of 128 threads are 0.86 of
   // one wave, 68 SMs hold four CTAs and 80 hold three).  Smaller CTAs, with or without a
   // shared-memory request that caps the CTAs per SM at an even 14 warps, do not pay
-  // (tools/sm_block_sweep.sh, D377_SM_BLOCK / D377_SM_SMEM): 20.5 Melem/s with 128 threads,
-  // 20.3 with 96, 20.3 / 20.2 with 64, 20.2 with 32 -- the kernel is bound by each thread's
-  // dependent chain, not by the warps an SM holds.
-  unsigned block = (unsigned)kCodecBlock;
-  size_t sm = codec_smem();
-  {
-    static const int xb = getenv("D377_SM_BLOCK") ? atoi(getenv("D377_SM_BLOCK")) : 0;
-    static const int xs = getenv("D377_SM_SMEM") ? atoi(getenv("D377_SM_SMEM")) : 0;
-    if (xb) { block = (unsigned)xb; sm = ISQRT_SMEM_WORDS(block) * sizeof(uint32_t); }
-    if (xs && (size_t)xs > sm) sm = (size_t)xs;
-  }
-  dim3 g(grid_for(n, block));
-#define SM_LAUNCH(F, E) k_scalar_mul<F, E><<<g, block, sm, st>>>(points, scalars, n, out, ok)
+  // (profiles/r2_scalar_mul_cta_sweep.txt): 20.5 Melem/s with 128 threads, 20.3 with 96,
+  // 20.3 / 20.2 with 64, 20.2 with 32 -- the kernel is bound by each thread's dependent chain,
+  // not by the warps an SM holds.
+  dim3 g(grid_for(n, kCodecBlock));
+#define SM_LAUNCH(F, E) k_scalar_mul<F, E><<<g, kCodecBlock, codec_smem(), st>>>(points, scalars, n, out, ok)
   switch (point_format) {
     case D377_PT_ELEMENT: if (encode) SM_LAUNCH(D377_PT_ELEMENT, true); else SM_LAUNCH(D377_PT_ELEMENT, false); break;
     case D377_PT_ENCODING: if (encode) SM_LAUNCH(D377_PT_ENCODING, true); else SM_LAUNCH(D377_PT_ENCODING, false); break;

@@ -581,35 +581,6 @@ def test_small_fixed_base_call_does_not_build_the_quartic_table():
     assert grew2 > 1500, "the large call should have built the 1.6 GB quartic table (%d MiB)" % grew2
 
 
-# ---- the TMA-staged operand stream (experiment kept behind D377_MSM_ACC_TMA) ---------------------
-_TMA = r"""
-import sys, numpy as np
-sys.path.insert(0, %r)
-import decaf377_b200 as d
-from oracle import c_oracle as co
-from oracle import decaf377_ref as o
-d.init(0)
-for n in (1, 33, 4097, 1 << 17):
-    raw = np.frombuffer(o.xof_bytes("tma_fq/%%d" %% n, n), np.uint8).reshape(n, 32).copy()
-    sc = np.frombuffer(o.xof_bytes("tma_sc/%%d" %% n, n), np.uint8).reshape(n, 32).copy()
-    sc[:, 31] &= 3
-    el = d.batch_encode_to_curve(raw, d.OUT_ELEMENT)
-    d.msm_set_normalize(1)          # affine bucket operands: the path the TMA kernel serves
-    got = d.vartime_multiscalar_mul(sc, el)[1].tobytes()
-    want = co.msm_pippenger(sc, el, threads=8)[1].tobytes()
-    assert got == want, n
-print("TMA_OK")
-"""
-
-
-def test_tma_staged_accumulation_is_bit_exact():
-    """k_msm_accumulate_tma (cp.async.bulk per record + one mbarrier per warp and stage) gives the
-    results of the register-staged kernel; it is slower (DESIGN.md 3.4) and therefore off by default."""
-    env = dict(os.environ, D377_MSM_ACC_TMA="1")
-    r = subprocess.run([sys.executable, "-c", _TMA % ROOT], capture_output=True, text=True, timeout=900, env=env)
-    assert r.returncode == 0 and "TMA_OK" in r.stdout, r.stdout + r.stderr
-
-
 # ---- the boundary from a non-Python host ---------------------------------------------------------
 def test_c_host_program_drives_the_abi(tmp_path):
     """tests/abi_smoke.c is compiled with gcc against include/decaf377_b200.h and linked with
@@ -635,7 +606,7 @@ def test_parity_suite_under_the_on_curve_debug_build():
     r = subprocess.run([sys.executable, "-m", "pytest", "-x", "-q", "-m", "gpu", "-p", "no:cacheprovider",
                         os.path.join(ROOT, "tests", "test_gpu_parity.py"),
                         os.path.join(ROOT, "tests", "test_gpu_round2.py"),
-                        "-k", "not debug_build and not c_host and not quartic_table and not tma_staged"],
+                        "-k", "not debug_build and not c_host and not quartic_table"],
                        capture_output=True, text=True, timeout=3000, env=env, cwd=ROOT)
     assert r.returncode == 0, r.stdout[-4000:] + r.stderr[-2000:]
     line = [ln for ln in r.stdout.splitlines() if ln.startswith("D377_DEBUG ")]

@@ -1,8 +1,7 @@
 #!/usr/bin/env python3
 """Wave-quantisation probe of the one-element-per-thread kernels (developer tool):
 decompress -> mul -> compress and compress at batch sizes around whole waves of
-148 SMs x 4 CTAs x 128 threads = 75 776 elements.  D377_CODEC_BLOCK picks the CTA size."""
-import os
+148 SMs x 4 CTAs x 128 threads = 75 776 elements."""
 import sys
 
 import torch
@@ -23,5 +22,5 @@ for n in (1 << 16, wave, wave + 128, 2 * wave, 1 << 18, 3 * wave, 4 * wave, 1 <<
     enc = dev.compress(el)
     ms1 = timeit(lambda: dev.scalar_mul(enc, sc, d.PT_ENCODING, d.OUT_ENCODING), iters=3)
     ms2 = timeit(lambda: dev.compress(el), iters=10)
-    print("block=%s n=%7d (%.3f waves): pipeline %.3f ms %.2f Melem/s   compress %.4f ms %.1f Melem/s" % (
-        os.environ.get("D377_CODEC_BLOCK", "auto"), n, n / wave, ms1, n / ms1 / 1e3, ms2, n / ms2 / 1e3), flush=True)
+    print("n=%7d (%.3f waves): pipeline %.3f ms %.2f Melem/s   compress %.4f ms %.1f Melem/s" % (
+        n, n / wave, ms1, n / ms1 / 1e3, ms2, n / ms2 / 1e3), flush=True)

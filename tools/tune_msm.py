@@ -1,6 +1,5 @@
 #!/usr/bin/env python3
-"""MSM stage timings (developer tool): python tools/tune_msm.py LOGN [c ...]
-Reads D377_ACC_RUN / D377_REDUCE_SEG from the environment (engine init)."""
+"""MSM stage timings (developer tool): python tools/tune_msm.py LOGN [c ...]"""
 import os
 import sys
 
@@ -39,9 +38,8 @@ for c in cs:
     t1.synchronize()
     ms = t0.elapsed_time(t1) / iters
     info = d.msm_stage_info()
-    print("n=2^%d c=%d W=%d run=%s seg=%s: %.3f ms  %.1f Mpt/s  %s" % (
-        logn, info["c"], info["W"], os.environ.get("D377_ACC_RUN", "auto"),
-        os.environ.get("D377_REDUCE_SEG", "auto"), ms, n / ms / 1e3,
+    print("n=2^%d c=%d W=%d: %.3f ms  %.1f Mpt/s  %s" % (
+        logn, info["c"], info["W"], ms, n / ms / 1e3,
         " ".join("%s=%.3f" % (k, v) for k, v in info["ms"].items())), flush=True)
     if os.environ.get("D377_TIMELINE"):
         for k, g in enumerate(d.msm_timeline()):
