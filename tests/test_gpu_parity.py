@@ -165,20 +165,33 @@ def test_encode_and_hash_to_curve(engine):
             assert henc[i].tobytes() == o.compress(o.hash_to_curve(x1, x2)), i
 
 
-def test_elligator_den_zero_is_identity(engine):
-    # SURVEY appendix B: d*r = d - a  or (d-a)*r = d  ->  identity
-    cases = []
-    for target in ((o.COEFF_D - o.COEFF_A) * pow(o.COEFF_D, -1, Q) % Q,
-                   o.COEFF_D * pow(o.COEFF_D - o.COEFF_A, -1, Q) % Q):
-        r0sq = target * pow(o.ZETA, -1, Q) % Q
-        ok, root = o.sqrt_ratio_zeta(r0sq, 1)
-        if ok:
-            cases.append(root)
-    if not cases:
-        pytest.skip("no such r0 in Fq")
-    enc = engine.batch_encode_to_curve(canon(cases), engine.OUT_ENCODING)
-    for i, c in enumerate(cases):
-        assert enc[i].tobytes() == o.compress(o.encode_to_curve(c)) == bytes(32)
+def test_elligator_zero_input_among_neighbours(engine):
+    """r0 = 0 is the Elligator input with a degenerate Jacobi-quartic pair, (s, t) = (0, -1),
+    so 1 / (s t) = 0 in k_elligator_encode's CTA-wide inversion; (0, 0) takes k_hash_encode's
+    generic fallback after the warp-wide inversion.  Planted at lanes 0, 15 and 31 of the last
+    warp of a CTA, across the first warp of the next, over one whole CTA and at both ends of
+    the batch (the padding lanes re-read index 0), between random inputs: every element is
+    the oracle's, the zero lanes and their good neighbours alike.  (The Elligator denominator
+    itself never vanishes: tests/test_jacobi_shortcuts_cpu.py.)"""
+    from oracle import c_oracle as co
+    n = 5 * 128 + 77
+    rng = np.random.default_rng(168)
+    r1 = rng.integers(0, 256, (n, 32), dtype=np.uint8)
+    r2 = rng.integers(0, 256, (n, 32), dtype=np.uint8)
+    zero = [0, 224, 239, 255] + list(range(256, 288)) + list(range(384, 512)) + [n - 1]
+    r1[zero] = 0
+    r2[zero] = 0
+    r2[[100, 600]] = 0                           # (x, 0): one degenerate map in the sum
+    r1[[101, 601]] = 0                           # (0, x)
+    enc = engine.batch_encode_to_curve(r1, engine.OUT_ENCODING)
+    henc = engine.batch_hash_to_curve(r1, r2, engine.OUT_ENCODING)
+    want = co.encode_to_curve(r1, out_enc=True, threads=4)
+    hwant = co.hash_to_curve(r1, r2, out_enc=True, threads=4)
+    for i in range(n):
+        assert enc[i].tobytes() == want[i].tobytes(), i
+        assert henc[i].tobytes() == hwant[i].tobytes(), i
+    assert want[0].tobytes() == o.compress(o.encode_to_curve(0)) == bytes(32)
+    assert hwant[0].tobytes() == o.compress(o.hash_to_curve(0, 0)) == bytes(32)
 
 
 # ---- group ops (rows a11, a12, a16) -------------------------------------------------

@@ -75,6 +75,18 @@ def test_elligator_pair_lies_on_the_quartic_and_maps_to_the_point():
         assert (X, Z) == (2 * s * t % Q, (1 - s * s) * t % Q)
 
 
+def test_elligator_denominator_never_vanishes():
+    """den = (d r - (d - a)) ((d - a) r - d), r = zeta r0^2, is zero only where zeta r0^2 is
+    (d - a) / d or d / (d - a).  Both targets are squares and zeta is not, so target / zeta
+    has no root in Fq: no r0 reaches a zero denominator.  The degenerate Jacobi-quartic pair
+    the kernels do meet is the one of r0 = 0, (s, t) = (0, -1)."""
+    for target in ((D - A) * inv(D) % Q, D * inv(D - A) % Q):
+        r0sq = target * inv(o.ZETA) % Q
+        assert pow(r0sq, (Q - 1) // 2, Q) == Q - 1           # Euler: not a square
+        assert o.sqrt_ratio_zeta(r0sq, 1)[0] is False
+    assert elligator_st(0) == (0, Q - 1)
+
+
 def test_encoding_of_elligator_output_is_abs_s_or_abs_inverse_s():
     """compress(encode_to_curve(r0)) = |s| if 2s/t is non-negative else |1/s|."""
     rnd = random.Random(2)
