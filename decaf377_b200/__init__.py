@@ -16,7 +16,7 @@ from .api import (  # noqa: F401
     batch_decompress, batch_compress, batch_compress_fmt, batch_affine_serialize, batch_affine_deserialize,
     batch_encode_to_curve, batch_hash_to_curve,
     batch_scalar_mul, fixed_base_mul, batch_add, batch_element_eq, element_sum,
-    vartime_multiscalar_mul, msm_submit, msm_wait, MsmBases, fq_batch_op, fq_batch_isqrt,
+    vartime_multiscalar_mul, msm_submit, msm_wait, MsmBases, FixedBases, fq_batch_op, fq_batch_isqrt,
     fq_batch_sqrt_ratio_zeta, field_batch_deserialize, batch_normalize, FIELD_FQ, FIELD_FR,
     PT_ELEMENT, PT_ENCODING, PT_AFFINE, PT_XYZ, PT_BASES, OUT_ELEMENT, OUT_ENCODING, SCALARS_MONTGOMERY,
 )

@@ -23,7 +23,7 @@ ERR_INVALID_ENCODING = -5
 
 PT_ELEMENT, PT_ENCODING, PT_AFFINE, PT_XYZ, PT_BASES = 0, 1, 2, 3, 4
 OUT_ELEMENT, OUT_ENCODING = 0, 1
-SCALARS_MONTGOMERY = 0x100   # OR into point_format (out_format for fixed_base_mul)
+SCALARS_MONTGOMERY = 0x100   # OR into point_format (out_format for fixed_base_mul / fixed_bases_mul)
 
 u8p = C.c_void_p
 _SIGS = {
@@ -77,6 +77,10 @@ _SIGS = {
     "d377_msm_bases_info": [C.c_void_p, C.POINTER(C.c_size_t), C.POINTER(C.c_int), C.POINTER(C.c_int),
                             C.POINTER(C.c_size_t)],
     "d377_msm_last_windowed": [C.POINTER(C.c_int)],
+    "d377_fixed_bases_create": [u8p, C.c_int, C.c_size_t, C.POINTER(C.c_void_p)],
+    "d377_fixed_bases_info": [C.c_void_p, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)],
+    "d377_fixed_bases_destroy": [C.c_void_p],
+    "d377_fixed_bases_mul": [C.c_void_p, u8p, C.c_size_t, u8p, C.c_int],
     "d377_msm_wait": [C.c_int, u8p, u8p],
     "d377_fq_batch_op": [C.c_int, u8p, u8p, C.c_size_t, u8p],
     "d377_fq_batch_isqrt": [u8p, C.c_size_t, u8p, u8p],
@@ -97,6 +101,7 @@ for _n in ["d377_batch_decompress", "d377_batch_compress", "d377_batch_encode_to
            "d377_batch_add", "d377_batch_element_eq", "d377_element_sum", "d377_msm",
            "d377_fq_batch_isqrt", "d377_fq_batch_sqrt_ratio_zeta", "d377_field_batch_deserialize",
            "d377_batch_normalize", "d377_msm_bases_create", "d377_msm_bases_create_windowed",
+           "d377_fixed_bases_create", "d377_fixed_bases_mul",
            "d377_batch_encode_to_curve_wide",
            "d377_batch_hash_to_curve_wide", "d377_fq_batch_from_le_bytes_mod_order",
            "d377_batch_sub", "d377_batch_neg", "d377_batch_double", "d377_batch_on_curve",

@@ -494,6 +494,72 @@ def _bases_ptr(b: "MsmBases"):
     return C.c_void_p(b.ptr)
 
 
+class FixedBases:
+    """Prepared fixed bases (d377_fixed_bases_create): window tables of k caller-chosen points
+    B_0..B_{k-1}, 48 MiB of device memory per base, built once.  ``mul(scalars)`` then computes
+    out[i] = sum_j scalars[i, j] * B_j for every row -- with k = 1, fixed-base multiplication by
+    an arbitrary point; with k = 2, e.g. Pedersen commitments v * G_a + r * H.  ``points``: k
+    inputs in `point_format` (host memory), or ``device_ptr`` / ``k`` for device memory.
+    ``.k``, ``.nbytes`` and ``len()`` describe the set; ``close()`` releases it."""
+
+    def __init__(self, points=None, point_format: int = PT_ELEMENT, *, device_ptr: int = 0, k: int = 0):
+        _ensure_init()
+        lib = _lib.load()
+        out = C.c_void_p(0)
+        if points is not None:
+            pts = _arr(points, _PT_WIDTH[point_format], "points")
+            k = pts.shape[0]
+            check(lib.d377_fixed_bases_create(_ptr(pts), point_format, k, C.byref(out)))
+        else:
+            check(lib.d377_fixed_bases_create_dev(C.c_void_p(device_ptr), point_format, int(k), C.byref(out)))
+        self.ptr = out.value or 0
+        kk, nb = C.c_size_t(0), C.c_size_t(0)
+        check(lib.d377_fixed_bases_info(C.c_void_p(self.ptr), C.byref(kk), C.byref(nb)))
+        self.k = int(kk.value)
+        self.nbytes = int(nb.value)
+
+    def _handle(self):
+        if not self.ptr:
+            raise ValueError("FixedBases has been closed")
+        return C.c_void_p(self.ptr)
+
+    def _scalars(self, scalars) -> np.ndarray:
+        """`scalars` as the [n, k, 32] uint8 array mul() passes on; [n, 32] is accepted for k = 1."""
+        sc = np.ascontiguousarray(scalars, dtype=np.uint8)
+        if sc.ndim == 2 and self.k == 1 and sc.shape[1] == 32:
+            sc = sc.reshape(-1, 1, 32)
+        if sc.ndim != 3 or sc.shape[1:] != (self.k, 32):
+            raise ValueError("scalars must have shape [n, %d, 32]%s, got %r"
+                             % (self.k, " or [n, 32]" if self.k == 1 else "", sc.shape))
+        return sc
+
+    def mul(self, scalars, out_format: int = OUT_ELEMENT, out: Optional[np.ndarray] = None,
+            scalars_montgomery: bool = False) -> np.ndarray:
+        """out[i] = sum_j scalars[i, j] * B_j -> [n, 128] Elements or [n, 32] encodings.  Each
+        scalar is any 256-bit little-endian integer; `scalars_montgomery`: the in-memory
+        Montgomery limbs of the reference's Fr (D377_SCALARS_MONTGOMERY)."""
+        sc = self._scalars(scalars)
+        n = sc.shape[0]
+        out = _out(out, (n, _OUT_WIDTH[out_format]))
+        check(_lib.load().d377_fixed_bases_mul(self._handle(), _ptr(sc), n, _ptr(out),
+                                               out_format | _mont(scalars_montgomery)))
+        return out
+
+    def close(self) -> None:
+        if self.ptr:
+            check(_lib.load().d377_fixed_bases_destroy(C.c_void_p(self.ptr)))
+            self.ptr = 0
+
+    def __len__(self) -> int:
+        return self.k
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 def vartime_multiscalar_mul(scalars, points, point_format: int = PT_ELEMENT,
                             scalars_montgomery: bool = False) -> Tuple[np.ndarray, np.ndarray]:
     """Element::vartime_multiscalar_mul: returns (element [128], encoding [32]).

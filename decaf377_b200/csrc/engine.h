@@ -43,6 +43,12 @@ struct BasesLayout {
   size_t bytes = 0;
 };
 
+// A set of prepared fixed bases (d377_fixed_bases_create*): k window tables back to back.
+struct FixedBasesInfo {
+  size_t k = 0;
+  size_t bytes = 0;
+};
+
 // Per-device state of the Pippenger pipeline (msm.cu).
 struct MsmState {
   bool ready = false;
@@ -123,6 +129,8 @@ struct Engine {
   DevBuf st_in[2][3], st_out[2][2];
   // prepared MSM bases handed out by d377_msm_bases_create*: device pointer -> layout
   std::unordered_map<const void*, BasesLayout> bases;
+  // prepared fixed bases handed out by d377_fixed_bases_create*: device pointer -> {k, bytes}
+  std::unordered_map<const void*, FixedBasesInfo> fixed_bases;
   // asynchronous MSMs (d377_msm_dev_async): sticky status word, reported by d377_sync
   bool async_status_dirty = false;
   MsmState msm;
@@ -227,8 +235,10 @@ void launch_scalar_mul(int point_format, bool encode, const uint8_t* points, con
                        size_t n, uint8_t* out, uint8_t* ok, cudaStream_t st);
 int ensure_fb_table();
 int ensure_fb_table_jq();
-void launch_fixed_base(bool encode, const void* table, const void* table_jq, const uint8_t* scalars,
+void launch_fixed_base(bool encode, const void* table, size_t k, const void* table_jq, const uint8_t* scalars,
                        size_t n, uint8_t* out, cudaStream_t st);
+size_t fixed_bases_bytes_per_base();
+int fixed_bases_fill(const uint8_t* points, int point_format, size_t k, void* table);
 
 // msm.cu
 void launch_seg_sum(const uint8_t* prods, const uint8_t* okp, const uint32_t* offs, size_t nseg,

@@ -318,6 +318,8 @@ static void engine_destroy(Engine& e) {
   // prepared bases still alive belong to the library (header contract): release them
   for (auto& kv : e.bases) cudaFree(const_cast<void*>(kv.first));
   e.bases.clear();
+  for (auto& kv : e.fixed_bases) cudaFree(const_cast<void*>(kv.first));
+  e.fixed_bases.clear();
   if (e.fb_table) cudaFree(e.fb_table);
   e.fb_table = nullptr;
   if (e.fb_table_jq) cudaFree(e.fb_table_jq);
@@ -742,8 +744,45 @@ int d377_fixed_base_mul_dev(const uint8_t* scalars, size_t n, uint8_t* out, int 
     cudaGetLastError();
     quartic = false;
   }
-  launch_fixed_base(out_format == D377_OUT_ENCODING, e.fb_table, quartic ? e.fb_table_jq : nullptr, scalars, n,
+  launch_fixed_base(out_format == D377_OUT_ENCODING, e.fb_table, 1, quartic ? e.fb_table_jq : nullptr, scalars, n,
                     out, e.stream);
+  D377_LAUNCHED();
+  D377_CUDA(cudaGetLastError());
+  return D377_OK;
+}
+
+// a live set of fixed bases of this engine -> its k
+static int fixed_bases_k(Engine& e, const uint8_t* tables, const char* who, size_t* k) {
+  auto it = e.fixed_bases.find(tables);
+  if (it == e.fixed_bases.end()) {
+    set_error("%s: %p is not a live set of fixed bases of device %d", who, (const void*)tables, e.device);
+    return D377_ERR_INVALID_ARG;
+  }
+  *k = it->second.k;
+  return D377_OK;
+}
+
+// n rows of k 32-byte scalars must stay addressable
+static int fixed_bases_rows(size_t n, size_t k) {
+  if (n > SIZE_MAX / 32 / k) {
+    set_error("fixed bases: %zu rows of %zu scalars overflow the address space", n, k);
+    return D377_ERR_INVALID_ARG;
+  }
+  return D377_OK;
+}
+
+int d377_fixed_bases_mul_dev(const uint8_t* tables, const uint8_t* scalars, size_t n, uint8_t* out, int out_format) {
+  D377_REQUIRE_READY();
+  const bool sc_mont = take_sc_mont(out_format);
+  if (!check_fmt(out_format)) { set_error("bad out_format %d", out_format); return D377_ERR_INVALID_ARG; }
+  Engine& e = _eng;
+  size_t k = 0;
+  TRY(fixed_bases_k(e, tables, "d377_fixed_bases_mul_dev", &k));
+  if (n == 0) return D377_OK;
+  if (!scalars || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
+  TRY(fixed_bases_rows(n, k));
+  if (sc_mont) TRY(canonical_scalars(e, scalars, n * k));
+  launch_fixed_base(out_format == D377_OUT_ENCODING, tables, k, nullptr, scalars, n, out, e.stream);
   D377_LAUNCHED();
   D377_CUDA(cudaGetLastError());
   return D377_OK;
@@ -1167,6 +1206,23 @@ int d377_fixed_base_mul(const uint8_t* scalars, size_t n, uint8_t* out, int out_
   return rc;
 }
 
+int d377_fixed_bases_mul(const uint8_t* tables, const uint8_t* scalars, size_t n, uint8_t* out, int out_format) {
+  D377_REQUIRE_READY();
+  const int fmt_word = out_format;
+  take_sc_mont(out_format);
+  if (!check_fmt(out_format)) { set_error("bad out_format %d", out_format); return D377_ERR_INVALID_ARG; }
+  size_t k = 0;
+  TRY(fixed_bases_k(_eng, tables, "d377_fixed_bases_mul", &k));
+  if (n == 0) return D377_OK;
+  if (!scalars || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
+  TRY(fixed_bases_rows(n, k));
+  HostIn ins[] = {{scalars, 32 * k}};
+  HostOut outs[] = {{out, out_bytes(out_format)}};
+  return run_pipelined(n, ins, 1, outs, 1, [&](uint8_t* const* di, uint8_t* const* dout, size_t len) {
+    return d377_fixed_bases_mul_dev(tables, di[0], len, dout[0], fmt_word);
+  });
+}
+
 static int binop_host(int op, const uint8_t* a, const uint8_t* b, size_t n, uint8_t* out) {
   D377_REQUIRE_READY();
   if (n == 0) return D377_OK;
@@ -1351,6 +1407,94 @@ int d377_msm_bases_destroy(uint8_t* bases) {
   D377_CUDA(cudaStreamSynchronize(e.stream));
   e.bases.erase(it);
   D377_CUDA(cudaFree(bases));
+  return D377_OK;
+}
+
+// ---- prepared fixed bases ----------------------------------------------------
+// Arguments of d377_fixed_bases_create*, checked before anything is allocated or read;
+// *bytes receives the size of the k tables.
+static int fixed_bases_args(int point_format, size_t k, uint8_t** tables, const uint8_t* points, size_t* bytes) {
+  if (point_format < 0 || point_format > 3) { set_error("bad point_format %d", point_format); return D377_ERR_INVALID_ARG; }
+  if (!tables || !points) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
+  if (k == 0) { set_error("fixed bases: k = 0"); return D377_ERR_INVALID_ARG; }
+  const size_t per = fixed_bases_bytes_per_base();
+  if (k > SIZE_MAX / per) {
+    set_error("fixed bases: %zu tables of %zu bytes overflow the address space", k, per);
+    return D377_ERR_INVALID_ARG;
+  }
+  *bytes = k * per;
+  return D377_OK;
+}
+
+// `host`: `points` is host memory, uploaded once the tables are allocated
+static int fixed_bases_create(const uint8_t* points, int point_format, size_t k, uint8_t** tables, bool host) {
+  Engine& e = engine();
+  size_t bytes = 0;
+  TRY(fixed_bases_args(point_format, k, tables, points, &bytes));
+  uint8_t* tab = nullptr;
+  cudaError_t ce = cudaMalloc(&tab, bytes);
+  if (ce != cudaSuccess) {
+    cudaGetLastError();
+    set_error("fixed bases: cannot allocate %zu bytes of device memory (%s)", bytes, cudaGetErrorString(ce));
+    return D377_ERR_CUDA;
+  }
+  int rc = D377_OK;
+  uint8_t* tmp = nullptr;
+  if (host) {
+    ce = cudaMalloc(&tmp, k * pt_bytes(point_format));
+    if (ce == cudaSuccess)
+      ce = cudaMemcpyAsync(tmp, points, k * pt_bytes(point_format), cudaMemcpyHostToDevice, e.stream);
+    if (ce != cudaSuccess) rc = cuda_fail(ce, "upload of the fixed bases", __FILE__, __LINE__);
+  }
+  if (!rc) rc = fixed_bases_fill(host ? tmp : points, point_format, k, tab);   // synchronises the stream
+  if (rc) cudaStreamSynchronize(e.stream);
+  if (tmp) cudaFree(tmp);
+  if (rc) {
+    cudaFree(tab);
+    return rc;
+  }
+  FixedBasesInfo info;
+  info.k = k;
+  info.bytes = bytes;
+  e.fixed_bases[tab] = info;
+  *tables = tab;
+  return D377_OK;
+}
+
+int d377_fixed_bases_create(const uint8_t* points, int point_format, size_t k, uint8_t** tables) {
+  D377_REQUIRE_READY();
+  return fixed_bases_create(points, point_format, k, tables, true);
+}
+
+int d377_fixed_bases_create_dev(const uint8_t* points, int point_format, size_t k, uint8_t** tables) {
+  D377_REQUIRE_READY();
+  return fixed_bases_create(points, point_format, k, tables, false);
+}
+
+int d377_fixed_bases_info(const uint8_t* tables, size_t* k, size_t* bytes) {
+  D377_REQUIRE_READY_NOJOIN();
+  auto it = _eng.fixed_bases.find(tables);
+  if (it == _eng.fixed_bases.end()) {
+    set_error("d377_fixed_bases_info: %p is not a live set of fixed bases of device %d", (const void*)tables, _eng.device);
+    return D377_ERR_INVALID_ARG;
+  }
+  if (k) *k = it->second.k;
+  if (bytes) *bytes = it->second.bytes;
+  return D377_OK;
+}
+
+int d377_fixed_bases_destroy(uint8_t* tables) {
+  if (!tables) return D377_OK;
+  D377_REQUIRE_READY();
+  Engine& e = _eng;
+  auto it = e.fixed_bases.find(tables);
+  if (it == e.fixed_bases.end()) {
+    set_error("d377_fixed_bases_destroy: %p is not a live set of fixed bases of device %d", (void*)tables, e.device);
+    return D377_ERR_INVALID_ARG;
+  }
+  D377_CUDA(cudaStreamSynchronize(e.stream));
+  e.fixed_bases.erase(it);
+  D377_CUDA(cudaFree(tables));
   return D377_OK;
 }
 

@@ -1,6 +1,6 @@
 // Scalar-multiplication kernels, one element per thread: variable-base &Element * &Fr,
-// fixed-base GENERATOR * s over GPU-built window tables (normalize_batch lives with the
-// MSM normalisation kernel in msm.cu).  Own translation unit so that the
+// fixed-base GENERATOR * s and sum_j s_j * B_j over GPU-built window tables (normalize_batch
+// lives with the MSM normalisation kernel in msm.cu).  Own translation unit so that the
 // heavy kernels of the library compile in parallel.
 #include "engine.h"
 #include "point.cuh"
@@ -44,31 +44,82 @@ k_scalar_mul(const uint8_t* __restrict__ pts, const uint8_t* __restrict__ scalar
 }
 
 // ---- fixed-base tables ------------------------------------------------------
-// T[w][j] = (j+1) * 2^(16 w) * G in cached affine form, w < 16, j < 2^15, followed by one
-// extra entry 2^256 * G: the carry out of the top window of a scalar >= 2^255 (never a
-// canonical Fr, but the entry points accept any 256-bit string).
+// Table of a base B: T[w][j] = (j+1) * 2^(16 w) * B in cached affine form, w < 16, j < 2^15,
+// followed by one extra entry 2^256 * B: the carry out of the top window of a scalar >= 2^255
+// (never a canonical Fr, but the entry points accept any 256-bit string).  A set of k bases
+// (d377_fixed_bases_create*) holds k such tables back to back, kFbStride records apart; the
+// generator's table is the set {G}.
 constexpr int kFbC = 16;
 constexpr int kFbW = 16;
 constexpr int kFbK = 1 << (kFbC - 1);
+constexpr size_t kFbStride = (size_t)kFbW * kFbK + 1;
 
-__global__ void k_fb_bases(pt_t* bases) {
+size_t fixed_bases_bytes_per_base() { return kFbStride * sizeof(niels_t); }
+
+// Element::GENERATOR, the starting point of the generator's table
+__global__ void k_fb_generator(pt_t* start) {
   pt_t p;
   p.x = fq_const(FQ_BX);
   p.y = fq_const(FQ_BY);
   p.z = fq_one();
   p.t = fq_const(FQ_BT);
+  start[0] = p;
+}
+
+// The caller's bases in point_format 0..3 -> extended points, one thread per base.  An
+// invalid encoding sets bit 0 of *flags (the base then reads as the identity).
+template <int kFmt>
+__global__ void __launch_bounds__(kCodecBlock)
+k_fb_load(const uint8_t* __restrict__ pts, size_t k, pt_t* __restrict__ start, uint32_t* __restrict__ flags) {
+  extern __shared__ uint32_t smem[];
+  size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= k) return;
+  pt_t p;
+  if (kFmt == D377_PT_ELEMENT) {
+    p = pt_load_wire(pts + 128 * j);
+  } else if (kFmt == D377_PT_AFFINE) {
+    p.x = fq_load_wire(pts + 64 * j);
+    p.y = fq_load_wire(pts + 64 * j + 32);
+    p.z = fq_one();
+    p.t = fq_mul(p.x, p.y);
+  } else if (kFmt == D377_PT_XYZ) {
+    // (X : Y : Z) without T: (XZ : YZ : Z^2 : XY) is the same point in extended coordinates
+    fq_t x = fq_load_wire(pts + 96 * j), y = fq_load_wire(pts + 96 * j + 32), z = fq_load_wire(pts + 96 * j + 64);
+    p.x = fq_mul(x, z);
+    p.y = fq_mul(y, z);
+    p.z = fq_sqr(z);
+    p.t = fq_mul(x, y);
+  } else {
+    bool good = pt_decompress(p, fq_load_raw(pts + 32 * j), isqrt_smem(smem));
+    if (!good) {
+      atomicOr(flags, 1u);
+      p = pt_identity();
+    }
+  }
+  D377_DBG_POINT(p);
+  start[j] = p;
+}
+
+// 2^(16 w) * B_j for w <= kFbW, one thread per base: bases[j * (kFbW + 1) + w]
+__global__ void k_fb_bases(const pt_t* __restrict__ start, size_t k, pt_t* __restrict__ bases) {
+  size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= k) return;
+  pt_t p = start[j];
   for (int w = 0; w <= kFbW; w++) {
-    bases[w] = p;
-    for (int k = 0; k < kFbC; k++) p = pt_dbl(p);
+    bases[j * (kFbW + 1) + w] = p;
+    for (int c = 0; c < kFbC; c++) p = pt_dbl(p);
   }
 }
 
-__global__ void k_fb_fill(const pt_t* __restrict__ bases, niels_t* __restrict__ table) {
+// All k tables in one launch; the entries are normalised affine, so a table depends on its
+// base only, not on the representative it was built from.
+__global__ void k_fb_fill(const pt_t* __restrict__ bases, size_t k, niels_t* __restrict__ table) {
   size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx > (size_t)kFbW * kFbK) return;   // the last index is the carry entry 1 * bases[kFbW]
-  int w = (int)(idx / kFbK);
-  uint32_t m = (uint32_t)(idx % kFbK) + 1;
-  pt_t base = bases[w];
+  if (idx >= k * kFbStride) return;
+  size_t j = idx / kFbStride, r = idx % kFbStride;   // r = kFbW * kFbK: the carry entry 1 * bases[kFbW]
+  int w = (int)(r / kFbK);
+  uint32_t m = (uint32_t)(r % kFbK) + 1;
+  pt_t base = bases[j * (kFbW + 1) + w];
   pt_t acc = pt_identity();
 #pragma unroll 1
   for (int i = kFbC - 1; i >= 0; i--) {
@@ -88,9 +139,8 @@ D377_DI niels_t niels_load(const niels_t* p) {
   return n;
 }
 
-// Element::GENERATOR * s with signed 16-bit windows over the table above.
-D377_DI pt_t fixed_base_edwards(const niels_t* __restrict__ table, const fq_raw_t& k) {
-  pt_t acc = pt_identity();
+// acc + s * B with signed 16-bit windows over the table of B.
+D377_DI pt_t fixed_base_edwards(const niels_t* __restrict__ table, const fq_raw_t& k, pt_t acc) {
   uint32_t carry = 0;
 #pragma unroll 1
   for (int w = 0; w < kFbW; w++) {
@@ -108,14 +158,19 @@ D377_DI pt_t fixed_base_edwards(const niels_t* __restrict__ table, const fq_raw_
   return acc;
 }
 
+// out[i] = sum_j s_ij * B_j over the k tables of a set, ONE accumulator through all of them:
+// 16 k mixed additions per row.  The generator is the set {G} (k = 1).
 template <bool kEncode>
 __global__ void __launch_bounds__(kCodecBlock)
-k_fixed_base(const niels_t* __restrict__ table, const uint8_t* __restrict__ scalars, size_t n,
+k_fixed_base(const niels_t* __restrict__ tables, size_t k, const uint8_t* __restrict__ scalars, size_t n,
              uint8_t* __restrict__ out) {
   extern __shared__ uint32_t smem[];
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  pt_t acc = fixed_base_edwards(table, fq_load_raw(scalars + 32 * i));
+  pt_t acc = pt_identity();
+#pragma unroll 1
+  for (size_t j = 0; j < k; j++)
+    acc = fixed_base_edwards(tables + j * kFbStride, fq_load_raw(scalars + 32 * (i * k + j)), acc);
   D377_DBG_POINT(acc);
   if (kEncode) {
     isqrt_smem_t sm = isqrt_smem(smem);
@@ -157,7 +212,7 @@ D377_DI fq_r fq_load_canon(const void* p) { return fq_assume<1000>(fq_load(p)); 
 
 __device__ __noinline__ fq_r fixed_base_generic_encoding(const niels_t* __restrict__ table,
                                                          const fq_raw_t& k, isqrt_smem_t sm) {
-  return pt_compress_to_field(fixed_base_edwards(table, k), sm);
+  return pt_compress_to_field(fixed_base_edwards(table, k, pt_identity()), sm);
 }
 
 // Every thread computes kPer elements before the CTA inverts once (Montgomery's trick per
@@ -279,21 +334,64 @@ __global__ void k_jq_fill(const fq_t* __restrict__ bases, jq_rec_t* __restrict__
   fq_store(rec + 96, fq_reduce(fq_neg(s)));
 }
 
+// k_fb_bases + k_fb_fill for the k start points at work[0, k); work[k, k + k (kFbW + 1)) holds
+// the window bases
+static void fb_build(pt_t* work, size_t k, niels_t* table, cudaStream_t st) {
+  k_fb_bases<<<grid_for(k, 32), 32, 0, st>>>(work, k, work + k);
+  D377_LAUNCHED();
+  k_fb_fill<<<grid_for(k * kFbStride, 128), 128, 0, st>>>(work + k, k, table);
+  D377_LAUNCHED();
+}
+
 int ensure_fb_table() {
   Engine& e = engine();
   if (e.fb_table) return D377_OK;
-  pt_t* bases = nullptr;
+  pt_t* work = nullptr;
   niels_t* table = nullptr;
-  D377_CUDA(cudaMalloc(&bases, sizeof(pt_t) * (kFbW + 1)));
-  D377_CUDA(cudaMalloc(&table, sizeof(niels_t) * ((size_t)kFbW * kFbK + 1)));
-  k_fb_bases<<<1, 1, 0, e.stream>>>(bases);
+  D377_CUDA(cudaMalloc(&work, sizeof(pt_t) * (kFbW + 2)));
+  D377_CUDA(cudaMalloc(&table, sizeof(niels_t) * kFbStride));
+  k_fb_generator<<<1, 1, 0, e.stream>>>(work);
   D377_LAUNCHED();
-  k_fb_fill<<<grid_for((size_t)kFbW * kFbK + 1, 128), 128, 0, e.stream>>>(bases, table);
-  D377_LAUNCHED();
+  fb_build(work, 1, table, e.stream);
   D377_CUDA(cudaGetLastError());
   D377_CUDA(cudaStreamSynchronize(e.stream));
-  D377_CUDA(cudaFree(bases));
+  D377_CUDA(cudaFree(work));
   e.fb_table = table;
+  return D377_OK;
+}
+
+// The tables of k caller-chosen bases (device memory, point_format 0..3) into `table`
+// (k * fixed_bases_bytes_per_base() bytes).  Synchronises the engine stream.
+int fixed_bases_fill(const uint8_t* points, int point_format, size_t k, void* table) {
+  Engine& e = engine();
+  uint32_t* dflags = (uint32_t*)(e.d_small + kSmallFlags);
+  uint32_t* hflags = (uint32_t*)(e.h_small + kSmallFlags);
+  pt_t* work = nullptr;
+  D377_CUDA(cudaMalloc(&work, sizeof(pt_t) * k * (kFbW + 2)));
+  cudaError_t ce = cudaMemsetAsync(dflags, 0, 4, e.stream);
+  if (ce == cudaSuccess) {
+    dim3 g(grid_for(k, kCodecBlock));
+    switch (point_format) {
+      case D377_PT_ELEMENT: k_fb_load<D377_PT_ELEMENT><<<g, kCodecBlock, 0, e.stream>>>(points, k, work, dflags); break;
+      case D377_PT_ENCODING:
+        k_fb_load<D377_PT_ENCODING><<<g, kCodecBlock, codec_smem(), e.stream>>>(points, k, work, dflags);
+        break;
+      case D377_PT_AFFINE: k_fb_load<D377_PT_AFFINE><<<g, kCodecBlock, 0, e.stream>>>(points, k, work, dflags); break;
+      default: k_fb_load<D377_PT_XYZ><<<g, kCodecBlock, 0, e.stream>>>(points, k, work, dflags); break;
+    }
+    D377_LAUNCHED();
+    fb_build(work, k, (niels_t*)table, e.stream);
+    ce = cudaGetLastError();
+  }
+  if (ce == cudaSuccess) ce = cudaMemcpyAsync(hflags, dflags, 4, cudaMemcpyDeviceToHost, e.stream);
+  cudaError_t se = cudaStreamSynchronize(e.stream);
+  if (ce == cudaSuccess) ce = se;
+  cudaFree(work);
+  if (ce != cudaSuccess) return cuda_fail(ce, "fixed bases: table build", __FILE__, __LINE__);
+  if (*hflags & 1u) {
+    set_error("fixed bases: a base is not a valid encoding");
+    return D377_ERR_INVALID_ENCODING;
+  }
   return D377_OK;
 }
 
@@ -334,7 +432,9 @@ void launch_scalar_mul(int point_format, bool encode, const uint8_t* points, con
 #undef SM_LAUNCH
 }
 
-void launch_fixed_base(bool encode, const void* table, const void* table_jq, const uint8_t* scalars,
+// table: a set of k tables (k = 1 for the generator); table_jq: the generator's quartic table
+// (only with k = 1), or null
+void launch_fixed_base(bool encode, const void* table, size_t k, const void* table_jq, const uint8_t* scalars,
                        size_t n, uint8_t* out, cudaStream_t st) {
   dim3 g(grid_for(n, kCodecBlock));
   const niels_t* tab = (const niels_t*)table;
@@ -350,8 +450,8 @@ void launch_fixed_base(bool encode, const void* table, const void* table_jq, con
     else
       k_fixed_base_jq<1><<<grid_for(n, kCodecBlock), kCodecBlock, codec_smem(), st>>>(jt, tab, scalars, n, out);
   }
-  else if (encode) k_fixed_base<true><<<g, kCodecBlock, codec_smem(), st>>>(tab, scalars, n, out);
-  else k_fixed_base<false><<<g, kCodecBlock, codec_smem(), st>>>(tab, scalars, n, out);
+  else if (encode) k_fixed_base<true><<<g, kCodecBlock, codec_smem(), st>>>(tab, k, scalars, n, out);
+  else k_fixed_base<false><<<g, kCodecBlock, codec_smem(), st>>>(tab, k, scalars, n, out);
 }
 
 D377_DBG_READER(scalar_debug_counts)

@@ -12,7 +12,7 @@ from typing import Optional, Tuple
 import torch
 
 from . import _lib, api
-from ._lib import OUT_ELEMENT, OUT_ENCODING, PT_ELEMENT, check
+from ._lib import OUT_ELEMENT, OUT_ENCODING, PT_ELEMENT, SCALARS_MONTGOMERY, check
 
 _ext_streams = {}
 
@@ -154,6 +154,27 @@ def fixed_base_mul(scalars: torch.Tensor, out_format: int = OUT_ELEMENT,
                       device=scalars.device) if out is None else out
     _after_torch()
     check(_lib.load().d377_fixed_base_mul_dev(scalars.data_ptr(), n, out.data_ptr(), out_format))
+    _then_torch()
+    return out
+
+
+def fixed_bases_mul(bases, scalars: torch.Tensor, out_format: int = OUT_ELEMENT,
+                    out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """d377_fixed_bases_mul_dev: out[i] = sum_j scalars[i, j] * B_j over an api.FixedBases set;
+    `scalars` is a contiguous CUDA uint8 tensor of shape [n, k, 32] ([n, 32] for k = 1);
+    OR SCALARS_MONTGOMERY into `out_format` for in-memory Fr limbs."""
+    if not (scalars.is_cuda and scalars.dtype == torch.uint8 and scalars.is_contiguous()):
+        raise ValueError("scalars must be a contiguous CUDA uint8 tensor")
+    if scalars.dim() == 2 and bases.k == 1 and scalars.shape[1] == 32:
+        n = scalars.shape[0]
+    elif scalars.dim() == 3 and tuple(scalars.shape[1:]) == (bases.k, 32):
+        n = scalars.shape[0]
+    else:
+        raise ValueError("scalars must have shape [n, %d, 32], got %r" % (bases.k, tuple(scalars.shape)))
+    width = 32 if (out_format & ~SCALARS_MONTGOMERY) == OUT_ENCODING else 128
+    out = torch.empty((n, width), dtype=torch.uint8, device=scalars.device) if out is None else out
+    _after_torch()
+    check(_lib.load().d377_fixed_bases_mul_dev(bases._handle(), scalars.data_ptr(), n, out.data_ptr(), out_format))
     _then_torch()
     return out
 

@@ -73,9 +73,9 @@ extern "C" {
  * (fields/fr/u64/wrapper.rs, fr/u32/wrapper.rs: x * 2^256 mod r), and Fr::to_bytes /
  * into_bigint costs a Montgomery reduction per scalar on the host -- more host time for
  * 2^24 scalars than the whole MSM takes on the GPU.  OR this flag into `point_format`
- * (d377_msm*, d377_batch_scalar_mul*) or into `out_format` (d377_fixed_base_mul*) and pass
- * the 32 bytes of the in-memory limbs instead: the conversion (Fr::into_bigint,
- * fields/fr/arkworks.rs:36-57) then runs on the GPU.  Every 256-bit string is a valid
+ * (d377_msm*, d377_batch_scalar_mul*) or into `out_format` (d377_fixed_base_mul*,
+ * d377_fixed_bases_mul*) and pass the 32 bytes of the in-memory limbs instead: the
+ * conversion (Fr::into_bigint, fields/fr/arkworks.rs:36-57) then runs on the GPU.  Every 256-bit string is a valid
  * Montgomery representative, so D377_ERR_SCALAR_RANGE cannot occur with it. */
 #define D377_SCALARS_MONTGOMERY 0x100
 
@@ -203,6 +203,35 @@ int d377_batch_scalar_mul_dev(const uint8_t* points, int point_format, const uin
  * smaller batches take the Edwards table + compress.  Both paths give the same bytes. */
 int d377_fixed_base_mul(const uint8_t* scalars, size_t n, uint8_t* out, int out_format);
 int d377_fixed_base_mul_dev(const uint8_t* scalars, size_t n, uint8_t* out, int out_format);
+
+/* ---- fixed-base multiplication over caller-chosen bases --------------------
+ * Prepared fixed bases: window tables of k caller-chosen points B_0..B_{k-1}, the geometry
+ * of the generator table (16 signed 16-bit windows, 2^15 cached affine multiples each, plus
+ * the 2^256 * B_j carry entry): (16 * 2^15 + 1) * 96 B = 48 MiB per base.  points: k inputs in
+ * point_format 0..3 (host memory; device memory for _dev).  An invalid encoding fails with
+ * D377_ERR_INVALID_ENCODING.  A table that cannot be allocated fails with D377_ERR_CUDA and
+ * d377_last_error names the byte count before any input is read; k = 0, a null pointer, a
+ * bad format and a k whose byte count overflows give D377_ERR_INVALID_ARG.  No failure leaves
+ * anything registered.  The handle is a device pointer owned by the library until
+ * d377_fixed_bases_destroy or d377_shutdown, and it is valid on the device it was created on
+ * (it is NOT a D377_PT_BASES handle of d377_msm*).  The creating call blocks. */
+int d377_fixed_bases_create(const uint8_t* points, int point_format, size_t k, uint8_t** tables);
+int d377_fixed_bases_create_dev(const uint8_t* points, int point_format, size_t k, uint8_t** tables);
+/* k and device bytes of a live handle */
+int d377_fixed_bases_info(const uint8_t* tables, size_t* k, size_t* bytes);
+/* a handle that is not live (destroyed, never created, of another device) is refused;
+ * NULL is a no-op */
+int d377_fixed_bases_destroy(uint8_t* tables);
+/* out[i] = sum_j scalars[i*k + j] * B_j for i < n: n rows of k 32-byte scalars, each ANY
+ * 256-bit LE integer (as d377_fixed_base_mul); OR D377_SCALARS_MONTGOMERY into out_format
+ * for in-memory Fr limbs.  out: n x 128 B (D377_OUT_ELEMENT) or n x 32 B (D377_OUT_ENCODING).
+ * Every call uses all k bases (a zero scalar adds the identity).  k = 1 is fixed-base
+ * multiplication by an arbitrary point.  One accumulator walks the 16 windows of every base
+ * in turn: 16 k mixed additions per row, plus one compress for encodings.  n = 0 is a no-op;
+ * a handle that is not a live fixed-bases handle of the calling thread's engine is refused
+ * with D377_ERR_INVALID_ARG. */
+int d377_fixed_bases_mul(const uint8_t* tables, const uint8_t* scalars, size_t n, uint8_t* out, int out_format);
+int d377_fixed_bases_mul_dev(const uint8_t* tables, const uint8_t* scalars, size_t n, uint8_t* out, int out_format);
 
 /* ---- Element + Element, PartialEq (ark_curve/ops/projective.rs:5-104,
  *      element/projective.rs:65-70) ------------------------------------- */

@@ -16,6 +16,7 @@
 //! | `Add / Sub / Neg` (ark_curve/ops/projective.rs:5-104), doubling     | `add_batch`, `sub_batch`, `neg_batch`, `double_batch` |
 //! | `Element::vartime_multiscalar_mul` (element/projective.rs:99-117)   | `vartime_multiscalar_mul`, `vartime_multiscalar_mul_multi_gpu`, `vartime_multiscalar_mul_batch` (many small ones) |
 //! | `VariableBaseMSM::msm` over long-lived bases (ark_curve/element.rs:27-37) | `GpuBases::new`, `GpuBases::msm` |
+//! | `B * s` / `sum_j s_j * B_j` for long-lived bases B_j (fixed-base tables) | `GpuFixedBases::new`, `GpuFixedBases::mul`, `GpuFixedBases::mul_compressed` |
 //! | `CurveGroup::normalize_batch` (ark_curve/element.rs:74-81)          | `normalize_batch` |
 //! | `OnCurve::is_on_curve` (ark_curve/on_curve.rs:17-38)                | `is_on_curve_batch` |
 //!
@@ -100,6 +101,9 @@ extern "C" {
                                           bases: *mut *mut u8) -> c_int;
     fn d377_msm_bases_info(bases: *const u8, n: *mut usize, c: *mut c_int, windows: *mut c_int,
                            bytes: *mut usize) -> c_int;
+    fn d377_fixed_bases_create(points: *const u8, point_format: c_int, k: usize, tables: *mut *mut u8) -> c_int;
+    fn d377_fixed_bases_destroy(tables: *mut u8) -> c_int;
+    fn d377_fixed_bases_mul(tables: *const u8, scalars: *const u8, n: usize, out: *mut u8, out_format: c_int) -> c_int;
     fn d377_host_alloc(bytes: usize) -> *mut c_void;
     fn d377_host_free(p: *mut c_void) -> c_int;
 }
@@ -603,6 +607,68 @@ impl Drop for GpuBases {
     }
 }
 
+/// Fixed-base window tables of k long-lived points B_0..B_{k-1} (d377_fixed_bases_create:
+/// 48 MiB of device memory per base).  `mul` computes `sum_j s_ij * B_j` for every row i of
+/// k scalars -- with k = 1 `B * s` for many s, with k = 2 e.g. Pedersen commitments
+/// `v * G_a + r * H` -- at 16 k mixed additions per row instead of k variable-base ladders.
+pub struct GpuFixedBases {
+    ptr: *mut u8,
+    len: usize,
+}
+
+// The handle is an opaque device pointer; the library serialises calls per engine.
+unsafe impl Send for GpuFixedBases {}
+
+impl GpuFixedBases {
+    pub fn new(points: &[Element]) -> Result<Self, GpuError> {
+        let w = elements_to_wire(points);
+        let mut ptr: *mut u8 = core::ptr::null_mut();
+        check(unsafe { d377_fixed_bases_create(w.as_ptr(), PT_ELEMENT, points.len(), &mut ptr) })?;
+        Ok(GpuFixedBases { ptr, len: points.len() })
+    }
+
+    /// k, the number of bases (and of scalars per row).
+    pub fn len(&self) -> usize {
+        self.len
+    }
+
+    pub fn is_empty(&self) -> bool {
+        self.len == 0
+    }
+
+    fn run(&self, scalars: &[Fr], out_format: c_int, width: usize) -> Result<Vec<u8>, GpuError> {
+        assert!(scalars.len() % self.len == 0, "scalars: rows of k = {} scalars", self.len);
+        let n = scalars.len() / self.len;
+        let ws = scalars_to_wire(scalars);
+        let mut out = vec![0u8; width * n];
+        check(unsafe {
+            d377_fixed_bases_mul(self.ptr as *const u8, ws.as_ptr(), n, out.as_mut_ptr(), out_format | SCALARS_MONTGOMERY)
+        })?;
+        Ok(out)
+    }
+
+    /// `sum_j scalars[i * k + j] * B_j` for every row i; `scalars` is row-major, its length a
+    /// multiple of k.
+    pub fn mul(&self, scalars: &[Fr]) -> Result<Vec<Element>, GpuError> {
+        Ok(wire_to_elements(&self.run(scalars, OUT_ELEMENT, 128)?))
+    }
+
+    /// The same, `vartime_compress`ed in the same launch.
+    pub fn mul_compressed(&self, scalars: &[Fr]) -> Result<Vec<Encoding>, GpuError> {
+        Ok(wire_to_encodings(&self.run(scalars, OUT_ENCODING, 32)?))
+    }
+}
+
+impl Drop for GpuFixedBases {
+    fn drop(&mut self) {
+        if !self.ptr.is_null() {
+            // after d377_shutdown the library has released the tables itself
+            let _ = unsafe { d377_fixed_bases_destroy(self.ptr) };
+            self.ptr = core::ptr::null_mut();
+        }
+    }
+}
+
 /// Page-locked staging buffer (`d377_host_alloc`): callers that build the wire images
 /// themselves (e.g. a prover that keeps its scalars in one allocation) get full PCIe speed
 /// and overlapped upload / compute from the host-buffer entry points with it.
@@ -679,6 +745,16 @@ mod tests {
         assert_eq!(bases.msm(&s).unwrap(), msm);
         let win = GpuBases::new_windowed(&p, 0).unwrap();
         assert_eq!(win.msm(&s).unwrap(), msm);
+        // k = 2 fixed bases: rows (s_i, s_{i+1}) against (p_0, p_1)
+        let fb = GpuFixedBases::new(&p[..2]).unwrap();
+        assert_eq!(fb.len(), 2);
+        let lc = fb.mul(&s[..16]).unwrap();
+        let lc_enc = fb.mul_compressed(&s[..16]).unwrap();
+        for i in 0..8 {
+            let want = p[0] * s[2 * i] + p[1] * s[2 * i + 1];
+            assert_eq!(lc[i], want);
+            assert_eq!(lc_enc[i], want.vartime_compress());
+        }
         let g = generator_mul_batch(&s).unwrap();
         for i in 0..s.len() {
             assert_eq!(g[i], Element::GENERATOR * s[i]);
