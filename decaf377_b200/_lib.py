@@ -23,6 +23,8 @@ ERR_INVALID_ENCODING = -5
 
 PT_ELEMENT, PT_ENCODING, PT_AFFINE, PT_XYZ, PT_BASES = 0, 1, 2, 3, 4
 OUT_ELEMENT, OUT_ENCODING = 0, 1
+PT_WIDTH = {PT_ELEMENT: 128, PT_ENCODING: 32, PT_AFFINE: 64, PT_XYZ: 96}   # bytes per point
+OUT_WIDTH = {OUT_ELEMENT: PT_WIDTH[PT_ELEMENT], OUT_ENCODING: PT_WIDTH[PT_ENCODING]}   # bytes per result
 SCALARS_MONTGOMERY = 0x100   # OR into point_format (out_format for fixed_base_mul / fixed_bases_mul)
 
 u8p = C.c_void_p

@@ -17,8 +17,8 @@ from typing import Iterable, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _lib
-from ._lib import (OUT_ELEMENT, OUT_ENCODING, PT_AFFINE, PT_BASES, PT_ELEMENT, PT_ENCODING, PT_XYZ,  # noqa: F401
-                   SCALARS_MONTGOMERY, D377Error, check)
+from ._lib import (OUT_ELEMENT, OUT_ENCODING, OUT_WIDTH, PT_AFFINE, PT_BASES, PT_ELEMENT,  # noqa: F401
+                   PT_ENCODING, PT_WIDTH, PT_XYZ, SCALARS_MONTGOMERY, D377Error, check)
 
 # moduli: src/fields/fq.rs:29-34, src/fields/fr.rs:29-34
 Q_MODULUS = 0x12AB655E9A2CA55660B44D1E5C37B00159AA76FED00000010A11800000000001
@@ -230,12 +230,8 @@ def _out(out: Optional[np.ndarray], shape, name: str = "out") -> np.ndarray:
     return out
 
 
-_PT_WIDTH = {PT_ELEMENT: 128, PT_ENCODING: 32, PT_AFFINE: 64, PT_XYZ: 96}
-
-
 def _mont(flag: bool) -> int:
     return SCALARS_MONTGOMERY if flag else 0
-_OUT_WIDTH = {OUT_ELEMENT: 128, OUT_ENCODING: 32}
 
 
 # ---------------------------------------------------------------------------
@@ -282,7 +278,7 @@ def batch_compress_fmt(points, point_format: int, out: Optional[np.ndarray] = No
     _ensure_init()
     if point_format not in (PT_ELEMENT, PT_AFFINE, PT_XYZ):
         raise ValueError("point_format must be PT_ELEMENT, PT_AFFINE or PT_XYZ")
-    pts = _arr(points, _PT_WIDTH[point_format], "points")
+    pts = _arr(points, PT_WIDTH[point_format], "points")
     n = pts.shape[0]
     out = _out(out, (n, 32))
     check(_lib.load().d377_batch_compress_fmt(_ptr(pts), point_format, n, _ptr(out)))
@@ -310,7 +306,7 @@ def batch_encode_to_curve(r, out_format: int = OUT_ELEMENT, out: Optional[np.nda
     _ensure_init()
     r = _wide(r, "r")
     n, w = r.shape
-    out = _out(out, (n, _OUT_WIDTH[out_format]))
+    out = _out(out, (n, OUT_WIDTH[out_format]))
     check(_lib.load().d377_batch_encode_to_curve_wide(_ptr(r), w, n, _ptr(out), out_format))
     return out
 
@@ -323,7 +319,7 @@ def batch_hash_to_curve(r1, r2, out_format: int = OUT_ELEMENT, out: Optional[np.
     if r1.shape != r2.shape:
         raise ValueError("r1 and r2 differ in shape")
     n, w = r1.shape
-    out = _out(out, (n, _OUT_WIDTH[out_format]))
+    out = _out(out, (n, OUT_WIDTH[out_format]))
     check(_lib.load().d377_batch_hash_to_curve_wide(_ptr(r1), _ptr(r2), w, n, _ptr(out), out_format))
     return out
 
@@ -345,12 +341,12 @@ def batch_scalar_mul(points, scalars, point_format: int = PT_ELEMENT,
     """out[i] = scalars[i] * points[i].  `scalars_montgomery`: the scalars are the in-memory
     Montgomery limbs of the reference's Fr (D377_SCALARS_MONTGOMERY), converted on the GPU."""
     _ensure_init()
-    pts = _arr(points, _PT_WIDTH[point_format], "points")
+    pts = _arr(points, PT_WIDTH[point_format], "points")
     sc = _arr(scalars, 32, "scalars")
     if pts.shape[0] != sc.shape[0]:
         raise ValueError("points and scalars differ in length")
     n = pts.shape[0]
-    out = _out(out, (n, _OUT_WIDTH[out_format]))
+    out = _out(out, (n, OUT_WIDTH[out_format]))
     ok = _out(ok, (n,), "ok")
     check(_lib.load().d377_batch_scalar_mul(_ptr(pts), point_format | _mont(scalars_montgomery), _ptr(sc),
                                             n, _ptr(out), out_format, _ptr(ok)))
@@ -363,7 +359,7 @@ def fixed_base_mul(scalars, out_format: int = OUT_ELEMENT, out: Optional[np.ndar
     _ensure_init()
     sc = _arr(scalars, 32, "scalars")
     n = sc.shape[0]
-    out = _out(out, (n, _OUT_WIDTH[out_format]))
+    out = _out(out, (n, OUT_WIDTH[out_format]))
     check(_lib.load().d377_fixed_base_mul(_ptr(sc), n, _ptr(out), out_format | _mont(scalars_montgomery)))
     return out
 
@@ -454,7 +450,7 @@ class MsmBases:
         lib = _lib.load()
         out = C.c_void_p(0)
         if points is not None:
-            pts = _arr(points, _PT_WIDTH[point_format], "points")
+            pts = _arr(points, PT_WIDTH[point_format], "points")
             n = pts.shape[0]
             if windowed:
                 check(lib.d377_msm_bases_create_windowed(_ptr(pts), point_format, n, int(c), C.byref(out)))
@@ -507,7 +503,7 @@ class FixedBases:
         lib = _lib.load()
         out = C.c_void_p(0)
         if points is not None:
-            pts = _arr(points, _PT_WIDTH[point_format], "points")
+            pts = _arr(points, PT_WIDTH[point_format], "points")
             k = pts.shape[0]
             check(lib.d377_fixed_bases_create(_ptr(pts), point_format, k, C.byref(out)))
         else:
@@ -540,7 +536,7 @@ class FixedBases:
         Montgomery limbs of the reference's Fr (D377_SCALARS_MONTGOMERY)."""
         sc = self._scalars(scalars)
         n = sc.shape[0]
-        out = _out(out, (n, _OUT_WIDTH[out_format]))
+        out = _out(out, (n, OUT_WIDTH[out_format]))
         check(_lib.load().d377_fixed_bases_mul(self._handle(), _ptr(sc), n, _ptr(out),
                                                out_format | _mont(scalars_montgomery)))
         return out
@@ -576,7 +572,7 @@ def vartime_multiscalar_mul(scalars, points, point_format: int = PT_ELEMENT,
         check(_lib.load().d377_msm(_ptr(sc), _bases_ptr(points), PT_BASES | _mont(scalars_montgomery), n,
                                    _ptr(oe), _ptr(oc)))
         return oe, oc
-    pts = _arr(points, _PT_WIDTH[point_format], "points")
+    pts = _arr(points, PT_WIDTH[point_format], "points")
     n = min(sc.shape[0], pts.shape[0])
     check(_lib.load().d377_msm(_ptr(sc), _ptr(pts), point_format | _mont(scalars_montgomery), n,
                                _ptr(oe), _ptr(oc)))
@@ -589,7 +585,7 @@ def msm_multi(scalars, points, point_format: int = PT_ELEMENT, ngpu: Optional[in
     GPU takes a contiguous slice, partial sums meet on the first GPU)."""
     _ensure_init()
     sc = _arr(scalars, 32, "scalars")
-    pts = _arr(points, _PT_WIDTH[point_format], "points")
+    pts = _arr(points, PT_WIDTH[point_format], "points")
     n = min(sc.shape[0], pts.shape[0])
     ngpu = len(device_list()) if ngpu is None else int(ngpu)
     oe = np.empty((128,), np.uint8)
@@ -605,14 +601,14 @@ def batch_msm(scalars, points, offsets, point_format: int = PT_ELEMENT, out_form
     (Element::vartime_multiscalar_mul called in a loop).  Returns [nmsm, 128 | 32] (and ok [nmsm])."""
     _ensure_init()
     sc = _arr(scalars, 32, "scalars")
-    pts = _arr(points, _PT_WIDTH[point_format], "points")
+    pts = _arr(points, PT_WIDTH[point_format], "points")
     off = np.ascontiguousarray(offsets, dtype=np.uint32)
     if off.ndim != 1 or off.size < 1:
         raise ValueError("offsets must hold nmsm + 1 entries")
     nmsm = off.size - 1
     if int(off[-1]) > min(sc.shape[0], pts.shape[0]):
         raise ValueError("offsets reach past the end of the inputs")
-    out = np.empty((nmsm, _OUT_WIDTH[out_format]), np.uint8)
+    out = np.empty((nmsm, OUT_WIDTH[out_format]), np.uint8)
     ok = np.empty((nmsm,), np.uint8)
     check(_lib.load().d377_batch_msm(_ptr(sc), _ptr(pts), point_format | _mont(scalars_montgomery),
                                      off.ctypes.data_as(C.c_void_p), nmsm, _ptr(out), out_format, _ptr(ok)))
@@ -630,7 +626,7 @@ def msm_submit(scalars, points, point_format: int = PT_ELEMENT, slot: int = 0,
         n = min(sc.shape[0], points.n)
         check(_lib.load().d377_msm_submit(_ptr(sc), _bases_ptr(points), PT_BASES | _mont(scalars_montgomery), n, slot))
         return
-    pts = _arr(points, _PT_WIDTH[point_format], "points")
+    pts = _arr(points, PT_WIDTH[point_format], "points")
     n = min(sc.shape[0], pts.shape[0])
     check(_lib.load().d377_msm_submit(_ptr(sc), _ptr(pts), point_format | _mont(scalars_montgomery), n, slot))
 

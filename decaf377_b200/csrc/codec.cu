@@ -61,21 +61,7 @@ k_compress(const uint8_t* __restrict__ in, size_t n, uint8_t* __restrict__ enc) 
   if (i >= n) return;
   isqrt_smem_t sm = isqrt_smem(smem);
   pt_t p;
-  if (kFmt == D377_PT_AFFINE) {
-    p.x = fq_load_wire(in + 64 * i);
-    p.y = fq_load_wire(in + 64 * i + 32);
-    p.z = fq_one();
-    p.t = fq_mul(p.x, p.y);
-  } else if (kFmt == D377_PT_XYZ) {
-    fq_t x = fq_load_wire(in + 96 * i), y = fq_load_wire(in + 96 * i + 32);
-    fq_t z = fq_load_wire(in + 96 * i + 64);
-    p.x = fq_mul(x, z);
-    p.y = fq_mul(y, z);
-    p.z = fq_sqr(z);
-    p.t = fq_mul(x, y);
-  } else {
-    p = pt_load_wire(in + 128 * i);
-  }
+  pt_load_fmt<kFmt>(p, in, i, sm);
   fq_store(enc + 32 * i, pt_compress_to_field(p, sm));
 }
 

@@ -217,6 +217,24 @@ struct EngineScope {
 
 inline unsigned grid_for(size_t n, unsigned block) { return (unsigned)((n + block - 1) / block); }
 
+// Bytes per element of a point array in format D377_PT_* (D377_PT_BASES: one prepared record)
+// and of a result in format D377_OUT_*.
+__host__ __device__ constexpr size_t pt_bytes(int fmt) {
+  return fmt == D377_PT_ENCODING ? 32 : fmt == D377_PT_AFFINE ? 64 : fmt == D377_PT_XYZ ? 96 : 128;
+}
+constexpr size_t out_bytes(int fmt) { return pt_bytes(fmt == D377_OUT_ENCODING ? D377_PT_ENCODING : D377_PT_ELEMENT); }
+
+// The set of format values an entry point accepts, as the `accepted` mask of parse_format.
+template <class... F>
+constexpr unsigned fmt_set(F... f) { return ((1u << f) | ...); }
+constexpr unsigned kPointFormats = fmt_set(D377_PT_ELEMENT, D377_PT_ENCODING, D377_PT_AFFINE, D377_PT_XYZ);
+constexpr unsigned kOutFormats = fmt_set(D377_OUT_ELEMENT, D377_OUT_ENCODING);
+
+// The format word of entry point `who` -> the format value (*fmt, if wanted) and, for a call
+// that takes scalars (sc_mont not null), the D377_SCALARS_MONTGOMERY flag riding on it
+// (*sc_mont).  A value outside `accepted` is refused with D377_ERR_INVALID_ARG.
+int parse_format(const char* who, int word, unsigned accepted, int* fmt, bool* sc_mont = nullptr);
+
 // kernels.cu
 void launch_fr_from_mont(const uint8_t* in, size_t n, uint8_t* out, cudaStream_t st);
 // codec.cu
@@ -250,6 +268,11 @@ int msm_dev(const uint8_t* scalars, const uint8_t* points, int point_format, siz
             uint8_t* out_element, uint8_t* out_encoding);
 int msm_dev_async(const uint8_t* scalars, const uint8_t* points, int point_format, size_t n,
                   uint8_t* out_element, uint8_t* out_encoding, int flags);
+// Arguments of the single-device MSM calls: the format word (any D377_PT_* format, split by
+// parse_format), null pointers and, for prepared bases, the handle.
+int msm_args_ok(Engine& e, const char* who, const uint8_t* scalars, const uint8_t* points, int point_format,
+                size_t n, int* fmt, bool* sc_mont);
+// `point_format`: a D377_PT_* value; `sc_mont`: the scalars are in Montgomery form.
 // `inputs_ready`: the inputs depend on nothing but chunk_ready[k] (nothing at all without
 // chunk_ready): the scalar side may then start under the previous MSM's accumulation.
 // `chunk` = 0: one Pippenger (split only above 2^26 pairs).  Otherwise the input is
@@ -257,7 +280,7 @@ int msm_dev_async(const uint8_t* scalars, const uint8_t* points, int point_forma
 // engine stream waits for chunk_ready[k] (if given) before it touches chunk k.
 // The result is complete on result_stream(): the tail stream, or the engine stream when the
 // tail overlap is switched off.
-int msm_enqueue(const uint8_t* scalars, const uint8_t* points, int point_format, size_t n,
+int msm_enqueue(const uint8_t* scalars, const uint8_t* points, int point_format, bool sc_mont, size_t n,
                 uint8_t* out_element, uint8_t* out_encoding, uint32_t* flags, size_t chunk = 0,
                 const cudaEvent_t* chunk_ready = nullptr, bool inputs_ready = false,
                 const cudaEvent_t* scalars_ready_ev = nullptr);

@@ -214,13 +214,20 @@ D377_DBG_READER(kernels_debug_counts)
 // host side of the API
 // ---------------------------------------------------------------------------
 
-static int check_fmt(int f) { return f == D377_OUT_ELEMENT || f == D377_OUT_ENCODING; }
 // D377_SCALARS_MONTGOMERY rides on the format word of every call that takes scalars
-static bool take_sc_mont(int& fmt) {
-  const bool m = fmt >= 0 && (fmt & D377_SCALARS_MONTGOMERY) != 0;
-  if (m) fmt &= ~D377_SCALARS_MONTGOMERY;
-  return m;
+int parse_format(const char* who, int word, unsigned accepted, int* fmt, bool* sc_mont) {
+  const bool m = sc_mont && word >= 0 && (word & D377_SCALARS_MONTGOMERY) != 0;
+  const int f = m ? word & ~D377_SCALARS_MONTGOMERY : word;
+  if (f < 0 || f > 31 || !((accepted >> f) & 1u)) {
+    set_error("%s: format word %d is not accepted", who, word);
+    return D377_ERR_INVALID_ARG;
+  }
+  if (fmt) *fmt = f;
+  if (sc_mont) *sc_mont = m;
+  return D377_OK;
 }
+// point formats of the calls that multiply caller's points by scalars one by one
+constexpr unsigned kMulFormats = fmt_set(D377_PT_ELEMENT, D377_PT_ENCODING, D377_PT_AFFINE);
 // scalars in the reference's Montgomery form -> canonical, into the engine's scratch
 static int canonical_scalars(Engine& e, const uint8_t*& scalars, size_t n) {
   int rc = ensure(e.sc_canon, n * 32 + 32);
@@ -229,11 +236,6 @@ static int canonical_scalars(Engine& e, const uint8_t*& scalars, size_t n) {
   scalars = (const uint8_t*)e.sc_canon.p;
   return D377_OK;
 }
-static size_t pt_bytes(int fmt) {
-  return fmt == D377_PT_ELEMENT || fmt == D377_PT_BASES ? 128 : fmt == D377_PT_ENCODING ? 32
-         : fmt == D377_PT_XYZ ? 96 : 64;
-}
-static size_t out_bytes(int fmt) { return fmt == D377_OUT_ENCODING ? 32 : 128; }
 
 void codec_debug_counts(unsigned long long*, unsigned long long*);
 void scalar_debug_counts(unsigned long long*, unsigned long long*);
@@ -623,30 +625,37 @@ int d377_batch_compress_dev(const uint8_t* elements, size_t n, uint8_t* enc) {
   return D377_OK;
 }
 
+static int null_pointer() {
+  set_error("null pointer");
+  return D377_ERR_INVALID_ARG;
+}
+
+static int decompress_fmt_args(const uint8_t* enc, size_t n, int out_format, const uint8_t* out) {
+  TRY(parse_format("d377_batch_decompress_fmt", out_format, fmt_set(D377_PT_ELEMENT, D377_PT_AFFINE), nullptr));
+  return n && (!enc || !out) ? null_pointer() : D377_OK;
+}
+
 int d377_batch_decompress_fmt_dev(const uint8_t* enc, size_t n, int out_format, uint8_t* out,
                                   uint8_t* ok) {
   D377_REQUIRE_READY();
-  if (out_format != D377_PT_ELEMENT && out_format != D377_PT_AFFINE) {
-    set_error("bad out_format %d (Element or AffinePoint)", out_format);
-    return D377_ERR_INVALID_ARG;
-  }
+  TRY(decompress_fmt_args(enc, n, out_format, out));
   if (n == 0) return D377_OK;
-  if (!enc || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   launch_decompress(enc, n, out, ok, _eng.stream, out_format);
   D377_LAUNCHED();
   D377_CUDA(cudaGetLastError());
   return D377_OK;
 }
 
+static int compress_fmt_args(const uint8_t* points, int point_format, size_t n, const uint8_t* enc) {
+  TRY(parse_format("d377_batch_compress_fmt", point_format, fmt_set(D377_PT_ELEMENT, D377_PT_AFFINE, D377_PT_XYZ),
+                   nullptr));
+  return n && (!enc || !points) ? null_pointer() : D377_OK;
+}
+
 int d377_batch_compress_fmt_dev(const uint8_t* points, int point_format, size_t n, uint8_t* enc) {
   D377_REQUIRE_READY();
-  if (point_format != D377_PT_ELEMENT && point_format != D377_PT_AFFINE &&
-      point_format != D377_PT_XYZ) {
-    set_error("bad point_format %d (Element, AffinePoint or X||Y||Z)", point_format);
-    return D377_ERR_INVALID_ARG;
-  }
+  TRY(compress_fmt_args(points, point_format, n, enc));
   if (n == 0) return D377_OK;
-  if (!enc || !points) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   launch_compress(points, n, enc, _eng.stream, point_format);
   D377_LAUNCHED();
   D377_CUDA(cudaGetLastError());
@@ -658,13 +667,20 @@ static int check_width(size_t w) {
   return D377_OK;
 }
 
+// encode_to_curve (r1) and hash_to_curve (r1, r2)
+static int elligator_args(bool hash, const uint8_t* r1, const uint8_t* r2, size_t in_width, size_t n,
+                          const uint8_t* out, int out_format) {
+  TRY(parse_format(hash ? "d377_batch_hash_to_curve" : "d377_batch_encode_to_curve", out_format, kOutFormats,
+                   nullptr));
+  TRY(check_width(in_width));
+  return n && (!r1 || (hash && !r2) || !out) ? null_pointer() : D377_OK;
+}
+
 int d377_batch_encode_to_curve_wide_dev(const uint8_t* r, size_t in_width, size_t n, uint8_t* out,
                                         int out_format) {
   D377_REQUIRE_READY();
-  if (!check_fmt(out_format)) { set_error("bad out_format %d", out_format); return D377_ERR_INVALID_ARG; }
-  if (int rc = check_width(in_width)) return rc;
+  TRY(elligator_args(false, r, nullptr, in_width, n, out, out_format));
   if (n == 0) return D377_OK;
-  if (!r || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   launch_elligator(false, out_format == D377_OUT_ENCODING, r, nullptr, in_width, n, out, _eng.stream);
   D377_LAUNCHED();
   D377_CUDA(cudaGetLastError());
@@ -678,10 +694,8 @@ int d377_batch_encode_to_curve_dev(const uint8_t* r, size_t n, uint8_t* out, int
 int d377_batch_hash_to_curve_wide_dev(const uint8_t* r1, const uint8_t* r2, size_t in_width, size_t n,
                                       uint8_t* out, int out_format) {
   D377_REQUIRE_READY();
-  if (!check_fmt(out_format)) { set_error("bad out_format %d", out_format); return D377_ERR_INVALID_ARG; }
-  if (int rc = check_width(in_width)) return rc;
+  TRY(elligator_args(true, r1, r2, in_width, n, out, out_format));
   if (n == 0) return D377_OK;
-  if (!r1 || !r2 || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   launch_elligator(true, out_format == D377_OUT_ENCODING, r1, r2, in_width, n, out, _eng.stream);
   D377_LAUNCHED();
   D377_CUDA(cudaGetLastError());
@@ -693,79 +707,94 @@ int d377_batch_hash_to_curve_dev(const uint8_t* r1, const uint8_t* r2, size_t n,
   return d377_batch_hash_to_curve_wide_dev(r1, r2, 32, n, out, out_format);
 }
 
+static int from_le_bytes_args(const uint8_t* bytes, size_t in_width, size_t n, const uint8_t* out) {
+  TRY(check_width(in_width));
+  return n && (!bytes || !out) ? null_pointer() : D377_OK;
+}
+
 int d377_fq_batch_from_le_bytes_mod_order_dev(const uint8_t* bytes, size_t in_width, size_t n,
                                               uint8_t* out) {
   D377_REQUIRE_READY();
-  if (int rc = check_width(in_width)) return rc;
+  TRY(from_le_bytes_args(bytes, in_width, n, out));
   if (n == 0) return D377_OK;
-  if (!bytes || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   k_fq_from_wide<<<grid_for(n, 128), 128, 0, _eng.stream>>>(bytes, in_width, n, out);
   D377_LAUNCHED();
   D377_CUDA(cudaGetLastError());
   return D377_OK;
 }
 
+// *pf, *sc_mont: the point format and the scalar form the format word carries
+static int scalar_mul_args(const uint8_t* points, int point_format, const uint8_t* scalars, size_t n,
+                           const uint8_t* out, int out_format, int* pf, bool* sc_mont) {
+  TRY(parse_format("d377_batch_scalar_mul", point_format, kMulFormats, pf, sc_mont));
+  TRY(parse_format("d377_batch_scalar_mul", out_format, kOutFormats, nullptr));
+  return n && (!points || !scalars || !out) ? null_pointer() : D377_OK;
+}
+
 int d377_batch_scalar_mul_dev(const uint8_t* points, int point_format, const uint8_t* scalars,
                               size_t n, uint8_t* out, int out_format, uint8_t* ok) {
   D377_REQUIRE_READY();
-  const bool sc_mont = take_sc_mont(point_format);
-  if (!check_fmt(out_format) || point_format < 0 || point_format > 2) {
-    set_error("bad format (%d, %d)", point_format, out_format);
-    return D377_ERR_INVALID_ARG;
-  }
+  int pf = 0;
+  bool sc_mont = false;
+  TRY(scalar_mul_args(points, point_format, scalars, n, out, out_format, &pf, &sc_mont));
   if (n == 0) return D377_OK;
-  if (!points || !scalars || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
-  if (sc_mont) { int rc = canonical_scalars(_eng, scalars, n); if (rc) return rc; }
-  launch_scalar_mul(point_format, out_format == D377_OUT_ENCODING, points, scalars, n, out, ok, _eng.stream);
+  if (sc_mont) TRY(canonical_scalars(_eng, scalars, n));
+  launch_scalar_mul(pf, out_format == D377_OUT_ENCODING, points, scalars, n, out, ok, _eng.stream);
   D377_LAUNCHED();
   D377_CUDA(cudaGetLastError());
   return D377_OK;
 }
 
+// *of, *sc_mont: the output format and the scalar form the format word carries
+static int fixed_base_args(const uint8_t* scalars, size_t n, const uint8_t* out, int out_format, int* of,
+                           bool* sc_mont) {
+  TRY(parse_format("d377_fixed_base_mul", out_format, kOutFormats, of, sc_mont));
+  return n && (!scalars || !out) ? null_pointer() : D377_OK;
+}
+
 int d377_fixed_base_mul_dev(const uint8_t* scalars, size_t n, uint8_t* out, int out_format) {
   D377_REQUIRE_READY();
-  const bool sc_mont = take_sc_mont(out_format);
-  if (!check_fmt(out_format)) { set_error("bad out_format %d", out_format); return D377_ERR_INVALID_ARG; }
+  int of = 0;
+  bool sc_mont = false;
+  TRY(fixed_base_args(scalars, n, out, out_format, &of, &sc_mont));
   if (n == 0) return D377_OK;
-  if (!scalars || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   Engine& e = _eng;
-  int rc = ensure_fb_table();
-  if (rc) return rc;
-  if (sc_mont && (rc = canonical_scalars(e, scalars, n))) return rc;
+  TRY(ensure_fb_table());
+  if (sc_mont) TRY(canonical_scalars(e, scalars, n));
   // The quartic table is 1.6 GB and takes ~0.15 s to build: only a batch large enough to
   // win that back builds it (or finds it built); smaller calls take the Edwards table +
   // compress, whose output is bit-identical.  The host-buffer entry point passes the size of
   // the whole batch through fb_batch_hint so that its chunks agree.
   constexpr size_t kFbQuarticMin = (size_t)1 << 18;
   const size_t batch = std::max(n, e.fb_batch_hint);
-  bool quartic = out_format == D377_OUT_ENCODING && (e.fb_table_jq != nullptr || batch >= kFbQuarticMin);
+  bool quartic = of == D377_OUT_ENCODING && (e.fb_table_jq != nullptr || batch >= kFbQuarticMin);
   if (quartic && ensure_fb_table_jq() != D377_OK) {
     // no room for the quartic table: the Edwards path gives the same bytes
     cudaGetLastError();
     quartic = false;
   }
-  launch_fixed_base(out_format == D377_OUT_ENCODING, e.fb_table, 1, quartic ? e.fb_table_jq : nullptr, scalars, n,
+  launch_fixed_base(of == D377_OUT_ENCODING, e.fb_table, 1, quartic ? e.fb_table_jq : nullptr, scalars, n,
                     out, e.stream);
   D377_LAUNCHED();
   D377_CUDA(cudaGetLastError());
   return D377_OK;
 }
 
-// a live set of fixed bases of this engine -> its k
-static int fixed_bases_k(Engine& e, const uint8_t* tables, const char* who, size_t* k) {
+// The table set must be a live set of fixed bases of this engine (checked before n = 0 is
+// looked at; *k receives its size); n rows of k 32-byte scalars must stay addressable.
+static int fixed_bases_mul_args(Engine& e, const uint8_t* tables, const uint8_t* scalars, size_t n,
+                                const uint8_t* out, int out_format, size_t* k, int* of, bool* sc_mont) {
+  TRY(parse_format("d377_fixed_bases_mul", out_format, kOutFormats, of, sc_mont));
   auto it = e.fixed_bases.find(tables);
   if (it == e.fixed_bases.end()) {
-    set_error("%s: %p is not a live set of fixed bases of device %d", who, (const void*)tables, e.device);
+    set_error("d377_fixed_bases_mul: %p is not a live set of fixed bases of device %d", (const void*)tables,
+              e.device);
     return D377_ERR_INVALID_ARG;
   }
   *k = it->second.k;
-  return D377_OK;
-}
-
-// n rows of k 32-byte scalars must stay addressable
-static int fixed_bases_rows(size_t n, size_t k) {
-  if (n > SIZE_MAX / 32 / k) {
-    set_error("fixed bases: %zu rows of %zu scalars overflow the address space", n, k);
+  if (n && (!scalars || !out)) return null_pointer();
+  if (n > SIZE_MAX / 32 / *k) {
+    set_error("fixed bases: %zu rows of %zu scalars overflow the address space", n, *k);
     return D377_ERR_INVALID_ARG;
   }
   return D377_OK;
@@ -773,16 +802,14 @@ static int fixed_bases_rows(size_t n, size_t k) {
 
 int d377_fixed_bases_mul_dev(const uint8_t* tables, const uint8_t* scalars, size_t n, uint8_t* out, int out_format) {
   D377_REQUIRE_READY();
-  const bool sc_mont = take_sc_mont(out_format);
-  if (!check_fmt(out_format)) { set_error("bad out_format %d", out_format); return D377_ERR_INVALID_ARG; }
   Engine& e = _eng;
   size_t k = 0;
-  TRY(fixed_bases_k(e, tables, "d377_fixed_bases_mul_dev", &k));
+  int of = 0;
+  bool sc_mont = false;
+  TRY(fixed_bases_mul_args(e, tables, scalars, n, out, out_format, &k, &of, &sc_mont));
   if (n == 0) return D377_OK;
-  if (!scalars || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
-  TRY(fixed_bases_rows(n, k));
   if (sc_mont) TRY(canonical_scalars(e, scalars, n * k));
-  launch_fixed_base(out_format == D377_OUT_ENCODING, tables, k, nullptr, scalars, n, out, e.stream);
+  launch_fixed_base(of == D377_OUT_ENCODING, tables, k, nullptr, scalars, n, out, e.stream);
   D377_LAUNCHED();
   D377_CUDA(cudaGetLastError());
   return D377_OK;
@@ -856,15 +883,18 @@ int d377_msm_dev_async(const uint8_t* scalars, const uint8_t* points, int point_
 }
 
 // ---- many independent small MSMs (Element::vartime_multiscalar_mul in a loop) -----------
+static int batch_msm_formats(int point_format, int out_format, int* pf, bool* sc_mont) {
+  TRY(parse_format("d377_batch_msm", point_format, kMulFormats, pf, sc_mont));
+  return parse_format("d377_batch_msm", out_format, kOutFormats, nullptr);
+}
+
 int d377_batch_msm_dev(const uint8_t* scalars, const uint8_t* points, int point_format,
                        const uint32_t* offsets, size_t nmsm, size_t n, uint8_t* out, int out_format,
                        uint8_t* ok) {
   D377_REQUIRE_READY();
-  const bool sc_mont = take_sc_mont(point_format);
-  if (!check_fmt(out_format) || point_format < 0 || point_format > 2) {
-    set_error("bad format (%d, %d)", point_format, out_format);
-    return D377_ERR_INVALID_ARG;
-  }
+  int pf = 0;
+  bool sc_mont = false;
+  TRY(batch_msm_formats(point_format, out_format, &pf, &sc_mont));
   if (nmsm == 0) return D377_OK;
   if (n > 0xfffffff0ull) { set_error("d377_batch_msm: too many pairs"); return D377_ERR_INVALID_ARG; }
   if (!offsets || !out || (n && (!scalars || !points))) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
@@ -872,10 +902,10 @@ int d377_batch_msm_dev(const uint8_t* scalars, const uint8_t* points, int point_
   TRY(ensure(e.bm_prod, n * 128 + 128));
   TRY(ensure(e.bm_ok, n + 16));
   uint8_t* prod = (uint8_t*)e.bm_prod.p;
-  uint8_t* okp = point_format == D377_PT_ENCODING ? (uint8_t*)e.bm_ok.p : nullptr;
+  uint8_t* okp = pf == D377_PT_ENCODING ? (uint8_t*)e.bm_ok.p : nullptr;
   if (n) {
     if (sc_mont) TRY(canonical_scalars(e, scalars, n));
-    launch_scalar_mul(point_format, false, points, scalars, n, prod, okp, e.stream);
+    launch_scalar_mul(pf, false, points, scalars, n, prod, okp, e.stream);
     D377_LAUNCHED();
   }
   uint8_t* sums = out;
@@ -895,9 +925,9 @@ int d377_batch_msm_dev(const uint8_t* scalars, const uint8_t* points, int point_
 int d377_batch_msm(const uint8_t* scalars, const uint8_t* points, int point_format, const uint32_t* offsets,
                    size_t nmsm, uint8_t* out, int out_format, uint8_t* ok) {
   D377_REQUIRE_READY();
-  int pf = point_format;
-  take_sc_mont(pf);
-  if (!check_fmt(out_format) || pf < 0 || pf > 2) { set_error("bad format (%d, %d)", point_format, out_format); return D377_ERR_INVALID_ARG; }
+  int pf = 0;
+  bool sc_mont = false;
+  TRY(batch_msm_formats(point_format, out_format, &pf, &sc_mont));
   if (nmsm == 0) return D377_OK;
   if (!offsets || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   if (nmsm > 0x7fffffffull) { set_error("d377_batch_msm: too many segments"); return D377_ERR_INVALID_ARG; }
@@ -966,11 +996,15 @@ int d377_fq_batch_isqrt_dev(const uint8_t* x, size_t n, uint8_t* out, uint8_t* w
   return D377_OK;
 }
 
+static int deserialize_args(int field, const uint8_t* bytes, size_t n, const uint8_t* ok) {
+  if (field != 0 && field != 1) { set_error("field must be 0 (Fq) or 1 (Fr)"); return D377_ERR_INVALID_ARG; }
+  return n && (!bytes || !ok) ? null_pointer() : D377_OK;
+}
+
 int d377_field_batch_deserialize_dev(int field, const uint8_t* bytes, size_t n, uint8_t* out, uint8_t* ok) {
   D377_REQUIRE_READY();
-  if (field != 0 && field != 1) { set_error("field must be 0 (Fq) or 1 (Fr)"); return D377_ERR_INVALID_ARG; }
+  TRY(deserialize_args(field, bytes, n, ok));
   if (n == 0) return D377_OK;
-  if (!bytes || !ok) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   Engine& e = _eng;
   if (field == 0)
     k_field_deserialize<0><<<grid_for(n, 256), 256, 0, e.stream>>>(bytes, n, out, ok);
@@ -1091,13 +1125,9 @@ int d377_batch_compress(const uint8_t* elements, size_t n, uint8_t* enc) {
 int d377_batch_decompress_fmt(const uint8_t* enc, size_t n, int out_format, uint8_t* out,
                               uint8_t* ok) {
   D377_REQUIRE_READY();
-  if (out_format != D377_PT_ELEMENT && out_format != D377_PT_AFFINE) {
-    set_error("bad out_format %d (Element or AffinePoint)", out_format);
-    return D377_ERR_INVALID_ARG;
-  }
+  TRY(decompress_fmt_args(enc, n, out_format, out));
   if (n == 0) return D377_OK;
-  if (!enc || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
-  HostIn ins[] = {{enc, 32}};
+  HostIn ins[] = {{enc, pt_bytes(D377_PT_ENCODING)}};
   HostOut outs[] = {{out, pt_bytes(out_format)}, {ok, 1}};
   return run_pipelined(n, ins, 1, outs, 2, [&](uint8_t* const* di, uint8_t* const* dout, size_t len) {
     return d377_batch_decompress_fmt_dev(di[0], len, out_format, dout[0], dout[1]);
@@ -1106,15 +1136,10 @@ int d377_batch_decompress_fmt(const uint8_t* enc, size_t n, int out_format, uint
 
 int d377_batch_compress_fmt(const uint8_t* points, int point_format, size_t n, uint8_t* enc) {
   D377_REQUIRE_READY();
-  if (point_format != D377_PT_ELEMENT && point_format != D377_PT_AFFINE &&
-      point_format != D377_PT_XYZ) {
-    set_error("bad point_format %d (Element, AffinePoint or X||Y||Z)", point_format);
-    return D377_ERR_INVALID_ARG;
-  }
+  TRY(compress_fmt_args(points, point_format, n, enc));
   if (n == 0) return D377_OK;
-  if (!enc || !points) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   HostIn ins[] = {{points, pt_bytes(point_format)}};
-  HostOut outs[] = {{enc, 32}};
+  HostOut outs[] = {{enc, pt_bytes(D377_PT_ENCODING)}};
   return run_pipelined(n, ins, 1, outs, 1, [&](uint8_t* const* di, uint8_t* const* dout, size_t len) {
     return d377_batch_compress_fmt_dev(di[0], point_format, len, dout[0]);
   });
@@ -1123,10 +1148,8 @@ int d377_batch_compress_fmt(const uint8_t* points, int point_format, size_t n, u
 int d377_batch_encode_to_curve_wide(const uint8_t* r, size_t in_width, size_t n, uint8_t* out,
                                     int out_format) {
   D377_REQUIRE_READY();
-  if (!check_fmt(out_format)) { set_error("bad out_format %d", out_format); return D377_ERR_INVALID_ARG; }
-  if (int rc = check_width(in_width)) return rc;
+  TRY(elligator_args(false, r, nullptr, in_width, n, out, out_format));
   if (n == 0) return D377_OK;
-  if (!r || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   HostIn ins[] = {{r, in_width}};
   HostOut outs[] = {{out, out_bytes(out_format)}};
   return run_pipelined(n, ins, 1, outs, 1, [&](uint8_t* const* di, uint8_t* const* dout, size_t len) {
@@ -1141,10 +1164,8 @@ int d377_batch_encode_to_curve(const uint8_t* r, size_t n, uint8_t* out, int out
 int d377_batch_hash_to_curve_wide(const uint8_t* r1, const uint8_t* r2, size_t in_width, size_t n,
                                   uint8_t* out, int out_format) {
   D377_REQUIRE_READY();
-  if (!check_fmt(out_format)) { set_error("bad out_format %d", out_format); return D377_ERR_INVALID_ARG; }
-  if (int rc = check_width(in_width)) return rc;
+  TRY(elligator_args(true, r1, r2, in_width, n, out, out_format));
   if (n == 0) return D377_OK;
-  if (!r1 || !r2 || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   HostIn ins[] = {{r1, in_width}, {r2, in_width}};
   HostOut outs[] = {{out, out_bytes(out_format)}};
   return run_pipelined(n, ins, 2, outs, 1, [&](uint8_t* const* di, uint8_t* const* dout, size_t len) {
@@ -1159,9 +1180,8 @@ int d377_batch_hash_to_curve(const uint8_t* r1, const uint8_t* r2, size_t n, uin
 
 int d377_fq_batch_from_le_bytes_mod_order(const uint8_t* bytes, size_t in_width, size_t n, uint8_t* out) {
   D377_REQUIRE_READY();
-  if (int rc = check_width(in_width)) return rc;
+  TRY(from_le_bytes_args(bytes, in_width, n, out));
   if (n == 0) return D377_OK;
-  if (!bytes || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   HostIn ins[] = {{bytes, in_width}};
   HostOut outs[] = {{out, 32}};
   return run_pipelined(n, ins, 1, outs, 1, [&](uint8_t* const* di, uint8_t* const* dout, size_t len) {
@@ -1172,35 +1192,30 @@ int d377_fq_batch_from_le_bytes_mod_order(const uint8_t* bytes, size_t in_width,
 int d377_batch_scalar_mul(const uint8_t* points, int point_format, const uint8_t* scalars,
                           size_t n, uint8_t* out, int out_format, uint8_t* ok) {
   D377_REQUIRE_READY();
-  const int fmt_word = point_format;
-  take_sc_mont(point_format);
-  if (!check_fmt(out_format) || point_format < 0 || point_format > 2) {
-    set_error("bad format (%d, %d)", point_format, out_format);
-    return D377_ERR_INVALID_ARG;
-  }
+  int pf = 0;
+  bool sc_mont = false;
+  TRY(scalar_mul_args(points, point_format, scalars, n, out, out_format, &pf, &sc_mont));
   if (n == 0) return D377_OK;
-  if (!points || !scalars || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
-  HostIn ins[] = {{points, pt_bytes(point_format)}, {scalars, 32}};
+  HostIn ins[] = {{points, pt_bytes(pf)}, {scalars, 32}};
   HostOut outs[] = {{out, out_bytes(out_format)}, {ok, 1}};
   return run_pipelined(n, ins, 2, outs, 2, [&](uint8_t* const* di, uint8_t* const* dout, size_t len) {
     // only encodings can fail to decode; every other format is always Ok
     D377_CUDA(cudaMemsetAsync(dout[1], 1, len, engine().stream));
-    return d377_batch_scalar_mul_dev(di[0], fmt_word, di[1], len, dout[0], out_format, dout[1]);
+    return d377_batch_scalar_mul_dev(di[0], point_format, di[1], len, dout[0], out_format, dout[1]);
   });
 }
 
 int d377_fixed_base_mul(const uint8_t* scalars, size_t n, uint8_t* out, int out_format) {
   D377_REQUIRE_READY();
-  const int fmt_word = out_format;
-  take_sc_mont(out_format);
-  if (!check_fmt(out_format)) { set_error("bad out_format %d", out_format); return D377_ERR_INVALID_ARG; }
+  int of = 0;
+  bool sc_mont = false;
+  TRY(fixed_base_args(scalars, n, out, out_format, &of, &sc_mont));
   if (n == 0) return D377_OK;
-  if (!scalars || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   HostIn ins[] = {{scalars, 32}};
-  HostOut outs[] = {{out, out_bytes(out_format)}};
+  HostOut outs[] = {{out, out_bytes(of)}};
   _eng.fb_batch_hint = n;
   int rc = run_pipelined(n, ins, 1, outs, 1, [&](uint8_t* const* di, uint8_t* const* dout, size_t len) {
-    return d377_fixed_base_mul_dev(di[0], len, dout[0], fmt_word);
+    return d377_fixed_base_mul_dev(di[0], len, dout[0], out_format);
   });
   _eng.fb_batch_hint = 0;
   return rc;
@@ -1208,18 +1223,15 @@ int d377_fixed_base_mul(const uint8_t* scalars, size_t n, uint8_t* out, int out_
 
 int d377_fixed_bases_mul(const uint8_t* tables, const uint8_t* scalars, size_t n, uint8_t* out, int out_format) {
   D377_REQUIRE_READY();
-  const int fmt_word = out_format;
-  take_sc_mont(out_format);
-  if (!check_fmt(out_format)) { set_error("bad out_format %d", out_format); return D377_ERR_INVALID_ARG; }
   size_t k = 0;
-  TRY(fixed_bases_k(_eng, tables, "d377_fixed_bases_mul", &k));
+  int of = 0;
+  bool sc_mont = false;
+  TRY(fixed_bases_mul_args(_eng, tables, scalars, n, out, out_format, &k, &of, &sc_mont));
   if (n == 0) return D377_OK;
-  if (!scalars || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
-  TRY(fixed_bases_rows(n, k));
   HostIn ins[] = {{scalars, 32 * k}};
-  HostOut outs[] = {{out, out_bytes(out_format)}};
+  HostOut outs[] = {{out, out_bytes(of)}};
   return run_pipelined(n, ins, 1, outs, 1, [&](uint8_t* const* di, uint8_t* const* dout, size_t len) {
-    return d377_fixed_bases_mul_dev(tables, di[0], len, dout[0], fmt_word);
+    return d377_fixed_bases_mul_dev(tables, di[0], len, dout[0], out_format);
   });
 }
 
@@ -1285,93 +1297,80 @@ int d377_element_sum(const uint8_t* elements, size_t n, uint8_t out_element[128]
   return small_results_back(out_element, out_encoding);
 }
 
-int d377_msm_bases_create_dev(const uint8_t* points, int point_format, size_t n, uint8_t** bases) {
-  D377_REQUIRE_READY();
-  if (point_format < 0 || point_format > 3) { set_error("bad point_format %d", point_format); return D377_ERR_INVALID_ARG; }
-  if (!bases || (n && !points)) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
-  uint8_t* rec = nullptr;
-  D377_CUDA(cudaMalloc(&rec, n * 128 + 128));
-  int rc = msm_bases_prepare(points, point_format, n, rec);
-  if (rc) { cudaFree(rec); return rc; }
-  BasesLayout bl;
-  bl.n = n;
-  bl.bytes = n * 128 + 128;
-  _eng.bases[rec] = bl;
-  *bases = rec;
-  return D377_OK;
-}
-
-int d377_msm_bases_create(const uint8_t* points, int point_format, size_t n, uint8_t** bases) {
-  D377_REQUIRE_READY();
-  if (point_format < 0 || point_format > 3) { set_error("bad point_format %d", point_format); return D377_ERR_INVALID_ARG; }
-  if (!bases || (n && !points)) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
-  Engine& e = _eng;
-  const size_t pb = pt_bytes(point_format);
-  uint8_t* tmp = nullptr;
-  D377_CUDA(cudaMalloc(&tmp, n * pb + 128));
-  cudaError_t ce = cudaMemcpyAsync(tmp, points, n * pb, cudaMemcpyHostToDevice, e.stream);
-  if (ce != cudaSuccess) { cudaStreamSynchronize(e.stream); cudaFree(tmp); return cuda_fail(ce, "upload of the bases", __FILE__, __LINE__); }
-  int rc = d377_msm_bases_create_dev(tmp, point_format, n, bases);   // synchronises the stream
-  if (rc) cudaStreamSynchronize(e.stream);
-  cudaFree(tmp);
-  return rc;
-}
-
-// Arguments of the windowed twins, checked before anything is allocated or read: *W receives
-// the number of windows of the width *c (0 = chosen from n).
-static int windowed_args(int point_format, size_t n, int* c, int* W, uint8_t** bases, const uint8_t* points) {
-  if (point_format < 0 || point_format > 3) { set_error("bad point_format %d", point_format); return D377_ERR_INVALID_ARG; }
-  if (!bases || (n && !points)) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
-  if (*c != 0 && (*c < 4 || *c > 22)) { set_error("window width %d out of range [4, 22]", *c); return D377_ERR_INVALID_ARG; }
-  if (*c == 0) *c = msm_windowed_c(n);
-  *W = (252 + *c - 1) / *c;
-  // the scatter stores a record index and a sign bit in 32 bits
-  if ((double)n * (double)*W >= 2147483648.0) {
-    set_error("windowed bases: n * W = %zu * %d records reach 2^31", n, *W);
-    return D377_ERR_INVALID_ARG;
+// d377_msm_bases_create* (windowed = false: a plain set, c = 0, W = 1) and
+// d377_msm_bases_create_windowed* (windowed = true, c = 0: the width is chosen from n).  Every
+// argument is checked before anything is allocated or read.  `host`: `points` is host memory,
+// uploaded once the set is allocated.
+static int msm_bases_create(const uint8_t* points, int point_format, size_t n, bool windowed, int c,
+                            uint8_t** bases, bool host) {
+  Engine& e = engine();
+  int fmt = 0, W = 1;
+  TRY(parse_format("d377_msm_bases_create", point_format, kPointFormats, &fmt));
+  if (!bases || (n && !points)) return null_pointer();
+  if (windowed) {
+    if (c != 0 && (c < 4 || c > 22)) { set_error("window width %d out of range [4, 22]", c); return D377_ERR_INVALID_ARG; }
+    if (c == 0) c = msm_windowed_c(n);
+    W = (252 + c - 1) / c;
+    // the scatter stores a record index and a sign bit in 32 bits
+    if ((double)n * (double)W >= 2147483648.0) {
+      set_error("windowed bases: n * W = %zu * %d records reach 2^31", n, W);
+      return D377_ERR_INVALID_ARG;
+    }
+  } else {
+    c = 0;
   }
-  return D377_OK;
-}
-
-int d377_msm_bases_create_windowed_dev(const uint8_t* points, int point_format, size_t n, int c, uint8_t** bases) {
-  D377_REQUIRE_READY();
-  int W = 0;
-  TRY(windowed_args(point_format, n, &c, &W, bases, points));
-  const size_t bytes = n * (size_t)W * 128 + 128;
+  const size_t bytes = (n * (size_t)W + 1) * pt_bytes(D377_PT_BASES);
   uint8_t* tab = nullptr;
   cudaError_t ce = cudaMalloc(&tab, bytes);
   if (ce != cudaSuccess) {
     cudaGetLastError();
-    set_error("windowed bases: cannot allocate %zu bytes of device memory (%s)", bytes, cudaGetErrorString(ce));
+    set_error("msm bases: cannot allocate %zu bytes of device memory (%s)", bytes, cudaGetErrorString(ce));
     return D377_ERR_CUDA;
   }
-  int rc = msm_bases_prepare(points, point_format, n, tab);   // slab 0 = the plain set
+  int rc = D377_OK;
+  uint8_t* tmp = nullptr;
+  if (host) {
+    ce = cudaMalloc(&tmp, n * pt_bytes(fmt) + 128);
+    if (ce == cudaSuccess) ce = cudaMemcpyAsync(tmp, points, n * pt_bytes(fmt), cudaMemcpyHostToDevice, e.stream);
+    if (ce != cudaSuccess) rc = cuda_fail(ce, "upload of the bases", __FILE__, __LINE__);
+  }
+  // slab 0 = the plain set (synchronises the stream), then the upper slabs of a windowed set
+  if (!rc) rc = msm_bases_prepare(host ? tmp : points, fmt, n, tab);
   if (!rc) rc = msm_bases_fill_windows(tab, n, c, W);
-  if (rc) { cudaStreamSynchronize(_eng.stream); cudaFree(tab); return rc; }
+  if (rc) cudaStreamSynchronize(e.stream);
+  if (tmp) cudaFree(tmp);
+  if (rc) {
+    cudaFree(tab);
+    return rc;
+  }
   BasesLayout bl;
   bl.n = n;
   bl.c = c;
   bl.W = W;
   bl.bytes = bytes;
-  _eng.bases[tab] = bl;
+  e.bases[tab] = bl;
   *bases = tab;
   return D377_OK;
 }
 
+int d377_msm_bases_create(const uint8_t* points, int point_format, size_t n, uint8_t** bases) {
+  D377_REQUIRE_READY();
+  return msm_bases_create(points, point_format, n, false, 0, bases, true);
+}
+
+int d377_msm_bases_create_dev(const uint8_t* points, int point_format, size_t n, uint8_t** bases) {
+  D377_REQUIRE_READY();
+  return msm_bases_create(points, point_format, n, false, 0, bases, false);
+}
+
 int d377_msm_bases_create_windowed(const uint8_t* points, int point_format, size_t n, int c, uint8_t** bases) {
   D377_REQUIRE_READY();
-  int W = 0, cc = c;
-  TRY(windowed_args(point_format, n, &cc, &W, bases, points));
-  Engine& e = _eng;
-  const size_t pb = pt_bytes(point_format);
-  uint8_t* tmp = nullptr;
-  D377_CUDA(cudaMalloc(&tmp, n * pb + 128));
-  cudaError_t ce = cudaMemcpyAsync(tmp, points, n * pb, cudaMemcpyHostToDevice, e.stream);
-  if (ce != cudaSuccess) { cudaStreamSynchronize(e.stream); cudaFree(tmp); return cuda_fail(ce, "upload of the bases", __FILE__, __LINE__); }
-  int rc = d377_msm_bases_create_windowed_dev(tmp, point_format, n, c, bases);   // synchronises the stream
-  if (rc) cudaStreamSynchronize(e.stream);
-  cudaFree(tmp);
-  return rc;
+  return msm_bases_create(points, point_format, n, true, c, bases, true);
+}
+
+int d377_msm_bases_create_windowed_dev(const uint8_t* points, int point_format, size_t n, int c, uint8_t** bases) {
+  D377_REQUIRE_READY();
+  return msm_bases_create(points, point_format, n, true, c, bases, false);
 }
 
 int d377_msm_bases_info(const uint8_t* bases, size_t* n, int* c, int* windows, size_t* bytes) {
@@ -1412,10 +1411,11 @@ int d377_msm_bases_destroy(uint8_t* bases) {
 
 // ---- prepared fixed bases ----------------------------------------------------
 // Arguments of d377_fixed_bases_create*, checked before anything is allocated or read;
-// *bytes receives the size of the k tables.
-static int fixed_bases_args(int point_format, size_t k, uint8_t** tables, const uint8_t* points, size_t* bytes) {
-  if (point_format < 0 || point_format > 3) { set_error("bad point_format %d", point_format); return D377_ERR_INVALID_ARG; }
-  if (!tables || !points) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
+// *fmt receives the point format, *bytes the size of the k tables.
+static int fixed_bases_args(int point_format, size_t k, uint8_t** tables, const uint8_t* points, int* fmt,
+                            size_t* bytes) {
+  TRY(parse_format("d377_fixed_bases_create", point_format, kPointFormats, fmt));
+  if (!tables || !points) return null_pointer();
   if (k == 0) { set_error("fixed bases: k = 0"); return D377_ERR_INVALID_ARG; }
   const size_t per = fixed_bases_bytes_per_base();
   if (k > SIZE_MAX / per) {
@@ -1429,8 +1429,9 @@ static int fixed_bases_args(int point_format, size_t k, uint8_t** tables, const 
 // `host`: `points` is host memory, uploaded once the tables are allocated
 static int fixed_bases_create(const uint8_t* points, int point_format, size_t k, uint8_t** tables, bool host) {
   Engine& e = engine();
+  int fmt = 0;
   size_t bytes = 0;
-  TRY(fixed_bases_args(point_format, k, tables, points, &bytes));
+  TRY(fixed_bases_args(point_format, k, tables, points, &fmt, &bytes));
   uint8_t* tab = nullptr;
   cudaError_t ce = cudaMalloc(&tab, bytes);
   if (ce != cudaSuccess) {
@@ -1441,12 +1442,11 @@ static int fixed_bases_create(const uint8_t* points, int point_format, size_t k,
   int rc = D377_OK;
   uint8_t* tmp = nullptr;
   if (host) {
-    ce = cudaMalloc(&tmp, k * pt_bytes(point_format));
-    if (ce == cudaSuccess)
-      ce = cudaMemcpyAsync(tmp, points, k * pt_bytes(point_format), cudaMemcpyHostToDevice, e.stream);
+    ce = cudaMalloc(&tmp, k * pt_bytes(fmt));
+    if (ce == cudaSuccess) ce = cudaMemcpyAsync(tmp, points, k * pt_bytes(fmt), cudaMemcpyHostToDevice, e.stream);
     if (ce != cudaSuccess) rc = cuda_fail(ce, "upload of the fixed bases", __FILE__, __LINE__);
   }
-  if (!rc) rc = fixed_bases_fill(host ? tmp : points, point_format, k, tab);   // synchronises the stream
+  if (!rc) rc = fixed_bases_fill(host ? tmp : points, fmt, k, tab);   // synchronises the stream
   if (rc) cudaStreamSynchronize(e.stream);
   if (tmp) cudaFree(tmp);
   if (rc) {
@@ -1520,9 +1520,7 @@ int check_bases(Engine& e, const uint8_t* points, size_t n, BasesLayout* layout)
 extern "C" {
 
 static int msm_submit_inner(Engine& e, const uint8_t* scalars, const uint8_t* points, int point_format,
-                            size_t n, int slot) {
-  const int fmt_word = point_format;
-  take_sc_mont(point_format);
+                            bool sc_mont, size_t n, int slot) {
   const bool prepared = point_format == D377_PT_BASES;
   size_t pb = pt_bytes(point_format);
   TRY(ensure(e.slot_sc[slot], n * 32 + 32));
@@ -1563,9 +1561,9 @@ static int msm_submit_inner(Engine& e, const uint8_t* scalars, const uint8_t* po
     }
     D377_CUDA(cudaEventRecord(e.ev_chunk[slot][k], e.copy_stream));
   }
-  TRY(msm_enqueue((uint8_t*)e.slot_sc[slot].p, prepared ? points : (const uint8_t*)e.slot_pt[slot].p, fmt_word, n, dres,
-                  dres + 128, (uint32_t*)(dres + 192), nch > 1 ? chunk : 0, e.ev_chunk[slot], true,
-                  n ? e.ev_chunk_sc[slot] : nullptr));
+  TRY(msm_enqueue((uint8_t*)e.slot_sc[slot].p, prepared ? points : (const uint8_t*)e.slot_pt[slot].p, point_format,
+                  sc_mont, n, dres, dres + 128, (uint32_t*)(dres + 192), nch > 1 ? chunk : 0, e.ev_chunk[slot],
+                  true, n ? e.ev_chunk_sc[slot] : nullptr));
   cudaStream_t rs = result_stream(e);
   D377_CUDA(cudaMemcpyAsync(e.h_small + kSmallSlots + 256 * slot, dres, 256, cudaMemcpyDeviceToHost, rs));
   D377_CUDA(cudaEventRecord(e.ev_done[slot], rs));
@@ -1576,16 +1574,13 @@ static int msm_submit_inner(Engine& e, const uint8_t* scalars, const uint8_t* po
 int d377_msm_submit(const uint8_t* scalars, const uint8_t* points, int point_format, size_t n,
                     int slot) {
   D377_REQUIRE_READY_NOJOIN();
-  const int fmt_word = point_format;
-  take_sc_mont(point_format);
-  if (point_format < 0 || point_format > 4) { set_error("bad point_format %d", point_format); return D377_ERR_INVALID_ARG; }
-  if (slot < 0 || slot >= Engine::kSlots) { set_error("slot %d out of range", slot); return D377_ERR_INVALID_ARG; }
-  if (n && (!scalars || !points)) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   Engine& e = _eng;
-  // prepared bases live on the device already: only the scalars are uploaded
-  if (point_format == D377_PT_BASES && n) TRY(check_bases(e, points, n));
+  int fmt = 0;
+  bool sc_mont = false;
+  TRY(msm_args_ok(e, "d377_msm_submit", scalars, points, point_format, n, &fmt, &sc_mont));
+  if (slot < 0 || slot >= Engine::kSlots) { set_error("slot %d out of range", slot); return D377_ERR_INVALID_ARG; }
   if (e.slot_busy[slot]) { set_error("slot %d still in flight: call d377_msm_wait first", slot); return D377_ERR_INVALID_ARG; }
-  int rc = msm_submit_inner(e, scalars, points, fmt_word, n, slot);
+  int rc = msm_submit_inner(e, scalars, points, fmt, sc_mont, n, slot);
   if (rc) drain(e);   // uploads from the caller's buffers may still be running
   return rc;
 }
@@ -1680,9 +1675,8 @@ int d377_batch_normalize(const uint8_t* elements, size_t n, uint8_t* affine) {
 
 int d377_field_batch_deserialize(int field, const uint8_t* bytes, size_t n, uint8_t* out, uint8_t* ok) {
   D377_REQUIRE_READY();
-  if (field != 0 && field != 1) { set_error("field must be 0 (Fq) or 1 (Fr)"); return D377_ERR_INVALID_ARG; }
+  TRY(deserialize_args(field, bytes, n, ok));
   if (n == 0) return D377_OK;
-  if (!bytes || !ok) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   HostIn ins[] = {{bytes, 32}};
   HostOut outs[] = {{out, 32}, {ok, 1}};
   return run_pipelined(n, ins, 1, outs, 2, [&](uint8_t* const* di, uint8_t* const* dout, size_t len) {

@@ -75,36 +75,14 @@ D377_DI void ptv_store(pt_t* p, const pt_t& v) { pt_store(reinterpret_cast<uint8
 // ---- 1. points -> cached ---------------------------------------------------
 constexpr int kBlk = 128;
 
+// Element / XYZ inputs -> cached projective records (small MSMs, no batch normalisation)
 template <int kFmt>
 __global__ void __launch_bounds__(kBlk)
-k_msm_points(const uint8_t* __restrict__ pts, size_t n, cached_t* __restrict__ out,
-             uint32_t* __restrict__ flags) {
-  extern __shared__ uint32_t smem[];
+k_msm_points(const uint8_t* __restrict__ pts, size_t n, cached_t* __restrict__ out) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   pt_t p;
-  if (kFmt == D377_PT_ELEMENT) {
-    p = pt_load_wire(pts + 128 * i);
-  } else if (kFmt == D377_PT_XYZ) {
-    // (X : Y : Z) without T: (XZ : YZ : Z^2 : XY) is the same point in extended coordinates
-    fq_t x = fq_load_wire(pts + 96 * i), y = fq_load_wire(pts + 96 * i + 32), z = fq_load_wire(pts + 96 * i + 64);
-    p.x = fq_mul(x, z);
-    p.y = fq_mul(y, z);
-    p.z = fq_sqr(z);
-    p.t = fq_mul(x, y);
-  } else if (kFmt == D377_PT_AFFINE) {
-    p.x = fq_load_wire(pts + 64 * i);
-    p.y = fq_load_wire(pts + 64 * i + 32);
-    p.z = fq_one();
-    p.t = fq_mul(p.x, p.y);
-  } else {
-    isqrt_smem_t sm = isqrt_smem(smem);
-    bool good = pt_decompress(p, fq_load_raw(pts + 32 * i), sm);
-    if (!good) {
-      atomicOr(flags, 2u);
-      p = pt_identity();
-    }
-  }
+  pt_load_fmt<kFmt>(p, pts, i, isqrt_smem_t{});
   cached_store(out + i, cached_from(p));
 }
 
@@ -117,22 +95,9 @@ k_msm_points_affine(const uint8_t* __restrict__ pts, size_t n, aff4_t* __restric
   extern __shared__ uint32_t smem[];
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  fq_t x, y;
-  if (kFmt == D377_PT_AFFINE) {
-    x = fq_load_wire(pts + 64 * i);
-    y = fq_load_wire(pts + 64 * i + 32);
-  } else {
-    isqrt_smem_t sm = isqrt_smem(smem);
-    pt_t p;
-    bool good = pt_decompress(p, fq_load_raw(pts + 32 * i), sm);
-    if (!good) {
-      atomicOr(flags, 2u);
-      p = pt_identity();
-    }
-    x = p.x;
-    y = p.y;
-  }
-  aff4_store(out + i, niels_from_affine(x, y));
+  pt_t p;
+  if (!pt_load_fmt<kFmt>(p, pts, i, isqrt_smem(smem))) atomicOr(flags, 2u);
+  aff4_store(out + i, niels_from_affine(p.x, p.y));
 }
 
 // Element inputs (projective) -> the same 96 B affine form, by Montgomery's trick with ONE
@@ -1282,15 +1247,11 @@ static void group_windows(int W, int ngroups, int* wlo, int* whi) {
 // adds the record w * N + i (= 2^(c w) P_i, N = the set's stride) into bucket |d| - 1, the
 // groups' bucket sets are reduced like windows, and the tail sums the group results without
 // any doubling.
-static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_format, size_t n,
+static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_format, bool sc_mont, size_t n,
                     uint8_t* out_element, uint8_t* out_encoding, uint32_t* flags /* device, OR-ed */,
                     const cudaEvent_t* scalars_ready = nullptr, const cudaEvent_t* points_ready = nullptr,
                     const BasesLayout* bases = nullptr) {
   Engine& e = engine();
-  // scalars as the reference holds them in memory (Montgomery limbs): converted on the sort
-  // stream into the workspace set before the digits are cut
-  const bool sc_mont = (point_format & D377_SCALARS_MONTGOMERY) != 0;
-  point_format &= ~D377_SCALARS_MONTGOMERY;
   int rc = msm_state_init(e);
   if (rc) return rc;
   MsmState& ms = e.msm;
@@ -1471,6 +1432,8 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
     if (pts_prefetch) D377_CUDA(cudaStreamWaitEvent(ps, ms.ev_tail_done[set], 0));
   }
   D377_CUDA(cudaEventRecord(ms.ev_sort0, ss));
+  // scalars as the reference holds them in memory (Montgomery limbs): converted on the sort
+  // stream into the workspace set before the digits are cut
   if (sc_mont) {
     launch_fr_from_mont(scalars, n, tw + o_sc, ss);
     scalars = tw + o_sc;
@@ -1509,9 +1472,9 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
       launch_points_affine(e, point_format, points, n, want_normalize > 0 ? 4 : 1, ws + o_norm, aff, flags, ps);
     } else {
       if (point_format == D377_PT_ELEMENT)
-        k_msm_points<D377_PT_ELEMENT><<<grid_for(n, kBlk), kBlk, 0, ps>>>(points, n, cached, flags);
+        k_msm_points<D377_PT_ELEMENT><<<grid_for(n, kBlk), kBlk, 0, ps>>>(points, n, cached);
       else
-        k_msm_points<D377_PT_XYZ><<<grid_for(n, kBlk), kBlk, 0, ps>>>(points, n, cached, flags);
+        k_msm_points<D377_PT_XYZ><<<grid_for(n, kBlk), kBlk, 0, ps>>>(points, n, cached);
       D377_LAUNCHED();
     }
     if (pts_prefetch) {
@@ -1607,15 +1570,12 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
 // Enqueue a whole MSM (no host synchronisation).  `flags` (device word, reset by the
 // caller) collects bit 0 = non-canonical scalar, bit 1 = invalid encoding.  The result is
 // complete on result_stream(e).
-int msm_enqueue(const uint8_t* scalars, const uint8_t* points, int point_format, size_t n,
+int msm_enqueue(const uint8_t* scalars, const uint8_t* points, int point_format, bool sc_mont, size_t n,
                 uint8_t* out_element, uint8_t* out_encoding, uint32_t* flags, size_t chunk,
                 const cudaEvent_t* chunk_ready, bool inputs_ready, const cudaEvent_t* scalars_ready_ev) {
   Engine& e = engine();
   const cudaEvent_t no_event = nullptr;
   if (n == 0) return finish(result_stream(e), nullptr, 0, 0, out_element, out_encoding);
-  const int pf = point_format & ~D377_SCALARS_MONTGOMERY;
-  const size_t pbytes = pf == D377_PT_ELEMENT || pf == D377_PT_BASES ? 128
-                        : pf == D377_PT_ENCODING ? 32 : pf == D377_PT_XYZ ? 96 : 64;
   const size_t kMax = (size_t)1 << 26;  // keeps n * W below 2^32
   if (chunk == 0 || chunk > kMax) chunk = kMax;
   size_t nchunks = (n + chunk - 1) / chunk;
@@ -1623,11 +1583,11 @@ int msm_enqueue(const uint8_t* scalars, const uint8_t* points, int point_format,
   // prepared bases: the set's layout (a windowed set keeps its stride N in every chunk, whose
   // records start at points + 128 * lo)
   BasesLayout layout;
-  if (pf == D377_PT_BASES) {
+  if (point_format == D377_PT_BASES) {
     int rc = check_bases(e, points, n, &layout);
     if (rc) return rc;
   }
-  const BasesLayout* bl = pf == D377_PT_BASES ? &layout : nullptr;
+  const BasesLayout* bl = point_format == D377_PT_BASES ? &layout : nullptr;
   // inputs_ready: the inputs depend on nothing but chunk_ready[k] (or on nothing)
   auto ready_of = [&](size_t k) -> const cudaEvent_t* {
     return !inputs_ready ? nullptr : chunk_ready ? &chunk_ready[k] : &no_event;
@@ -1639,14 +1599,14 @@ int msm_enqueue(const uint8_t* scalars, const uint8_t* points, int point_format,
   };
   if (nchunks == 1) {
     if (chunk_ready) D377_CUDA(cudaStreamWaitEvent(e.stream, chunk_ready[0], 0));
-    return msm_once(scalars, points, point_format, n, out_element, out_encoding, flags, sc_ready_of(0), ready_of(0),
-                    bl);
+    return msm_once(scalars, points, point_format, sc_mont, n, out_element, out_encoding, flags, sc_ready_of(0),
+                    ready_of(0), bl);
   }
   pt_t* partials = (pt_t*)(e.d_small + kSmallPartials);  // up to 16 chunk results
   for (size_t k = 0; k < nchunks; k++) {
     size_t lo = k * chunk, len = std::min(chunk, n - lo);
     if (chunk_ready) D377_CUDA(cudaStreamWaitEvent(e.stream, chunk_ready[k], 0));
-    int rc = msm_once(scalars + 32 * lo, points + pbytes * lo, point_format, len,
+    int rc = msm_once(scalars + 32 * lo, points + pt_bytes(point_format) * lo, point_format, sc_mont, len,
                       (uint8_t*)(partials + k), nullptr, flags, sc_ready_of(k), ready_of(k), bl);
     if (rc) return rc;
   }
@@ -1670,23 +1630,26 @@ int msm_check_flags(uint32_t flags) {
   return D377_OK;
 }
 
-static int msm_args_ok(Engine& e, const uint8_t* scalars, const uint8_t* points, int point_format, size_t n) {
-  if (point_format >= 0) point_format &= ~D377_SCALARS_MONTGOMERY;
-  if (point_format < 0 || point_format > 4) { set_error("bad point_format %d", point_format); return D377_ERR_INVALID_ARG; }
+int msm_args_ok(Engine& e, const char* who, const uint8_t* scalars, const uint8_t* points, int point_format,
+                size_t n, int* fmt, bool* sc_mont) {
+  int rc = parse_format(who, point_format, kPointFormats | fmt_set(D377_PT_BASES), fmt, sc_mont);
+  if (rc) return rc;
   if (n && (!scalars || !points)) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
-  if (point_format == D377_PT_BASES && n) return check_bases(e, points, n);
+  if (*fmt == D377_PT_BASES && n) return check_bases(e, points, n);
   return D377_OK;
 }
 
 int msm_dev(const uint8_t* scalars, const uint8_t* points, int point_format, size_t n,
             uint8_t* out_element, uint8_t* out_encoding) {
   Engine& e = engine();
-  int rc = msm_args_ok(e, scalars, points, point_format, n);
+  int fmt = 0;
+  bool sc_mont = false;
+  int rc = msm_args_ok(e, "d377_msm_dev", scalars, points, point_format, n, &fmt, &sc_mont);
   if (rc) return rc;
   uint32_t* dflags = (uint32_t*)(e.d_small + kSmallFlags);
   uint32_t* hflags = (uint32_t*)(e.h_small + kSmallFlags);
   D377_CUDA(cudaMemsetAsync(dflags, 0, 4, e.stream));
-  rc = msm_enqueue(scalars, points, point_format, n, out_element, out_encoding, dflags);
+  rc = msm_enqueue(scalars, points, fmt, sc_mont, n, out_element, out_encoding, dflags);
   if (rc) return rc;
   // status word: the only host read-back of the pipeline
   cudaStream_t rs = result_stream(e);
@@ -1700,10 +1663,12 @@ int msm_dev(const uint8_t* scalars, const uint8_t* points, int point_format, siz
 int msm_dev_async(const uint8_t* scalars, const uint8_t* points, int point_format, size_t n,
                   uint8_t* out_element, uint8_t* out_encoding, int flags) {
   Engine& e = engine();
-  int rc = msm_args_ok(e, scalars, points, point_format, n);
+  int fmt = 0;
+  bool sc_mont = false;
+  int rc = msm_args_ok(e, "d377_msm_dev_async", scalars, points, point_format, n, &fmt, &sc_mont);
   if (rc) return rc;
   e.async_status_dirty = true;
-  return msm_enqueue(scalars, points, point_format, n, out_element, out_encoding,
+  return msm_enqueue(scalars, points, fmt, sc_mont, n, out_element, out_encoding,
                      (uint32_t*)(e.d_small + kSmallAsyncFlags), 0, nullptr,
                      (flags & D377_MSM_INPUTS_READY) != 0);
 }

@@ -59,16 +59,11 @@ static int worker_wait(Engine& e) {
   return e.wrc;
 }
 
-static size_t point_bytes(int fmt) {
-  fmt &= ~D377_SCALARS_MONTGOMERY;
-  return fmt == D377_PT_ELEMENT ? 128 : fmt == D377_PT_ENCODING ? 32 : fmt == D377_PT_XYZ ? 96 : 64;
-}
-
 // One GPU's share: a Pippenger over its slice, the partial sum sent to the gathering
 // engine.  Runs on the engine's worker thread; returns after the GPU has finished (the
 // status word has to be read anyway).
 static int leg(Engine& e, Engine& root, int index, bool host, const uint8_t* scalars,
-               const uint8_t* points, int point_format, size_t n) {
+               const uint8_t* points, int point_format, bool sc_mont, size_t n) {
   EngineScope scope(e);
   uint8_t* dres = e.d_small + kSmallResult;
   uint32_t* dflags = (uint32_t*)(e.d_small + kSmallFlags);
@@ -89,7 +84,7 @@ static int leg(Engine& e, Engine& root, int index, bool host, const uint8_t* sca
   if (host && n) {
     // same upload pipeline as d377_msm_submit: sub-MSM chunks, the Pippenger of chunk k
     // overlaps the upload of chunk k+1
-    const size_t pb = point_bytes(point_format);
+    const size_t pb = pt_bytes(point_format);
     if ((rc = ensure(e.slot_sc[0], n * 32 + 32))) return rc;
     if ((rc = ensure(e.slot_pt[0], n * pb + 128))) return rc;
     // A slice of a multi-GPU call is link-bound (all GPUs pull from the same host memory),
@@ -126,8 +121,8 @@ static int leg(Engine& e, Engine& root, int index, bool host, const uint8_t* sca
   // compute kernel, no copy in between; without it the sum lands locally and is copied.
   uint8_t* dst = root.d_small + kSmallGather + 128 * index;
   const bool direct = &e == &root || ((e.peer_mask >> root.device) & 1ull);
-  rc = msm_enqueue(dsc, dpt, point_format, n, direct ? dst : dres, nullptr, dflags, chunk, ready, ready != nullptr,
-                   ready ? e.ev_chunk_sc[0] : nullptr);
+  rc = msm_enqueue(dsc, dpt, point_format, sc_mont, n, direct ? dst : dres, nullptr, dflags, chunk, ready,
+                   ready != nullptr, ready ? e.ev_chunk_sc[0] : nullptr);
   if (rc) return fail(rc);
   cudaStream_t rs = result_stream(e);
   if (!direct) ce = cudaMemcpyPeerAsync(dst, root.device, dres, e.device, 128, rs);
@@ -147,11 +142,11 @@ static int msm_multi(bool host, const uint8_t* const* scalars, const uint8_t* co
     set_error("d377_msm_multi: ngpu = %d but %d device(s) initialised (d377_init_multi)", ngpu, have);
     return have ? D377_ERR_INVALID_ARG : D377_ERR_NOT_INITIALISED;
   }
-  const int pf = point_format < 0 ? point_format : (point_format & ~D377_SCALARS_MONTGOMERY);
-  if (pf < 0 || pf > 3) {
-    set_error("d377_msm_multi: point_format %d (prepared bases belong to one device; use d377_msm on it)", point_format);
-    return D377_ERR_INVALID_ARG;
-  }
+  // prepared bases belong to one device: d377_msm takes them
+  int pf = 0;
+  bool sc_mont = false;
+  int rc = parse_format("d377_msm_multi", point_format, kPointFormats, &pf, &sc_mont);
+  if (rc) return rc;
   Engine* eng[8];
   for (int k = 0; k < ngpu; k++) {
     eng[k] = engine_for(devs[k]);
@@ -164,9 +159,8 @@ static int msm_multi(bool host, const uint8_t* const* scalars, const uint8_t* co
     Engine* e = eng[k];
     const uint8_t *s = scalars[k], *p = points[k];
     const size_t nk = n[k];
-    worker_post(*e, [=, &root]() { return leg(*e, root, k, host, s, p, point_format, nk); });
+    worker_post(*e, [=, &root]() { return leg(*e, root, k, host, s, p, pf, sc_mont, nk); });
   }
-  int rc = D377_OK;
   for (int k = 0; k < ngpu; k++) {
     int r = worker_wait(*eng[k]);
     if (r && !rc) rc = r;
@@ -205,7 +199,7 @@ static Engine* g_gather_root = nullptr;
 static int g_ring = 0;
 
 static int leg_async(Engine& e, Engine& root, int index, int ring, const uint8_t* scalars,
-                     const uint8_t* points, int point_format, size_t n) {
+                     const uint8_t* points, int point_format, bool sc_mont, size_t n) {
   EngineScope scope(e);
   uint8_t* dres = e.d_small + kSmallResult;
   uint8_t* dst = root.d_small + kGatherOff[ring] + 128 * index;
@@ -215,7 +209,7 @@ static int leg_async(Engine& e, Engine& root, int index, int ring, const uint8_t
   // the gather area may still be read by the sum of the call that used it last (the tail that
   // writes it runs on the result stream, so the wait goes there before the MSM is enqueued)
   if (g_gather_used[ring]) D377_CUDA(cudaStreamWaitEvent(rs, g_gather_free[ring], 0));
-  int rc = msm_enqueue(scalars, points, point_format, n, direct ? dst : dres, nullptr,
+  int rc = msm_enqueue(scalars, points, point_format, sc_mont, n, direct ? dst : dres, nullptr,
                        (uint32_t*)(e.d_small + kSmallAsyncFlags), 0, nullptr, true);
   if (rc) return rc;
   if (!direct) D377_CUDA(cudaMemcpyPeerAsync(dst, root.device, dres, e.device, 128, rs));
@@ -231,8 +225,10 @@ static int msm_multi_async(const uint8_t* const* scalars, const uint8_t* const* 
     set_error("d377_msm_multi_dev_async: ngpu = %d but %d device(s) initialised (d377_init_multi)", ngpu, have);
     return have ? D377_ERR_INVALID_ARG : D377_ERR_NOT_INITIALISED;
   }
-  const int pf = point_format < 0 ? point_format : (point_format & ~D377_SCALARS_MONTGOMERY);
-  if (pf < 0 || pf > 3) { set_error("d377_msm_multi_dev_async: bad point_format %d", point_format); return D377_ERR_INVALID_ARG; }
+  int pf = 0;
+  bool sc_mont = false;
+  int rc = parse_format("d377_msm_multi_dev_async", point_format, kPointFormats, &pf, &sc_mont);
+  if (rc) return rc;
   Engine* eng[8];
   for (int k = 0; k < ngpu; k++) {
     eng[k] = engine_for(devs[k]);
@@ -259,9 +255,8 @@ static int msm_multi_async(const uint8_t* const* scalars, const uint8_t* const* 
     Engine* e = eng[k];
     const uint8_t *sp = scalars[k], *pp = points[k];
     const size_t nk = n[k];
-    worker_post(*e, [=, &root]() { return leg_async(*e, root, k, ring, sp, pp, point_format, nk); });
+    worker_post(*e, [=, &root]() { return leg_async(*e, root, k, ring, sp, pp, pf, sc_mont, nk); });
   }
-  int rc = D377_OK;
   for (int k = 0; k < ngpu; k++) {
     int r = worker_wait(*eng[k]);
     if (r && !rc) rc = r;
@@ -319,12 +314,14 @@ int d377_multi_sync(void) {
 int d377_msm_multi(const uint8_t* scalars, const uint8_t* points, int point_format, size_t n, int ngpu,
                    uint8_t out_element[128], uint8_t out_encoding[32]) {
   if (ngpu < 1 || ngpu > 8) { set_error("d377_msm_multi: ngpu must be 1..8"); return D377_ERR_INVALID_ARG; }
-  const int pf = point_format < 0 ? point_format : (point_format & ~D377_SCALARS_MONTGOMERY);
-  if (pf < 0 || pf > 3) { set_error("d377_msm_multi: bad point_format %d", point_format); return D377_ERR_INVALID_ARG; }
+  int pf = 0;
+  bool sc_mont = false;   // passed on in the format word
+  const int rc = parse_format("d377_msm_multi", point_format, kPointFormats, &pf, &sc_mont);
+  if (rc) return rc;
   if (n && (!scalars || !points)) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   const uint8_t *sc[8], *pt[8];
   size_t cnt[8];
-  const size_t pb = point_bytes(point_format);
+  const size_t pb = pt_bytes(pf);
   // contiguous slices whose sizes differ by at most one (dist.shard_range)
   const size_t base = n / (size_t)ngpu, rem = n % (size_t)ngpu;
   size_t lo = 0;

@@ -13,6 +13,7 @@
 // The addition law is complete (a = -1 is a square, d a non-square mod q), so
 // none of these has exceptional inputs and every thread runs the same code.
 #pragma once
+#include "engine.h"
 #include "isqrt.cuh"
 
 // Every coordinate kept in a pt_t / niels_t / cached_t is a storage-class value (< 2q,
@@ -320,6 +321,35 @@ D377_DI bool pt_decompress(pt_t& out, const fq_raw_t& s_raw, const isqrt_smem_t&
   out.z = fq_one();
   out.t = fq_mul(out.x, out.y);
   return ok;
+}
+
+// Element i of a caller's point array in format kFmt (D377_PT_ELEMENT, _ENCODING, _AFFINE or
+// _XYZ) -> extended coordinates.  An invalid encoding reads as the identity and returns false;
+// `sm` is used by encodings only.
+template <int kFmt>
+D377_DI bool pt_load_fmt(pt_t& p, const uint8_t* pts, size_t i, const isqrt_smem_t& sm) {
+  const uint8_t* b = pts + d377::pt_bytes(kFmt) * i;
+  if (kFmt == D377_PT_ENCODING) {
+    const bool good = pt_decompress(p, fq_load_raw(b), sm);
+    p = pt_select(good, p, pt_identity());
+    return good;
+  }
+  if (kFmt == D377_PT_ELEMENT) {
+    p = pt_load_wire(b);
+  } else if (kFmt == D377_PT_AFFINE) {
+    p.x = fq_load_wire(b);
+    p.y = fq_load_wire(b + 32);
+    p.z = fq_one();
+    p.t = fq_mul(p.x, p.y);
+  } else {
+    // (X : Y : Z) without T: (XZ : YZ : Z^2 : XY) is the same point in extended coordinates
+    fq_t x = fq_load_wire(b), y = fq_load_wire(b + 32), z = fq_load_wire(b + 64);
+    p.x = fq_mul(x, z);
+    p.y = fq_mul(y, z);
+    p.z = fq_sqr(z);
+    p.t = fq_mul(x, y);
+  }
+  return true;
 }
 
 // ark_curve/elligator.rs:15-54: r0 (Montgomery form) -> the Jacobi-quartic pair (s, t).

@@ -22,18 +22,9 @@ k_scalar_mul(const uint8_t* __restrict__ pts, const uint8_t* __restrict__ scalar
   if (i >= n) return;
   isqrt_smem_t sm = isqrt_smem(smem);
   pt_t p;
-  if (kFmt == D377_PT_ELEMENT) {
-    p = pt_load_wire(pts + 128 * i);
-  } else if (kFmt == D377_PT_AFFINE) {
-    p.x = fq_load_wire(pts + 64 * i);
-    p.y = fq_load_wire(pts + 64 * i + 32);
-    p.z = fq_one();
-    p.t = fq_mul(p.x, p.y);
-  } else {
-    bool good = pt_decompress(p, fq_load_raw(pts + 32 * i), sm);
-    p = pt_select(good, p, pt_identity());
-    if (ok) ok[i] = good ? 1 : 0;
-  }
+  const bool good = pt_load_fmt<kFmt>(p, pts, i, sm);
+  // only encodings can fail to decode; the host entry point fills `ok` for the other formats
+  if (kFmt == D377_PT_ENCODING && ok) ok[i] = good ? 1 : 0;
   fq_raw_t k = fq_load_raw(scalars + 32 * i);
   pt_t r = pt_scalar_mul(p, k);
   D377_DBG_POINT(r);
@@ -75,27 +66,7 @@ k_fb_load(const uint8_t* __restrict__ pts, size_t k, pt_t* __restrict__ start, u
   size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= k) return;
   pt_t p;
-  if (kFmt == D377_PT_ELEMENT) {
-    p = pt_load_wire(pts + 128 * j);
-  } else if (kFmt == D377_PT_AFFINE) {
-    p.x = fq_load_wire(pts + 64 * j);
-    p.y = fq_load_wire(pts + 64 * j + 32);
-    p.z = fq_one();
-    p.t = fq_mul(p.x, p.y);
-  } else if (kFmt == D377_PT_XYZ) {
-    // (X : Y : Z) without T: (XZ : YZ : Z^2 : XY) is the same point in extended coordinates
-    fq_t x = fq_load_wire(pts + 96 * j), y = fq_load_wire(pts + 96 * j + 32), z = fq_load_wire(pts + 96 * j + 64);
-    p.x = fq_mul(x, z);
-    p.y = fq_mul(y, z);
-    p.z = fq_sqr(z);
-    p.t = fq_mul(x, y);
-  } else {
-    bool good = pt_decompress(p, fq_load_raw(pts + 32 * j), isqrt_smem(smem));
-    if (!good) {
-      atomicOr(flags, 1u);
-      p = pt_identity();
-    }
-  }
+  if (!pt_load_fmt<kFmt>(p, pts, j, isqrt_smem(smem))) atomicOr(flags, 1u);
   D377_DBG_POINT(p);
   start[j] = p;
 }

@@ -12,7 +12,7 @@ from typing import Optional, Tuple
 import torch
 
 from . import _lib, api
-from ._lib import OUT_ELEMENT, OUT_ENCODING, PT_ELEMENT, SCALARS_MONTGOMERY, check
+from ._lib import OUT_ELEMENT, OUT_WIDTH, PT_ELEMENT, PT_WIDTH, SCALARS_MONTGOMERY, check
 
 _ext_streams = {}
 
@@ -61,7 +61,6 @@ def _then_torch() -> None:
     torch.cuda.current_stream().wait_stream(engine_stream())
 
 
-_W = {0: 128, 1: 32, 2: 64, 3: 96}
 
 
 def decompress(enc: torch.Tensor, out: Optional[torch.Tensor] = None,
@@ -88,7 +87,7 @@ def decompress_fmt(enc: torch.Tensor, out_format: int, out: Optional[torch.Tenso
                    ok: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
     """d377_batch_decompress_fmt_dev: Element (128 B) or AffinePoint (64 B) outputs."""
     n = _chk(enc, 32, "enc")
-    out = torch.empty((n, _W[out_format]), dtype=torch.uint8, device=enc.device) if out is None else out
+    out = torch.empty((n, PT_WIDTH[out_format]), dtype=torch.uint8, device=enc.device) if out is None else out
     ok = torch.empty((n,), dtype=torch.uint8, device=enc.device) if ok is None else ok
     _after_torch()
     check(_lib.load().d377_batch_decompress_fmt_dev(enc.data_ptr(), n, out_format, out.data_ptr(),
@@ -100,7 +99,7 @@ def decompress_fmt(enc: torch.Tensor, out_format: int, out: Optional[torch.Tenso
 def compress_fmt(points: torch.Tensor, point_format: int,
                  out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """d377_batch_compress_fmt_dev: Element, AffinePoint or X||Y||Z inputs."""
-    n = _chk(points, _W[point_format], "points")
+    n = _chk(points, PT_WIDTH[point_format], "points")
     out = torch.empty((n, 32), dtype=torch.uint8, device=points.device) if out is None else out
     _after_torch()
     check(_lib.load().d377_batch_compress_fmt_dev(points.data_ptr(), point_format, n, out.data_ptr()))
@@ -111,7 +110,7 @@ def compress_fmt(points: torch.Tensor, point_format: int,
 def encode_to_curve(r: torch.Tensor, out_format: int = OUT_ELEMENT,
                     out: Optional[torch.Tensor] = None) -> torch.Tensor:
     n = _chk(r, 32, "r")
-    out = torch.empty((n, _W[0] if out_format == OUT_ELEMENT else 32), dtype=torch.uint8,
+    out = torch.empty((n, OUT_WIDTH[out_format]), dtype=torch.uint8,
                       device=r.device) if out is None else out
     _after_torch()
     check(_lib.load().d377_batch_encode_to_curve_dev(r.data_ptr(), n, out.data_ptr(), out_format))
@@ -123,7 +122,7 @@ def hash_to_curve(r1: torch.Tensor, r2: torch.Tensor, out_format: int = OUT_ELEM
                   out: Optional[torch.Tensor] = None) -> torch.Tensor:
     n = _chk(r1, 32, "r1")
     _chk(r2, 32, "r2")
-    out = torch.empty((n, 128 if out_format == OUT_ELEMENT else 32), dtype=torch.uint8,
+    out = torch.empty((n, OUT_WIDTH[out_format]), dtype=torch.uint8,
                       device=r1.device) if out is None else out
     _after_torch()
     check(_lib.load().d377_batch_hash_to_curve_dev(r1.data_ptr(), r2.data_ptr(), n, out.data_ptr(),
@@ -135,9 +134,9 @@ def hash_to_curve(r1: torch.Tensor, r2: torch.Tensor, out_format: int = OUT_ELEM
 def scalar_mul(points: torch.Tensor, scalars: torch.Tensor, point_format: int = PT_ELEMENT,
                out_format: int = OUT_ELEMENT, out: Optional[torch.Tensor] = None,
                ok: Optional[torch.Tensor] = None) -> torch.Tensor:
-    n = _chk(points, _W[point_format], "points")
+    n = _chk(points, PT_WIDTH[point_format], "points")
     _chk(scalars, 32, "scalars")
-    out = torch.empty((n, 128 if out_format == OUT_ELEMENT else 32), dtype=torch.uint8,
+    out = torch.empty((n, OUT_WIDTH[out_format]), dtype=torch.uint8,
                       device=points.device) if out is None else out
     _after_torch()
     check(_lib.load().d377_batch_scalar_mul_dev(points.data_ptr(), point_format, scalars.data_ptr(),
@@ -150,7 +149,7 @@ def scalar_mul(points: torch.Tensor, scalars: torch.Tensor, point_format: int = 
 def fixed_base_mul(scalars: torch.Tensor, out_format: int = OUT_ELEMENT,
                    out: Optional[torch.Tensor] = None) -> torch.Tensor:
     n = _chk(scalars, 32, "scalars")
-    out = torch.empty((n, 128 if out_format == OUT_ELEMENT else 32), dtype=torch.uint8,
+    out = torch.empty((n, OUT_WIDTH[out_format & ~SCALARS_MONTGOMERY]), dtype=torch.uint8,
                       device=scalars.device) if out is None else out
     _after_torch()
     check(_lib.load().d377_fixed_base_mul_dev(scalars.data_ptr(), n, out.data_ptr(), out_format))
@@ -171,8 +170,8 @@ def fixed_bases_mul(bases, scalars: torch.Tensor, out_format: int = OUT_ELEMENT,
         n = scalars.shape[0]
     else:
         raise ValueError("scalars must have shape [n, %d, 32], got %r" % (bases.k, tuple(scalars.shape)))
-    width = 32 if (out_format & ~SCALARS_MONTGOMERY) == OUT_ENCODING else 128
-    out = torch.empty((n, width), dtype=torch.uint8, device=scalars.device) if out is None else out
+    out = torch.empty((n, OUT_WIDTH[out_format & ~SCALARS_MONTGOMERY]), dtype=torch.uint8,
+                      device=scalars.device) if out is None else out
     _after_torch()
     check(_lib.load().d377_fixed_bases_mul_dev(bases._handle(), scalars.data_ptr(), n, out.data_ptr(), out_format))
     _then_torch()
@@ -244,7 +243,7 @@ def msm_async(scalars: torch.Tensor, points: torch.Tensor, point_format: int = P
             raise ValueError("fewer prepared bases than scalars")
         pptr, point_format = points.ptr, 4
     else:
-        if _chk(points, _W[point_format], "points") != n:
+        if _chk(points, PT_WIDTH[point_format], "points") != n:
             raise ValueError("scalars and points differ in length")
         pptr = points.data_ptr()
     oe = torch.empty((128,), dtype=torch.uint8, device=scalars.device) if out_element is None else out_element
@@ -278,7 +277,7 @@ def msm_multi(scalars, points, point_format: int = PT_ELEMENT):
     ns = []
     for s_k, p_k in zip(scalars, points):
         n_k = _chk(s_k, 32, "scalars")
-        if _chk(p_k, _W[point_format], "points") != n_k:
+        if _chk(p_k, PT_WIDTH[point_format], "points") != n_k:
             raise ValueError("scalars and points differ in length")
         ns.append(n_k)
     for s_k in scalars:                       # inputs produced by torch: wait for them
@@ -302,7 +301,7 @@ def msm_multi_async(scalars, points, point_format: int = PT_ELEMENT,
     k = len(scalars)
     ns = [_chk(s_k, 32, "scalars") for s_k in scalars]
     for p_k, n_k in zip(points, ns):
-        if _chk(p_k, _W[point_format], "points") != n_k:
+        if _chk(p_k, PT_WIDTH[point_format], "points") != n_k:
             raise ValueError("scalars and points differ in length")
     dev0 = scalars[0].device
     oe = torch.empty((128,), dtype=torch.uint8, device=dev0) if out_element is None else out_element
@@ -329,7 +328,7 @@ def msm(scalars: torch.Tensor, points: torch.Tensor, point_format: int = PT_ELEM
             raise ValueError("fewer prepared bases than scalars")
         pptr, point_format = points.ptr, 4                        # D377_PT_BASES
     else:
-        if _chk(points, _W[point_format], "points") != n:
+        if _chk(points, PT_WIDTH[point_format], "points") != n:
             raise ValueError("scalars and points differ in length")
         pptr = points.data_ptr()
     oe = torch.empty((128,), dtype=torch.uint8, device=scalars.device)
