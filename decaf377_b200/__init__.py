@@ -11,6 +11,7 @@ from .api import (  # noqa: F401
     init, init_multi, set_device, get_device, device_list, shutdown, sync, join, launch_count,
     imad_peak, msm_set_window, msm_set_host_chunks, msm_set_tail_overlap, debug_build, debug_counts,
     batch_sub, batch_neg, batch_double, batch_on_curve, fq_batch_from_le_bytes_mod_order, msm_multi, batch_msm,
+    msm_segmented, msm_segmented_last,
     msm_set_normalize, msm_set_groups,
     msm_stage_info, msm_timeline, pinned_empty, pinned_copy,
     batch_decompress, batch_compress, batch_compress_fmt, batch_affine_serialize, batch_affine_deserialize,

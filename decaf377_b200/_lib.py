@@ -57,6 +57,8 @@ _SIGS = {
     "d377_multi_sync": [],
     "d377_batch_msm": [u8p, u8p, C.c_int, u8p, C.c_size_t, u8p, C.c_int, u8p],
     "d377_batch_msm_dev": [u8p, u8p, C.c_int, u8p, C.c_size_t, C.c_size_t, u8p, C.c_int, u8p],
+    "d377_msm_segmented": [u8p, u8p, C.c_int, u8p, C.c_size_t, u8p, C.c_int, u8p],
+    "d377_msm_segmented_last": [C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_size_t)],
     "d377_msm_set_window": [C.c_int],
     "d377_msm_set_host_chunks": [C.c_int],
     "d377_host_free": [C.c_void_p],
@@ -107,7 +109,7 @@ for _n in ["d377_batch_decompress", "d377_batch_compress", "d377_batch_encode_to
            "d377_batch_encode_to_curve_wide",
            "d377_batch_hash_to_curve_wide", "d377_fq_batch_from_le_bytes_mod_order",
            "d377_batch_sub", "d377_batch_neg", "d377_batch_double", "d377_batch_on_curve",
-           "d377_batch_decompress_fmt", "d377_batch_compress_fmt"]:
+           "d377_batch_decompress_fmt", "d377_batch_compress_fmt", "d377_msm_segmented"]:
     _SIGS[_n + "_dev"] = _SIGS[_n]
 
 EXPORTS = sorted(list(_SIGS) + ["d377_stream", "d377_result_stream", "d377_last_error",

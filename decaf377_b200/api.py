@@ -615,6 +615,34 @@ def batch_msm(scalars, points, offsets, point_format: int = PT_ELEMENT, out_form
     return (out, ok) if return_ok else out
 
 
+def msm_segmented(scalars, points, offsets, point_format: int = PT_ELEMENT, out_format: int = OUT_ELEMENT,
+                  return_ok: bool = False, scalars_montgomery: bool = False):
+    """d377_msm_segmented: the results of ``batch_msm`` (MSM j covers pairs
+    offsets[j]..offsets[j+1]) from one segmented Pippenger over all segments -- the call for
+    many MSMs of tens to tens of thousands of pairs.  Returns [nmsm, 128 | 32] (and ok [nmsm])."""
+    _ensure_init()
+    sc = _arr(scalars, 32, "scalars")
+    pts = _arr(points, PT_WIDTH[point_format], "points")
+    off = np.ascontiguousarray(offsets, dtype=np.uint32)
+    if off.ndim != 1 or off.size < 1:
+        raise ValueError("offsets must hold nmsm + 1 entries")
+    nmsm = off.size - 1
+    if int(off[-1]) > min(sc.shape[0], pts.shape[0]):
+        raise ValueError("offsets reach past the end of the inputs")
+    out = np.empty((nmsm, OUT_WIDTH[out_format]), np.uint8)
+    ok = np.empty((nmsm,), np.uint8)
+    check(_lib.load().d377_msm_segmented(_ptr(sc), _ptr(pts), point_format | _mont(scalars_montgomery),
+                                         off.ctypes.data_as(C.c_void_p), nmsm, _ptr(out), out_format, _ptr(ok)))
+    return (out, ok) if return_ok else out
+
+
+def msm_segmented_last() -> Tuple[int, int, int]:
+    """d377_msm_segmented_last: (c, W, chunks) of the most recent segmented MSM."""
+    c, w, k = C.c_int(), C.c_int(), C.c_size_t()
+    check(_lib.load().d377_msm_segmented_last(C.byref(c), C.byref(w), C.byref(k)))
+    return c.value, w.value, k.value
+
+
 def msm_submit(scalars, points, point_format: int = PT_ELEMENT, slot: int = 0,
                scalars_montgomery: bool = False) -> None:
     """d377_msm_submit: start an MSM over host buffers without waiting (slots 0..3).

@@ -101,6 +101,15 @@ struct Engine {
   DevBuf sc_canon;
   // d377_batch_msm: products, their decode status, segment sums; host-call staging
   DevBuf bm_prod, bm_ok, bm_sum, bm_sc, bm_pt, bm_off, bm_out, bm_okout;
+  // d377_msm_segmented*: workspace (converted points, one chunk's sort and tail), pinned
+  // staging of the host offsets with the event after their upload, and the geometry of the
+  // most recent call (d377_msm_segmented_last)
+  DevBuf seg_ws;
+  void* seg_off_host = nullptr;
+  size_t seg_off_cap = 0;
+  cudaEvent_t ev_seg_off = nullptr;
+  int seg_last_c = 0, seg_last_W = 0;
+  size_t seg_last_chunks = 0;
   // fixed-base table (niels, affine) and its geometry
   void* fb_table = nullptr;
   void* fb_table_jq = nullptr;   // the same multiples on the Jacobi quartic (encoding output)
@@ -293,6 +302,13 @@ int msm_bases_prepare(const uint8_t* points, int point_format, size_t n, uint8_t
 int msm_bases_fill_windows(uint8_t* table, size_t n, int c, int W);
 int msm_windowed_c(size_t n);    // window width of a windowed set when the caller passes c = 0
 bool msm_last_windowed();
+// d377_msm_segmented*: the window width for these (validated, host) offsets -- refused with
+// D377_ERR_INVALID_ARG when some segment does not fit a chunk of its own -- and the enqueue
+// on the engine stream (device scalars, points, out, ok; host offsets)
+int msm_segmented_width(Engine& e, int fmt, const uint32_t* offsets, size_t nmsm, int* c);
+int msm_segmented_enqueue(const uint8_t* scalars, const uint8_t* points, int fmt, bool sc_mont,
+                          const uint32_t* offsets, size_t nmsm, int c, uint8_t* out, int out_format, uint8_t* ok);
+int msm_segmented_last(int* c, int* W, size_t* chunks);
 int msm_stage_info(float* ms, int* c, int* W, uint64_t* n);
 int msm_timeline(float* ms, int cap, int* ngroups);
 bool msm_last_mixed();

@@ -312,11 +312,18 @@ static void engine_destroy(Engine& e) {
                     &e.slot_pt[0], &e.slot_pt[1], &e.st_in[0][0], &e.st_in[0][1], &e.st_in[0][2],
                     &e.st_in[1][0], &e.st_in[1][1], &e.st_in[1][2], &e.st_out[0][0], &e.st_out[0][1],
                     &e.st_out[1][0], &e.st_out[1][1], &e.sum_ws[0], &e.sum_ws[1], &e.bm_prod, &e.bm_ok,
-                    &e.bm_sum, &e.bm_sc, &e.bm_pt, &e.bm_off, &e.bm_out, &e.bm_okout}) {
+                    &e.bm_sum, &e.bm_sc, &e.bm_pt, &e.bm_off, &e.bm_out, &e.bm_okout, &e.seg_ws}) {
     if (b->p) cudaFree(b->p);
     b->p = nullptr;
     b->cap = 0;
   }
+  if (e.seg_off_host) cudaFreeHost(e.seg_off_host);
+  e.seg_off_host = nullptr;
+  e.seg_off_cap = 0;
+  if (e.ev_seg_off) cudaEventDestroy(e.ev_seg_off);
+  e.ev_seg_off = nullptr;
+  e.seg_last_c = e.seg_last_W = 0;
+  e.seg_last_chunks = 0;
   // prepared bases still alive belong to the library (header contract): release them
   for (auto& kv : e.bases) cudaFree(const_cast<void*>(kv.first));
   e.bases.clear();
@@ -960,6 +967,76 @@ int d377_batch_msm(const uint8_t* scalars, const uint8_t* points, int point_form
   int rc = body();
   if (rc) drain(e);
   return rc;
+}
+
+// ---- many independent MSMs in one segmented Pippenger ---------------------------------------
+// Both forms: formats, null pointers (n = offsets[nmsm]), the host offsets (offsets[0] = 0,
+// non-decreasing, n <= 0xfffffff0) and the window width.  Nothing is read or launched before
+// this passes; nmsm = 0 passes with nothing else checked but the formats.
+static int msm_segmented_args(Engine& e, const uint8_t* scalars, const uint8_t* points, int point_format,
+                              const uint32_t* offsets, size_t nmsm, const uint8_t* out, int out_format, int* pf,
+                              bool* sc_mont, int* c) {
+  TRY(parse_format("d377_msm_segmented", point_format, kPointFormats, pf, sc_mont));
+  TRY(parse_format("d377_msm_segmented", out_format, kOutFormats, nullptr));
+  if (nmsm == 0) return D377_OK;
+  if (!offsets || !out) return null_pointer();
+  if (nmsm > 0x7fffffffull) { set_error("d377_msm_segmented: too many segments"); return D377_ERR_INVALID_ARG; }
+  if (offsets[0] != 0) { set_error("d377_msm_segmented: offsets[0] must be 0"); return D377_ERR_INVALID_ARG; }
+  for (size_t j = 0; j < nmsm; j++)
+    if (offsets[j + 1] < offsets[j]) {
+      set_error("d377_msm_segmented: offsets must not decrease (segment %zu)", j);
+      return D377_ERR_INVALID_ARG;
+    }
+  const size_t n = offsets[nmsm];
+  if (n > 0xfffffff0ull) { set_error("d377_msm_segmented: too many pairs"); return D377_ERR_INVALID_ARG; }
+  if (n && (!scalars || !points)) return null_pointer();
+  return msm_segmented_width(e, *pf, offsets, nmsm, c);
+}
+
+int d377_msm_segmented_dev(const uint8_t* scalars, const uint8_t* points, int point_format, const uint32_t* offsets,
+                           size_t nmsm, uint8_t* out, int out_format, uint8_t* ok) {
+  D377_REQUIRE_READY();
+  int pf = 0, c = 0;
+  bool sc_mont = false;
+  TRY(msm_segmented_args(_eng, scalars, points, point_format, offsets, nmsm, out, out_format, &pf, &sc_mont, &c));
+  if (nmsm == 0) return D377_OK;
+  return msm_segmented_enqueue(scalars, points, pf, sc_mont, offsets, nmsm, c, out, out_format, ok);
+}
+
+int d377_msm_segmented(const uint8_t* scalars, const uint8_t* points, int point_format, const uint32_t* offsets,
+                       size_t nmsm, uint8_t* out, int out_format, uint8_t* ok) {
+  D377_REQUIRE_READY();
+  Engine& e = _eng;
+  int pf = 0, c = 0;
+  bool sc_mont = false;
+  TRY(msm_segmented_args(e, scalars, points, point_format, offsets, nmsm, out, out_format, &pf, &sc_mont, &c));
+  if (nmsm == 0) return D377_OK;
+  const size_t n = offsets[nmsm];
+  const size_t pb = pt_bytes(pf), ob = out_bytes(out_format);
+  TRY(ensure(e.bm_sc, n * 32 + 32));
+  TRY(ensure(e.bm_pt, n * pb + 128));
+  TRY(ensure(e.bm_out, nmsm * ob));
+  TRY(ensure(e.bm_okout, nmsm + 16));
+  auto body = [&]() -> int {
+    if (n) {
+      D377_CUDA(cudaMemcpyAsync(e.bm_sc.p, scalars, n * 32, cudaMemcpyHostToDevice, e.stream));
+      D377_CUDA(cudaMemcpyAsync(e.bm_pt.p, points, n * pb, cudaMemcpyHostToDevice, e.stream));
+    }
+    TRY(msm_segmented_enqueue((const uint8_t*)e.bm_sc.p, (const uint8_t*)e.bm_pt.p, pf, sc_mont, offsets, nmsm, c,
+                              (uint8_t*)e.bm_out.p, out_format, ok ? (uint8_t*)e.bm_okout.p : nullptr));
+    D377_CUDA(cudaMemcpyAsync(out, e.bm_out.p, nmsm * ob, cudaMemcpyDeviceToHost, e.stream));
+    if (ok) D377_CUDA(cudaMemcpyAsync(ok, e.bm_okout.p, nmsm, cudaMemcpyDeviceToHost, e.stream));
+    D377_CUDA(cudaStreamSynchronize(e.stream));
+    return D377_OK;
+  };
+  int rc = body();
+  if (rc) drain(e);
+  return rc;
+}
+
+int d377_msm_segmented_last(int* c, int* windows, size_t* chunks) {
+  D377_REQUIRE_READY();
+  return msm_segmented_last(c, windows, chunks);
 }
 
 int d377_batch_normalize_dev(const uint8_t* elements, size_t n, uint8_t* affine) {

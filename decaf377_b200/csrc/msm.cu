@@ -26,6 +26,7 @@
 //      k_finish        Horner over the windows, optional fused compress.
 #include <algorithm>
 #include <cmath>
+#include <cstring>
 #include <vector>
 
 #include "engine.h"
@@ -994,6 +995,119 @@ void launch_seg_sum(const uint8_t* prods, const uint8_t* okp, const uint32_t* of
   D377_LAUNCHED();
 }
 
+// ---- many independent MSMs in one segmented Pippenger (d377_msm_segmented*) ---------------
+// Segment j of a chunk owns the "virtual windows" j W .. j W + W - 1: its window w adds into
+// the bucket set of virtual window j W + w, so sort, accumulation, stitch, bucket reduction
+// and weighted tree run over a flat bucket space exactly as for one MSM with J W windows.
+// Scalars are any 256-bit integers, so the recoding covers 257 bits: W = ceil(257 / c)
+// leaves no carry out of the top window.
+
+// bits [w*c, w*c + c) of the 256-bit little-endian scalar; bits at or above 256 read 0 (when
+// c divides 256 the top window starts at bit 256)
+D377_DI uint32_t scalar_window_257(const fq_raw_t& s, int w, int c) {
+  const int bit = w * c;
+  if (bit >= 256) return 0u;
+  const int limb = bit >> 5, off = bit & 31;
+  uint64_t v = s.l[limb];
+  if (limb + 1 < 8) v |= (uint64_t)s.l[limb + 1] << 32;
+  return (uint32_t)(v >> off) & ((1u << c) - 1u);
+}
+
+// One thread per pair of a chunk of J segments.  `offs` (J + 1 entries) are the chunk's
+// segment bounds as absolute pair indices; pair i of the chunk is pair offs[0] + i.  The
+// entry of window w goes to row w of `dig` (window-major, as k_msm_count) with the bucket id
+// (seg W + w) K + |d| - 1 (sign in bit 31, 0xffffffff for a zero digit).  No range check:
+// every 256-bit integer is a valid scalar here.
+__global__ void __launch_bounds__(256, 8)
+k_msm_count_seg(const uint8_t* __restrict__ scalars, size_t n, const uint32_t* __restrict__ offs, uint32_t J,
+                MsmGeom g, uint32_t* __restrict__ counts, uint32_t* __restrict__ dig) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t p = offs[0] + (uint32_t)i;
+  // the segment holding pair p: the last j < J with offs[j] <= p (empty segments before it
+  // have offs[j] = offs[j + 1] <= p and are passed over)
+  uint32_t lo = 0, hi = J;   // invariant: offs[lo] <= p < offs[hi]
+  while (hi - lo > 1) {
+    const uint32_t m = lo + ((hi - lo) >> 1);
+    if (offs[m] <= p) lo = m; else hi = m;
+  }
+  const fq_raw_t s = fq_load_raw(scalars + 32 * i);
+  uint32_t carry = 0;
+  uint32_t id = lo * (uint32_t)g.W * g.K;
+  uint32_t* row = dig + i;
+#pragma unroll 1
+  for (int w = 0; w < g.W; w++, row += n, id += g.K) {
+    const uint32_t raw = scalar_window_257(s, w, g.c) + carry;
+    carry = raw > g.K ? 1u : 0u;
+    const int32_t d = (int32_t)raw - (int32_t)(carry << g.c);
+    uint32_t e = 0xffffffffu;
+    if (d != 0) {
+      const uint32_t mag = d < 0 ? (uint32_t)(-d) : (uint32_t)d;
+      atomicAdd(&counts[id + mag - 1], 1u);   // result unused: RED.E.ADD
+      e = (id + mag - 1) | (d < 0 ? 0x80000000u : 0u);
+    }
+    *row = e;
+  }
+}
+
+// Encodings -> affine bucket operands as k_msm_points_affine<D377_PT_ENCODING>, with the decode
+// status of every pair in ok[i] (an invalid encoding is stored as the identity).
+__global__ void __launch_bounds__(kBlk)
+k_msm_points_enc_ok(const uint8_t* __restrict__ pts, size_t n, aff4_t* __restrict__ out, uint8_t* __restrict__ ok) {
+  extern __shared__ uint32_t smem[];
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  pt_t p;
+  ok[i] = pt_load_fmt<D377_PT_ENCODING>(p, pts, i, isqrt_smem(smem)) ? 1 : 0;
+  aff4_store(out + i, niels_from_affine(p.x, p.y));
+}
+
+// Horner over the W window sums of every segment of a chunk: one four-lane group per segment
+// (pt_dbl4 / pt_add4 as in k_finish), eight segments per warp.  wsums[j W + w] is window w of
+// segment j.  Stores the canonical Element (out_el + 128 j) and / or the encoding
+// (out_enc + 32 j); ok_out[j] (if wanted) is the AND of the segment's per-pair decode status
+// ok_in[offs[j] .. offs[j + 1]) (all good when ok_in is null).
+constexpr int kSegFinishBlk = 128;
+
+__global__ void __launch_bounds__(kSegFinishBlk)
+k_msm_finish_seg(const pt_t* __restrict__ wsums, uint32_t J, int W, int c, const uint32_t* __restrict__ offs,
+                 const uint8_t* __restrict__ ok_in, uint8_t* __restrict__ out_el, uint8_t* __restrict__ out_enc,
+                 uint8_t* __restrict__ ok_out) {
+  extern __shared__ uint32_t smem[];
+  const int lane = threadIdx.x & 31, role = lane & 3, base = lane & ~3;
+  const size_t seg = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 2;
+  // groups past the end repeat the last segment: the four-lane operations shuffle with a
+  // full mask, so whole warps stay in the loop; only real segments store
+  const bool real = seg < J;
+  const size_t j = real ? seg : (size_t)J - 1;
+  const pt_t* __restrict__ ws = wsums + j * (size_t)W;
+  pt_t r = ptv_load(ws + (W - 1));
+#pragma unroll 1
+  for (int w = W - 2; w >= 0; w--) {
+#pragma unroll 1
+    for (int k = 0; k < c; k++) r = pt_dbl4(r, role, base);
+    r = pt_add4(r, ptv_load(ws + w), role, base);
+  }
+  if (real && role == 0) {
+    D377_DBG_POINT(r);
+    if (out_el) pt_store_canon(out_el + 128 * seg, r);
+  }
+  if (out_enc) {
+    isqrt_smem_t sm = isqrt_smem(smem);
+    fq_t s = pt_compress_to_field(r, sm);
+    if (real && role == 0) fq_store(out_enc + 32 * seg, s);
+  }
+  if (ok_out) {
+    bool good = true;
+    if (ok_in) {
+#pragma unroll 4
+      for (uint32_t i = offs[j] + role; i < offs[j + 1]; i += 4) good = good && ok_in[i] != 0;
+    }
+    const uint32_t bad = __ballot_sync(0xffffffffu, !good);
+    if (real && role == 0) ok_out[seg] = ((bad >> base) & 0xfu) == 0 ? 1 : 0;
+  }
+}
+
 D377_DBG_READER(msm_debug_counts)
 
 // ---------------------------------------------------------------------------
@@ -1228,6 +1342,49 @@ static void group_windows(int W, int ngroups, int* wlo, int* whi) {
   for (int k = 0; k < ngroups; k++) {
     whi[k] = W - cut[k];
     wlo[k] = W - cut[k + 1];
+  }
+}
+
+// Stitch the bucket pieces the accumulation left in 2 * nthreads slots (pb / part) into
+// `bsum`; the slot lists of the later levels rotate through (kbuf[0], pbuf[0]) and
+// (kbuf[1], pbuf[1]).
+static void launch_stitch(cudaStream_t ts, const int32_t* pb, const pt_t* part, size_t nthreads, pt_t* bsum,
+                          int32_t* const kbuf[2], pt_t* const pbuf[2]) {
+  const int32_t* kin = pb;
+  const pt_t* pin = part;
+  size_t nslots = 2 * nthreads;
+  for (int lvl = 0;; lvl++) {
+    size_t nt = (nslots + kSegG - 1) / kSegG;
+    int32_t* kout = kbuf[lvl & 1];
+    pt_t* pout = pbuf[lvl & 1];
+    // work-efficient serial fold while the level is large, warp scan (log depth) below
+    if (nslots <= kStitchWarpSlots)
+      k_msm_seg_reduce_warp<<<grid_for(nt * 32, kBlk), kBlk, 0, ts>>>(kin, pin, nslots, bsum, kout, pout, nt);
+    else
+      k_msm_seg_reduce<<<grid_for(nt, kBlk), kBlk, 0, ts>>>(kin, pin, nslots, bsum, kout, pout, nt);
+    D377_LAUNCHED();
+    if (nt == 1) break;
+    nslots = 2 * nt;
+    kin = kout;
+    pin = pout;
+  }
+}
+
+// Weighted tree over `rows` rows of `len` segment nodes (a, p) -> one node per row, in (a, p)
+// on return (the buffers ping-pong with a2 / p2).  The row is gridDim.y, so a launch covers
+// at most 65 535 rows; more rows are launched in slices.
+static void launch_wsum_tree(cudaStream_t ts, pt_t*& a, pt_t*& p, pt_t*& a2, pt_t*& p2, uint32_t len, size_t rows) {
+  constexpr size_t kMaxRows = 65535;
+  while (len > 1) {
+    const uint32_t olen = (len + kWT - 1) / kWT;
+    for (size_t r0 = 0; r0 < rows; r0 += kMaxRows) {
+      const unsigned nr = (unsigned)std::min(kMaxRows, rows - r0);
+      k_wsum_tree<<<dim3(olen, nr), 2 * kWT, 0, ts>>>(a + r0 * len, p + r0 * len, len, a2 + r0 * olen, p2 + r0 * olen);
+      D377_LAUNCHED();
+    }
+    std::swap(a, a2);
+    std::swap(p, p2);
+    len = olen;
   }
 }
 
@@ -1507,29 +1664,11 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   // ---- tail: everything below runs on the tail stream ----
   D377_CUDA(cudaEventRecord(ms.ev_acc_done, st));
   if (ts != st) D377_CUDA(cudaStreamWaitEvent(ts, ms.ev_acc_done, 0));
-  // 6: stitch the bucket pieces of all groups; the slot lists of the levels rotate through
-  // two buffers (the first level reads the accumulation's own part / pb arrays)
+  // 6: stitch the bucket pieces of all groups
   {
-    const int32_t* kin = pb;
-    const pt_t* pin = part;
-    size_t nslots = 2 * nthreads;
     int32_t* kbuf[2] = {(int32_t*)(tw + o_pb2), (int32_t*)(tw + o_pb3)};
     pt_t* pbuf[2] = {(pt_t*)(tw + o_part2), (pt_t*)(tw + o_part3)};
-    for (int lvl = 0;; lvl++) {
-      size_t nt = (nslots + kSegG - 1) / kSegG;
-      int32_t* kout = kbuf[lvl & 1];
-      pt_t* pout = pbuf[lvl & 1];
-      // work-efficient serial fold while the level is large, warp scan (log depth) below
-      if (nslots <= kStitchWarpSlots)
-        k_msm_seg_reduce_warp<<<grid_for(nt * 32, kBlk), kBlk, 0, ts>>>(kin, pin, nslots, bsum, kout, pout, nt);
-      else
-        k_msm_seg_reduce<<<grid_for(nt, kBlk), kBlk, 0, ts>>>(kin, pin, nslots, bsum, kout, pout, nt);
-      D377_LAUNCHED();
-      if (nt == 1) break;
-      nslots = 2 * nt;
-      kin = kout;
-      pin = pout;
-    }
+    launch_stitch(ts, pb, part, nthreads, bsum, kbuf, pbuf);
   }
   D377_CUDA(stage_mark(6, ts));
   // 7: bucket reduction of every window
@@ -1549,14 +1688,7 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   D377_CUDA(cudaGetLastError());
   D377_CUDA(stage_mark(7, ts));
   // 8: weighted tree -> one sum per window, Horner over the windows, output
-  for (uint32_t len = S; len > 1;) {
-    const uint32_t olen = (len + kWT - 1) / kWT;
-    k_wsum_tree<<<dim3(olen, (unsigned)rg.W), 2 * kWT, 0, ts>>>(a, p, len, a2, p2);
-    D377_LAUNCHED();
-    std::swap(a, a2);
-    std::swap(p, p2);
-    len = olen;
-  }
+  launch_wsum_tree(ts, a, p, a2, p2, S, (size_t)rg.W);
   // windowed: the group sums are already weighted by 2^(c w), k_finish only adds them
   rc = finish(ts, a, rg.W, windowed ? 0 : g.c, out_element, out_encoding);
   if (rc) return rc;
@@ -1671,6 +1803,243 @@ int msm_dev_async(const uint8_t* scalars, const uint8_t* points, int point_forma
   return msm_enqueue(scalars, points, fmt, sc_mont, n, out_element, out_encoding,
                      (uint32_t*)(e.d_small + kSmallAsyncFlags), 0, nullptr,
                      (flags & D377_MSM_INPUTS_READY) != 0);
+}
+
+// ---- many independent MSMs in one segmented Pippenger (d377_msm_segmented*) --------------
+// A chunk's bucket sums (J W K x 128 B) stay under this budget; chunks are cut at segment
+// bounds and run one after the other over one workspace.
+constexpr size_t kSegBucketBudget = (size_t)1 << 30;
+constexpr size_t kSegMaxEntries = 0xfffffff0ull;   // entries (pairs x W) of a chunk, as msm_once
+
+static MsmGeom seg_geom(int c) {
+  MsmGeom g;
+  g.c = c;
+  g.W = (257 + c - 1) / c;   // any 256-bit scalar: no carry out of the top window
+  g.K = 1u << (c - 1);
+  return g;
+}
+
+// Bucket operands: affine records (7 M per addition) unless projective inputs are too few for
+// the batch normalisation to pay -- msm_once's rule, over all pairs of the call.
+static bool seg_normalize(const Engine& e, int fmt, size_t n) {
+  const bool projective = fmt == D377_PT_ELEMENT || fmt == D377_PT_XYZ;
+  const int want = e.msm_normalize_override;
+  return projective && (want > 0 || (want == 0 && (n >> 17) >= 8));
+}
+
+int msm_segmented_width(Engine& e, int fmt, const uint32_t* offsets, size_t nmsm, int* c_out) {
+  const size_t n = offsets[nmsm];
+  size_t longest = 0;
+  for (size_t j = 0; j < nmsm; j++) longest = std::max<size_t>(longest, offsets[j + 1] - offsets[j]);
+  const bool projective = fmt == D377_PT_ELEMENT || fmt == D377_PT_XYZ;
+  const double madd = projective && !seg_normalize(e, fmt, n) ? 8.0 : 7.0;
+  const int lo = e.msm_window_override ? e.msm_window_override : 4;
+  const int hi = e.msm_window_override ? e.msm_window_override : 16;
+  int best_c = 0;
+  double best = 1e300;
+  for (int c = lo; c <= hi; c++) {
+    const MsmGeom g = seg_geom(c);
+    // every segment must fit a chunk of its own
+    if ((size_t)g.W * g.K * sizeof(pt_t) > kSegBucketBudget || longest * (size_t)g.W >= kSegMaxEntries) continue;
+    // one bucket addition per (pair, window); two additions (~32 M with the tree) per bucket,
+    // empty or not; the four-lane Horner tail of every segment
+    const double K = (double)g.K, W = (double)g.W;
+    const double cost = (double)n * W * madd + (double)nmsm * W * K * 32.0 + (double)nmsm * W * (c + 1) * 8.0;
+    if (cost < best) { best = cost; best_c = c; }
+  }
+  if (!best_c) {
+    set_error("d377_msm_segmented: a segment of %zu pairs does not fit one chunk at window width %s%d", longest,
+              e.msm_window_override ? "" : "<= ", hi);
+    return D377_ERR_INVALID_ARG;
+  }
+  *c_out = best_c;
+  return D377_OK;
+}
+
+// Enqueue on the engine stream; arguments checked, `offsets` in host memory, c from
+// msm_segmented_width.  Device pointers: scalars, points, out, ok (may be null).
+int msm_segmented_enqueue(const uint8_t* scalars, const uint8_t* points, int fmt, bool sc_mont,
+                          const uint32_t* offsets, size_t nmsm, int c, uint8_t* out, int out_format, uint8_t* ok) {
+  Engine& e = engine();
+  const MsmGeom g = seg_geom(c);
+  const size_t n = offsets[nmsm];
+  const size_t WK = (size_t)g.W * g.K;
+  // chunks of whole segments: J W K x 128 B of buckets within the budget (so J W K < 2^31
+  // too) and fewer than kSegMaxEntries entries
+  struct Chunk { size_t j0, J; };
+  std::vector<Chunk> chunks;
+  size_t max_pairs = 0, max_J = 0;
+  for (size_t j0 = 0; j0 < nmsm;) {
+    size_t J = 1;
+    while (j0 + J < nmsm && (J + 1) * WK * sizeof(pt_t) <= kSegBucketBudget &&
+           (size_t)(offsets[j0 + J + 1] - offsets[j0]) * g.W < kSegMaxEntries)
+      J++;
+    chunks.push_back({j0, J});
+    max_pairs = std::max<size_t>(max_pairs, offsets[j0 + J] - offsets[j0]);
+    max_J = std::max(max_J, J);
+    j0 += J;
+  }
+  const size_t max_entries = max_pairs * g.W;
+  const int L = max_entries >= ((size_t)1 << 27) ? 128 : max_entries >= ((size_t)1 << 25) ? 64 : 32;
+  const int log_lseg = g.c >= 18 ? 6 : g.c == 17 ? 5 : 4;
+  const uint32_t Lseg = 1u << log_lseg;
+  const uint32_t S = (g.K + Lseg - 1) / Lseg;
+  const bool normalize = seg_normalize(e, fmt, n);
+  const bool affine = !(fmt == D377_PT_ELEMENT || fmt == D377_PT_XYZ) || normalize;
+
+  // ---- workspace: the call's converted points, then one chunk's sort and tail ----
+  size_t off = 0;
+  auto carve = [&](size_t bytes) { size_t o = off; off += align_up(bytes); return o; };
+  const size_t o_offs = carve((nmsm + 1) * 4);
+  const size_t o_sc = carve(sc_mont ? n * 32 : 0);
+  const size_t o_pts = carve(n * 128);
+  const size_t o_norm = carve(normalize ? n * 32 : 0);
+  const size_t o_okp = carve(fmt == D377_PT_ENCODING ? n : 0);
+  const size_t max_nb = max_J * WK, max_threads = (max_entries + L - 1) / L;
+  const size_t max_tiles = (max_nb + 1 + kScanTile - 1) / kScanTile;
+  const size_t o_dig = carve(max_entries * 4);
+  const size_t o_sorted = carve(max_entries * 4);
+  const size_t o_counts = carve((max_nb + 1) * 4);
+  const size_t o_cursor = carve((max_nb + 1) * 4);
+  const size_t o_tiles = carve(max_tiles * 4 + 4);
+  const size_t o_bsum = carve(max_nb * sizeof(pt_t));
+  const size_t o_part = carve(2 * max_threads * sizeof(pt_t));
+  const size_t o_pb = carve(2 * max_threads * 4);
+  const size_t nthreads2 = (2 * max_threads + kSegG - 1) / kSegG;
+  const size_t nthreads3 = (2 * nthreads2 + kSegG - 1) / kSegG;
+  const size_t o_part2 = carve(2 * nthreads2 * sizeof(pt_t));
+  const size_t o_pb2 = carve(2 * nthreads2 * 4);
+  const size_t o_part3 = carve(2 * nthreads3 * sizeof(pt_t));
+  const size_t o_pb3 = carve(2 * nthreads3 * 4);
+  const size_t max_rows = max_J * g.W;
+  const size_t o_seg_a = carve(max_rows * S * sizeof(pt_t));
+  const size_t o_seg_p = carve(max_rows * S * sizeof(pt_t));
+  const size_t o_seg_a2 = carve(max_rows * ((S + kWT - 1) / kWT) * sizeof(pt_t));
+  const size_t o_seg_p2 = carve(max_rows * ((S + kWT - 1) / kWT) * sizeof(pt_t));
+  int rc = ensure(e.seg_ws, off);
+  if (rc) return rc;
+  uint8_t* ws = (uint8_t*)e.seg_ws.p;
+  cudaStream_t st = e.stream;
+
+  // The offsets go up through a pinned staging copy, so that the caller may reuse its array
+  // as soon as the call returns; the previous call's upload must have left the staging buffer.
+  const size_t off_bytes = (nmsm + 1) * 4;
+  if (!e.ev_seg_off) D377_CUDA(cudaEventCreateWithFlags(&e.ev_seg_off, cudaEventDisableTiming));
+  else D377_CUDA(cudaEventSynchronize(e.ev_seg_off));
+  if (e.seg_off_cap < off_bytes) {
+    if (e.seg_off_host) D377_CUDA(cudaFreeHost(e.seg_off_host));
+    e.seg_off_host = nullptr;
+    e.seg_off_cap = 0;
+    D377_CUDA(cudaHostAlloc(&e.seg_off_host, off_bytes, cudaHostAllocDefault));
+    e.seg_off_cap = off_bytes;
+  }
+  memcpy(e.seg_off_host, offsets, off_bytes);
+  uint32_t* d_offs = (uint32_t*)(ws + o_offs);
+  D377_CUDA(cudaMemcpyAsync(d_offs, e.seg_off_host, off_bytes, cudaMemcpyHostToDevice, st));
+  D377_CUDA(cudaEventRecord(e.ev_seg_off, st));
+
+  // ---- once per call: canonical scalars, bucket operands (and per-pair decode status) ----
+  uint8_t* okp = fmt == D377_PT_ENCODING ? ws + o_okp : nullptr;
+  if (n) {
+    if (sc_mont) {
+      launch_fr_from_mont(scalars, n, ws + o_sc, st);
+      scalars = ws + o_sc;
+    }
+    if (fmt == D377_PT_ENCODING) {
+      k_msm_points_enc_ok<<<grid_for(n, kBlk), kBlk, ISQRT_SMEM_WORDS(kBlk) * 4, st>>>(points, n, (aff4_t*)(ws + o_pts),
+                                                                                        okp);
+      D377_LAUNCHED();
+    } else if (affine) {
+      // Affine inputs never fail to load and normalisation reports nothing: no flags word
+      launch_points_affine(e, fmt, points, n, e.msm_normalize_override > 0 ? 4 : 1, ws + o_norm,
+                           (aff4_t*)(ws + o_pts), nullptr, st);
+    } else {
+      if (fmt == D377_PT_ELEMENT)
+        k_msm_points<D377_PT_ELEMENT><<<grid_for(n, kBlk), kBlk, 0, st>>>(points, n, (cached_t*)(ws + o_pts));
+      else
+        k_msm_points<D377_PT_XYZ><<<grid_for(n, kBlk), kBlk, 0, st>>>(points, n, (cached_t*)(ws + o_pts));
+      D377_LAUNCHED();
+    }
+  }
+
+  // ---- chunk by chunk ----
+  uint32_t* dig = (uint32_t*)(ws + o_dig);
+  uint32_t* sorted = (uint32_t*)(ws + o_sorted);
+  uint32_t* counts = (uint32_t*)(ws + o_counts);
+  uint32_t* cursor = (uint32_t*)(ws + o_cursor);
+  uint32_t* tiles = (uint32_t*)(ws + o_tiles);
+  pt_t* bsum = (pt_t*)(ws + o_bsum);
+  pt_t* part = (pt_t*)(ws + o_part);
+  int32_t* pb = (int32_t*)(ws + o_pb);
+  int32_t* kbuf[2] = {(int32_t*)(ws + o_pb2), (int32_t*)(ws + o_pb3)};
+  pt_t* pbuf[2] = {(pt_t*)(ws + o_part2), (pt_t*)(ws + o_part3)};
+  const size_t ob = out_bytes(out_format);
+  for (const Chunk& ch : chunks) {
+    const size_t p0 = offsets[ch.j0], np = offsets[ch.j0 + ch.J] - p0;
+    const size_t nb = ch.J * WK, nthreads = (np * g.W + L - 1) / L;
+    const size_t ntiles = (nb + 1 + kScanTile - 1) / kScanTile;
+    const uint32_t* offs = d_offs + ch.j0;
+    D377_CUDA(cudaMemsetAsync(counts, 0, (nb + 1) * 4, st));
+    if (np) {
+      k_msm_count_seg<<<grid_for(np, 256), 256, 0, st>>>(scalars + 32 * p0, np, offs, (uint32_t)ch.J, g, counts, dig);
+      D377_LAUNCHED();
+    }
+    k_scan_tiles<<<(unsigned)ntiles, kScanBlock, 0, st>>>(counts, nb + 1, tiles);
+    D377_LAUNCHED();
+    k_scan_sums<<<1, kScanBlock, 0, st>>>(tiles, ntiles, tiles + ntiles);
+    D377_LAUNCHED();
+    k_scan_apply<<<(unsigned)ntiles, kScanBlock, 0, st>>>(counts, nb + 1, tiles, cursor);
+    D377_LAUNCHED();
+    if (np) {
+      // stored index: the pair within the chunk, whose bucket operands start at p0
+      k_msm_scatter<<<(unsigned)((size_t)grid_for(np, 256 * kScatterIlp) * g.W), 256, 0, st>>>(
+          dig, np, (uint32_t)g.W, cursor, sorted, 0u, 0u);
+      D377_LAUNCHED();
+      D377_CUDA(cudaMemsetAsync(pb, 0xff, 2 * nthreads * 4, st));
+      const uint8_t* recs = ws + o_pts + 128 * p0;
+      if (affine)
+        k_msm_accumulate<true><<<grid_for(nthreads, kBlk), kBlk, 0, st>>>(recs, sorted, counts, (uint32_t)nb, L, bsum,
+                                                                           part, pb, 0);
+      else
+        k_msm_accumulate<false><<<grid_for(nthreads, kBlk), kBlk, 0, st>>>(recs, sorted, counts, (uint32_t)nb, L, bsum,
+                                                                            part, pb, 0);
+      D377_LAUNCHED();
+      launch_stitch(st, pb, part, nthreads, bsum, kbuf, pbuf);
+    }
+    // bucket reduction: one group of J W virtual windows
+    const size_t rows = ch.J * g.W;
+    pt_t *a = (pt_t*)(ws + o_seg_a), *p = (pt_t*)(ws + o_seg_p);
+    pt_t *a2 = (pt_t*)(ws + o_seg_a2), *p2 = (pt_t*)(ws + o_seg_p2);
+    GroupTab gt;
+    gt.ng = 1;
+    gt.wlo[0] = 0;
+    gt.whi[0] = (int)rows;
+    gt.offs[0] = counts;
+    MsmGeom rg = g;
+    rg.W = (int)rows;
+    k_msm_bucket_reduce_ap<<<grid_for(rows * S, kBlk), kBlk, 0, st>>>(bsum, gt, rg, Lseg, log_lseg, S, a, p);
+    D377_LAUNCHED();
+    launch_wsum_tree(st, a, p, a2, p2, S, rows);
+    k_msm_finish_seg<<<grid_for(ch.J * 4, kSegFinishBlk), kSegFinishBlk,
+                       out_format == D377_OUT_ENCODING ? ISQRT_SMEM_WORDS(kSegFinishBlk) * 4 : 0, st>>>(
+        a, (uint32_t)ch.J, g.W, g.c, offs, okp, out_format == D377_OUT_ELEMENT ? out + ob * ch.j0 : nullptr,
+        out_format == D377_OUT_ENCODING ? out + ob * ch.j0 : nullptr, ok ? ok + ch.j0 : nullptr);
+    D377_LAUNCHED();
+    D377_CUDA(cudaGetLastError());
+  }
+  e.seg_last_c = g.c;
+  e.seg_last_W = g.W;
+  e.seg_last_chunks = chunks.size();
+  return D377_OK;
+}
+
+int msm_segmented_last(int* c, int* W, size_t* chunks) {
+  Engine& e = engine();
+  if (!e.seg_last_c) { set_error("no segmented msm has run yet"); return D377_ERR_INVALID_ARG; }
+  if (c) *c = e.seg_last_c;
+  if (W) *W = e.seg_last_W;
+  if (chunks) *chunks = e.seg_last_chunks;
+  return D377_OK;
 }
 
 bool msm_last_mixed() { return engine().msm.last_affine; }

@@ -178,6 +178,38 @@ def fixed_bases_mul(bases, scalars: torch.Tensor, out_format: int = OUT_ELEMENT,
     return out
 
 
+def msm_segmented(scalars: torch.Tensor, points: torch.Tensor, offsets, point_format: int = PT_ELEMENT,
+                  out_format: int = OUT_ELEMENT, out: Optional[torch.Tensor] = None,
+                  ok: Optional[torch.Tensor] = None, scalars_montgomery: bool = False) -> torch.Tensor:
+    """d377_msm_segmented_dev over device-resident scalars / points: MSM j covers pairs
+    offsets[j]..offsets[j+1].  `offsets` stays on the host (a sequence, numpy array or CPU
+    tensor of nmsm + 1 entries); `ok` (optional, [nmsm] uint8 on the device) receives the
+    per-segment decode status."""
+    import numpy as np
+    n = _chk(scalars, 32, "scalars")
+    if _chk(points, PT_WIDTH[point_format], "points") < n:
+        raise ValueError("fewer points than scalars")
+    if isinstance(offsets, torch.Tensor):
+        if offsets.is_cuda:
+            raise ValueError("offsets must be in host memory")
+        offsets = offsets.numpy()
+    off = np.ascontiguousarray(offsets, dtype=np.uint32)
+    if off.ndim != 1 or off.size < 1:
+        raise ValueError("offsets must hold nmsm + 1 entries")
+    if int(off[-1]) > n:
+        raise ValueError("offsets reach past the end of the inputs")
+    nmsm = off.size - 1
+    out = torch.empty((nmsm, OUT_WIDTH[out_format]), dtype=torch.uint8,
+                      device=scalars.device) if out is None else out
+    _after_torch()
+    check(_lib.load().d377_msm_segmented_dev(scalars.data_ptr(), points.data_ptr(),
+                                             point_format | (SCALARS_MONTGOMERY if scalars_montgomery else 0),
+                                             off.ctypes.data, nmsm, out.data_ptr(), out_format,
+                                             None if ok is None else ok.data_ptr()))
+    _then_torch()
+    return out
+
+
 def normalize(elements: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """CurveGroup::normalize_batch on device-resident elements -> affine [n, 64]."""
     n = _chk(elements, 128, "elements")

@@ -280,6 +280,37 @@ int d377_batch_msm_dev(const uint8_t* scalars, const uint8_t* points, int point_
                        const uint32_t* offsets, size_t nmsm, size_t n, uint8_t* out, int out_format,
                        uint8_t* ok);
 
+/* ---- many independent MSMs in one segmented Pippenger ----------------------------------
+ * The results and contract of d377_batch_msm (MSM j = sum over i in [offsets[j], offsets[j+1])
+ * of scalars[i] * points[i]; an empty segment gives the identity; scalars are any 256-bit LE
+ * integers, optionally | D377_SCALARS_MONTGOMERY on point_format; out: nmsm x 128 B canonical
+ * Elements or nmsm x 32 B encodings; ok (may be NULL): ok[j] = 0 iff segment j holds an
+ * invalid encoding, which counts as the identity), computed by one Pippenger over all
+ * segments: segment j's window w is bucket set j*W + w of one flat bucket space, so sort,
+ * accumulation and bucket reduction are shared, and each segment ends in its own Horner.
+ * point_format 0..3 (D377_PT_BASES is refused).  The cost is per pair and window plus per
+ * bucket (2^(c-1) per segment and window), not a ladder per pair.
+ * Measured on one B200 (1000 W power limit), device resident, back to back, 2^22 pairs: faster
+ * than d377_batch_msm at every segment length measured, from 64 pairs (3.1x) to 65 536 (11x),
+ * and faster than one d377_msm_dev_async per segment at every length up to 65 536 pairs (4.2x
+ * there, 62x at 1 024); DESIGN.md 3.4.1 has the table.
+ * `offsets` is HOST memory for BOTH forms: the library validates it (offsets[0] = 0,
+ * non-decreasing, offsets[nmsm] <= 0xfffffff0), chooses the window width c (4..16;
+ * d377_msm_set_window applies) and cuts the segments into chunks whose bucket sums stay under
+ * 1 GiB before anything is launched, and copies it up itself (the array may be reused when
+ * the call returns).  A segment too long for one chunk at the width is refused with
+ * D377_ERR_INVALID_ARG.  _dev takes device scalars, points, out and ok and only enqueues on
+ * the engine stream (d377_stream()), behind every earlier call; the outputs are complete there.
+ * Refusals leave out / ok untouched; nmsm = 0 is a no-op. */
+int d377_msm_segmented(const uint8_t* scalars, const uint8_t* points, int point_format,
+                       const uint32_t* offsets, size_t nmsm, uint8_t* out, int out_format, uint8_t* ok);
+int d377_msm_segmented_dev(const uint8_t* scalars, const uint8_t* points, int point_format,
+                           const uint32_t* offsets /* HOST */, size_t nmsm, uint8_t* out, int out_format,
+                           uint8_t* ok);
+/* c, W = ceil(257 / c) and the number of segment chunks of the most recent d377_msm_segmented*
+ * call of this engine (any pointer may be NULL); D377_ERR_INVALID_ARG before the first. */
+int d377_msm_segmented_last(int* c, int* windows, size_t* chunks);
+
 /* ---- CurveGroup::normalize_batch / ScalarMul::batch_convert_to_mul_base
  *      (ark_curve/element.rs:27-34,74-81) ----------------------------------
  * Element (128 B) -> AffinePoint x||y (64 B montgomery, x = X/Z, y = Y/Z), one field

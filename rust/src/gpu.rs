@@ -93,6 +93,8 @@ extern "C" {
                       out_element: *mut u8, out_encoding: *mut u8) -> c_int;
     fn d377_batch_msm(scalars: *const u8, points: *const u8, point_format: c_int, offsets: *const u32, nmsm: usize,
                       out: *mut u8, out_format: c_int, ok: *mut u8) -> c_int;
+    fn d377_msm_segmented(scalars: *const u8, points: *const u8, point_format: c_int, offsets: *const u32,
+                          nmsm: usize, out: *mut u8, out_format: c_int, ok: *mut u8) -> c_int;
     fn d377_msm_bases_create(points: *const u8, point_format: c_int, n: usize, bases: *mut *mut u8) -> c_int;
     fn d377_msm_bases_destroy(bases: *mut u8) -> c_int;
     fn d377_msm_bases_create_windowed(points: *const u8, point_format: c_int, n: usize, c: c_int,
@@ -493,10 +495,9 @@ pub fn vartime_multiscalar_mul_multi_gpu(scalars: &[Fr], points: &[Element], ngp
     Ok(wire_to_element(&out))
 }
 
-/// Many independent `Element::vartime_multiscalar_mul` calls in one launch (e.g. a batch of
-/// verification equations): `jobs[j]` is one (scalars, points) pair of slices, zipped like the
-/// crate's fold.  Cost is per pair, not per job; see `d377_batch_msm`.
-pub fn vartime_multiscalar_mul_batch(jobs: &[(&[Fr], &[Element])]) -> Result<Vec<Element>, GpuError> {
+/// The pairs of `jobs` back to back (Montgomery scalars, Element wire images) and the
+/// segment offsets of the batch entry points.
+fn pack_jobs(jobs: &[(&[Fr], &[Element])]) -> (Vec<u32>, Vec<u8>, Vec<u8>) {
     let mut offsets: Vec<u32> = Vec::with_capacity(jobs.len() + 1);
     offsets.push(0);
     let mut total = 0usize;
@@ -515,10 +516,31 @@ pub fn vartime_multiscalar_mul_batch(jobs: &[(&[Fr], &[Element])]) -> Result<Vec
             k += 1;
         }
     }
+    (offsets, ws, wp)
+}
+
+/// Many independent `Element::vartime_multiscalar_mul` calls in one launch (e.g. a batch of
+/// verification equations): `jobs[j]` is one (scalars, points) pair of slices, zipped like the
+/// crate's fold.  Cost is per pair, not per job; see `d377_batch_msm`.
+pub fn vartime_multiscalar_mul_batch(jobs: &[(&[Fr], &[Element])]) -> Result<Vec<Element>, GpuError> {
+    let (offsets, ws, wp) = pack_jobs(jobs);
     let mut out = vec![0u8; 128 * jobs.len()];
     check(unsafe {
         d377_batch_msm(ws.as_ptr(), wp.as_ptr(), PT_ELEMENT | SCALARS_MONTGOMERY, offsets.as_ptr(), jobs.len(),
                        out.as_mut_ptr(), OUT_ELEMENT, core::ptr::null_mut())
+    })?;
+    Ok(wire_to_elements(&out))
+}
+
+/// The same results as `vartime_multiscalar_mul_batch`, from one segmented Pippenger over all
+/// jobs (`d377_msm_segmented`): the cost is per pair and window plus per bucket instead of a
+/// ladder per pair -- the call for many jobs of tens to tens of thousands of pairs.
+pub fn vartime_multiscalar_mul_segmented(jobs: &[(&[Fr], &[Element])]) -> Result<Vec<Element>, GpuError> {
+    let (offsets, ws, wp) = pack_jobs(jobs);
+    let mut out = vec![0u8; 128 * jobs.len()];
+    check(unsafe {
+        d377_msm_segmented(ws.as_ptr(), wp.as_ptr(), PT_ELEMENT | SCALARS_MONTGOMERY, offsets.as_ptr(), jobs.len(),
+                           out.as_mut_ptr(), OUT_ELEMENT, core::ptr::null_mut())
     })?;
     Ok(wire_to_elements(&out))
 }
