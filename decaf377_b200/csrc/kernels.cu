@@ -890,6 +890,49 @@ int d377_msm_dev_async(const uint8_t* scalars, const uint8_t* points, int point_
 }
 
 // ---- many independent small MSMs (Element::vartime_multiscalar_mul in a loop) -----------
+// The host offsets of a segmented call (`who` names the entry point in the error text): at
+// most 2^31 - 1 segments, offsets[0] = 0, non-decreasing.
+static int segment_offsets_ok(const char* who, const uint32_t* offsets, size_t nmsm) {
+  if (nmsm > 0x7fffffffull) { set_error("%s: too many segments", who); return D377_ERR_INVALID_ARG; }
+  if (offsets[0] != 0) { set_error("%s: offsets[0] must be 0", who); return D377_ERR_INVALID_ARG; }
+  for (size_t j = 0; j < nmsm; j++)
+    if (offsets[j + 1] < offsets[j]) {
+      set_error("%s: offsets must not decrease (segment %zu)", who, j);
+      return D377_ERR_INVALID_ARG;
+    }
+  return D377_OK;
+}
+
+// Host-buffer form of a segmented call: the n scalars and points (format pf) go up into
+// bm_sc / bm_pt, `run(scalars, points, out, ok)` enqueues the device-side call on the engine
+// stream, and the nmsm results (and decode status, if wanted) come back.  Blocks until they
+// have landed; on an error the streams are drained first.
+using SegmentedRun = std::function<int(const uint8_t*, const uint8_t*, uint8_t*, uint8_t*)>;
+
+static int staged_segments(Engine& e, const uint8_t* scalars, const uint8_t* points, int pf, size_t n, size_t nmsm,
+                           uint8_t* out, int out_format, uint8_t* ok, const SegmentedRun& run) {
+  const size_t pb = pt_bytes(pf), ob = out_bytes(out_format);
+  TRY(ensure(e.bm_sc, n * 32 + 32));
+  TRY(ensure(e.bm_pt, n * pb + 128));
+  TRY(ensure(e.bm_out, nmsm * ob));
+  TRY(ensure(e.bm_okout, nmsm + 16));
+  auto body = [&]() -> int {
+    if (n) {
+      D377_CUDA(cudaMemcpyAsync(e.bm_sc.p, scalars, n * 32, cudaMemcpyHostToDevice, e.stream));
+      D377_CUDA(cudaMemcpyAsync(e.bm_pt.p, points, n * pb, cudaMemcpyHostToDevice, e.stream));
+    }
+    TRY(run((const uint8_t*)e.bm_sc.p, (const uint8_t*)e.bm_pt.p, (uint8_t*)e.bm_out.p,
+            ok ? (uint8_t*)e.bm_okout.p : nullptr));
+    D377_CUDA(cudaMemcpyAsync(out, e.bm_out.p, nmsm * ob, cudaMemcpyDeviceToHost, e.stream));
+    if (ok) D377_CUDA(cudaMemcpyAsync(ok, e.bm_okout.p, nmsm, cudaMemcpyDeviceToHost, e.stream));
+    D377_CUDA(cudaStreamSynchronize(e.stream));
+    return D377_OK;
+  };
+  int rc = body();
+  if (rc) drain(e);
+  return rc;
+}
+
 static int batch_msm_formats(int point_format, int out_format, int* pf, bool* sc_mont) {
   TRY(parse_format("d377_batch_msm", point_format, kMulFormats, pf, sc_mont));
   return parse_format("d377_batch_msm", out_format, kOutFormats, nullptr);
@@ -937,36 +980,18 @@ int d377_batch_msm(const uint8_t* scalars, const uint8_t* points, int point_form
   TRY(batch_msm_formats(point_format, out_format, &pf, &sc_mont));
   if (nmsm == 0) return D377_OK;
   if (!offsets || !out) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
-  if (nmsm > 0x7fffffffull) { set_error("d377_batch_msm: too many segments"); return D377_ERR_INVALID_ARG; }
-  if (offsets[0] != 0) { set_error("d377_batch_msm: offsets[0] must be 0"); return D377_ERR_INVALID_ARG; }
-  for (size_t j = 0; j < nmsm; j++)
-    if (offsets[j + 1] < offsets[j]) { set_error("d377_batch_msm: offsets must not decrease (segment %zu)", j); return D377_ERR_INVALID_ARG; }
+  TRY(segment_offsets_ok("d377_batch_msm", offsets, nmsm));
   const size_t n = offsets[nmsm];
   if (n && (!scalars || !points)) { set_error("null pointer"); return D377_ERR_INVALID_ARG; }
   Engine& e = _eng;
-  const size_t pb = pt_bytes(pf), ob = out_bytes(out_format);
-  TRY(ensure(e.bm_sc, n * 32 + 32));
-  TRY(ensure(e.bm_pt, n * pb + 128));
   TRY(ensure(e.bm_off, (nmsm + 1) * 4));
-  TRY(ensure(e.bm_out, nmsm * ob));
-  TRY(ensure(e.bm_okout, nmsm + 16));
-  auto body = [&]() -> int {
-    if (n) {
-      D377_CUDA(cudaMemcpyAsync(e.bm_sc.p, scalars, n * 32, cudaMemcpyHostToDevice, e.stream));
-      D377_CUDA(cudaMemcpyAsync(e.bm_pt.p, points, n * pb, cudaMemcpyHostToDevice, e.stream));
-    }
-    D377_CUDA(cudaMemcpyAsync(e.bm_off.p, offsets, (nmsm + 1) * 4, cudaMemcpyHostToDevice, e.stream));
-    TRY(d377_batch_msm_dev((const uint8_t*)e.bm_sc.p, (const uint8_t*)e.bm_pt.p, point_format,
-                           (const uint32_t*)e.bm_off.p, nmsm, n, (uint8_t*)e.bm_out.p, out_format,
-                           ok ? (uint8_t*)e.bm_okout.p : nullptr));
-    D377_CUDA(cudaMemcpyAsync(out, e.bm_out.p, nmsm * ob, cudaMemcpyDeviceToHost, e.stream));
-    if (ok) D377_CUDA(cudaMemcpyAsync(ok, e.bm_okout.p, nmsm, cudaMemcpyDeviceToHost, e.stream));
-    D377_CUDA(cudaStreamSynchronize(e.stream));
-    return D377_OK;
-  };
-  int rc = body();
-  if (rc) drain(e);
-  return rc;
+  return staged_segments(e, scalars, points, pf, n, nmsm, out, out_format, ok,
+                         [&](const uint8_t* sc, const uint8_t* pt, uint8_t* dout, uint8_t* dok) -> int {
+                           D377_CUDA(cudaMemcpyAsync(e.bm_off.p, offsets, (nmsm + 1) * 4, cudaMemcpyHostToDevice,
+                                                     e.stream));
+                           return d377_batch_msm_dev(sc, pt, point_format, (const uint32_t*)e.bm_off.p, nmsm, n, dout,
+                                                     out_format, dok);
+                         });
 }
 
 // ---- many independent MSMs in one segmented Pippenger ---------------------------------------
@@ -980,13 +1005,7 @@ static int msm_segmented_args(Engine& e, const uint8_t* scalars, const uint8_t* 
   TRY(parse_format("d377_msm_segmented", out_format, kOutFormats, nullptr));
   if (nmsm == 0) return D377_OK;
   if (!offsets || !out) return null_pointer();
-  if (nmsm > 0x7fffffffull) { set_error("d377_msm_segmented: too many segments"); return D377_ERR_INVALID_ARG; }
-  if (offsets[0] != 0) { set_error("d377_msm_segmented: offsets[0] must be 0"); return D377_ERR_INVALID_ARG; }
-  for (size_t j = 0; j < nmsm; j++)
-    if (offsets[j + 1] < offsets[j]) {
-      set_error("d377_msm_segmented: offsets must not decrease (segment %zu)", j);
-      return D377_ERR_INVALID_ARG;
-    }
+  TRY(segment_offsets_ok("d377_msm_segmented", offsets, nmsm));
   const size_t n = offsets[nmsm];
   if (n > 0xfffffff0ull) { set_error("d377_msm_segmented: too many pairs"); return D377_ERR_INVALID_ARG; }
   if (n && (!scalars || !points)) return null_pointer();
@@ -1011,27 +1030,10 @@ int d377_msm_segmented(const uint8_t* scalars, const uint8_t* points, int point_
   bool sc_mont = false;
   TRY(msm_segmented_args(e, scalars, points, point_format, offsets, nmsm, out, out_format, &pf, &sc_mont, &c));
   if (nmsm == 0) return D377_OK;
-  const size_t n = offsets[nmsm];
-  const size_t pb = pt_bytes(pf), ob = out_bytes(out_format);
-  TRY(ensure(e.bm_sc, n * 32 + 32));
-  TRY(ensure(e.bm_pt, n * pb + 128));
-  TRY(ensure(e.bm_out, nmsm * ob));
-  TRY(ensure(e.bm_okout, nmsm + 16));
-  auto body = [&]() -> int {
-    if (n) {
-      D377_CUDA(cudaMemcpyAsync(e.bm_sc.p, scalars, n * 32, cudaMemcpyHostToDevice, e.stream));
-      D377_CUDA(cudaMemcpyAsync(e.bm_pt.p, points, n * pb, cudaMemcpyHostToDevice, e.stream));
-    }
-    TRY(msm_segmented_enqueue((const uint8_t*)e.bm_sc.p, (const uint8_t*)e.bm_pt.p, pf, sc_mont, offsets, nmsm, c,
-                              (uint8_t*)e.bm_out.p, out_format, ok ? (uint8_t*)e.bm_okout.p : nullptr));
-    D377_CUDA(cudaMemcpyAsync(out, e.bm_out.p, nmsm * ob, cudaMemcpyDeviceToHost, e.stream));
-    if (ok) D377_CUDA(cudaMemcpyAsync(ok, e.bm_okout.p, nmsm, cudaMemcpyDeviceToHost, e.stream));
-    D377_CUDA(cudaStreamSynchronize(e.stream));
-    return D377_OK;
-  };
-  int rc = body();
-  if (rc) drain(e);
-  return rc;
+  return staged_segments(e, scalars, points, pf, offsets[nmsm], nmsm, out, out_format, ok,
+                         [&](const uint8_t* sc, const uint8_t* pt, uint8_t* dout, uint8_t* dok) {
+                           return msm_segmented_enqueue(sc, pt, pf, sc_mont, offsets, nmsm, c, dout, out_format, dok);
+                         });
 }
 
 int d377_msm_segmented_last(int* c, int* windows, size_t* chunks) {

@@ -23,7 +23,7 @@
 //                      serial walk)
 //   7. k_msm_bucket_reduce_ap  per 16-bucket segment: running sums (A, P)
 //   8. k_wsum_tree     weighted tree over the segments -> one sum per window;
-//      k_finish        Horner over the windows, optional fused compress.
+//      k_msm_finish    Horner over the windows, optional fused compress.
 #include <algorithm>
 #include <cmath>
 #include <cstring>
@@ -89,15 +89,20 @@ k_msm_points(const uint8_t* __restrict__ pts, size_t n, cached_t* __restrict__ o
 
 // Inputs that already have Z = 1 (AffinePoint, Encoding) -> canonical (y-x, y+x, 2d*x*y),
 // 96 B each: the bucket additions then cost 7 multiplications instead of 8.
+// Only an encoding can fail to load (it is stored as the identity).  With `ok` the kernel
+// writes the decode status of every pair there; otherwise a failure sets bit 1 of `flags`
+// (if given).
 template <int kFmt>
 __global__ void __launch_bounds__(kBlk)
 k_msm_points_affine(const uint8_t* __restrict__ pts, size_t n, aff4_t* __restrict__ out,
-                    uint32_t* __restrict__ flags) {
+                    uint32_t* __restrict__ flags, uint8_t* __restrict__ ok) {
   extern __shared__ uint32_t smem[];
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   pt_t p;
-  if (!pt_load_fmt<kFmt>(p, pts, i, isqrt_smem(smem))) atomicOr(flags, 2u);
+  const bool good = pt_load_fmt<kFmt>(p, pts, i, isqrt_smem(smem));
+  if (kFmt == D377_PT_ENCODING && ok) ok[i] = good ? 1 : 0;
+  else if (!good && flags) atomicOr(flags, 2u);
   aff4_store(out + i, niels_from_affine(p.x, p.y));
 }
 
@@ -201,22 +206,28 @@ void launch_normalize(const uint8_t* el, size_t n, uint8_t* scratch, uint8_t* ou
   k_msm_normalize<128, true><<<(unsigned)(T / kNormBlk), kNormBlk, 0, st>>>(el, n, T, scratch, out);
 }
 
-// Input points of any wire format -> affine bucket operands on `st`: Element / XYZ by batch
-// normalisation (normalize_threads(n, min_per), `scratch` n x 32 B), AffinePoint / Encoding
-// one point per thread (an invalid encoding sets bit 1 of `flags`).
-static void launch_points_affine(const Engine& e, int point_format, const uint8_t* pts, size_t n, size_t min_per,
-                                 uint8_t* scratch, aff4_t* out, uint32_t* flags, cudaStream_t st) {
-  if (point_format == D377_PT_ELEMENT || point_format == D377_PT_XYZ) {
+static bool projective_format(int fmt) { return fmt == D377_PT_ELEMENT || fmt == D377_PT_XYZ; }
+
+// n input points of any wire format -> bucket operands in `out` (n x 128 B) on `st`.  Affine
+// records where `affine`: Element / XYZ by batch normalisation (normalize_threads(n, min_per),
+// `scratch` n x 32 B), AffinePoint / Encoding one point per thread (an invalid encoding is
+// reported in `ok` or `flags`, see k_msm_points_affine).  Otherwise cached projective records
+// (Element / XYZ only).
+static void launch_operands(const Engine& e, int fmt, bool affine, size_t min_per, const uint8_t* pts, size_t n,
+                            uint8_t* scratch, uint8_t* out, uint32_t* flags, uint8_t* ok, cudaStream_t st) {
+  aff4_t* aff = (aff4_t*)out;
+  if (!affine) {
+    auto k = fmt == D377_PT_ELEMENT ? k_msm_points<D377_PT_ELEMENT> : k_msm_points<D377_PT_XYZ>;
+    k<<<grid_for(n, kBlk), kBlk, 0, st>>>(pts, n, (cached_t*)out);
+  } else if (projective_format(fmt)) {
     const size_t T = normalize_threads(n, min_per, e.sm_count);
-    if (point_format == D377_PT_ELEMENT)
-      k_msm_normalize<128><<<(unsigned)(T / kNormBlk), kNormBlk, 0, st>>>(pts, n, T, scratch, out);
-    else
-      k_msm_normalize<96><<<(unsigned)(T / kNormBlk), kNormBlk, 0, st>>>(pts, n, T, scratch, out);
-  } else if (point_format == D377_PT_AFFINE) {
-    k_msm_points_affine<D377_PT_AFFINE><<<grid_for(n, kBlk), kBlk, 0, st>>>(pts, n, out, flags);
+    auto k = fmt == D377_PT_ELEMENT ? k_msm_normalize<128> : k_msm_normalize<96>;
+    k<<<(unsigned)(T / kNormBlk), kNormBlk, 0, st>>>(pts, n, T, scratch, aff);
+  } else if (fmt == D377_PT_AFFINE) {
+    k_msm_points_affine<D377_PT_AFFINE><<<grid_for(n, kBlk), kBlk, 0, st>>>(pts, n, aff, flags, ok);
   } else {
-    k_msm_points_affine<D377_PT_ENCODING><<<grid_for(n, kBlk), kBlk, ISQRT_SMEM_WORDS(kBlk) * 4, st>>>(pts, n, out,
-                                                                                                        flags);
+    k_msm_points_affine<D377_PT_ENCODING><<<grid_for(n, kBlk), kBlk, ISQRT_SMEM_WORDS(kBlk) * 4, st>>>(pts, n, aff,
+                                                                                                        flags, ok);
   }
   D377_LAUNCHED();
 }
@@ -251,17 +262,38 @@ k_msm_bases_double(uint8_t* __restrict__ run, const aff4_t* __restrict__ first, 
 // ---- 2./4. signed-digit recoding ------------------------------------------
 struct MsmGeom {
   int c;        // window width
-  int W;        // number of windows = ceil(252 / c)
+  int W;        // number of windows = ceil(252 / c) (ceil(257 / c) for any 256-bit scalar)
   uint32_t K;   // buckets per window = 2^(c-1)
 };
 
-// bits [w*c, w*c + c) of the 256-bit little-endian scalar
+static MsmGeom geom(int c, int W) { return MsmGeom{c, W, 1u << (c - 1)}; }
+
+// bits [w*c, w*c + c) of the 256-bit little-endian scalar; bits at or above 256 read 0 (when
+// c divides 256 the top window of a 257-bit recoding starts at bit 256)
 D377_DI uint32_t scalar_window(const fq_raw_t& s, int w, int c) {
-  int bit = w * c;
-  int limb = bit >> 5, off = bit & 31;
+  const int bit = w * c;
+  if (bit >= 256) return 0u;
+  const int limb = bit >> 5, off = bit & 31;
   uint64_t v = s.l[limb];
   if (limb + 1 < 8) v |= (uint64_t)s.l[limb + 1] << 32;
   return (uint32_t)(v >> off) & ((1u << c) - 1u);
+}
+
+// One signed-digit step: window w of s plus the carry in -> digit d in (-K, K] and the carry
+// out.  A nonzero digit (when `take`) bumps the count of bucket id0 + |d| - 1 and returns that
+// id with the sign in bit 31; otherwise the entry is 0xffffffff.
+D377_DI uint32_t digit_entry(const fq_raw_t& s, int w, const MsmGeom& g, uint32_t& carry, uint32_t id0, bool take,
+                             uint32_t* __restrict__ counts) {
+  const uint32_t raw = scalar_window(s, w, g.c) + carry;
+  carry = raw > g.K ? 1u : 0u;
+  const int32_t d = (int32_t)raw - (int32_t)(carry << g.c);
+  uint32_t e = 0xffffffffu;
+  if (d != 0 && take) {
+    const uint32_t id = id0 + (d < 0 ? (uint32_t)(-d) : (uint32_t)d) - 1;
+    atomicAdd(&counts[id], 1u);   // result unused: compiles to RED.E.ADD
+    e = id | (d < 0 ? 0x80000000u : 0u);
+  }
+  return e;
 }
 
 // Pass 1 (one thread per scalar): range check, signed-digit recoding, bucket histogram.
@@ -285,22 +317,17 @@ k_msm_count(const uint8_t* __restrict__ scalars, size_t n, MsmGeom g, int wa, in
     const bool ok = fr_raw_is_canonical(s);
     if (!ok) atomicOr(flags, 1u);  // contributes nothing; the call reports D377_ERR_SCALAR_RANGE
     uint32_t carry = 0;
+    // W = ceil(252 / c): every window starts below bit 252 (scalar_window's bit-256 test folds away)
 #pragma unroll 1
-    for (int w = 0; w < wa; w++) carry = (scalar_window(s, w, g.c) + carry) > g.K ? 1u : 0u;
+    for (int w = 0; w < wa; w++) {
+      __builtin_assume(w * g.c < 252);
+      carry = (scalar_window(s, w, g.c) + carry) > g.K ? 1u : 0u;
+    }
     uint32_t* row = dig + i;
 #pragma unroll 1
     for (int w = wa; w < wb; w++, row += n) {
-      uint32_t raw = scalar_window(s, w, g.c) + carry;
-      carry = raw > g.K ? 1u : 0u;
-      int32_t d = (int32_t)raw - (int32_t)(carry << g.c);
-      uint32_t e = 0xffffffffu;
-      if (d != 0 && ok) {
-        uint32_t mag = d < 0 ? (uint32_t)(-d) : (uint32_t)d;
-        uint32_t id = (uint32_t)(w - wa) * wstride + (mag - 1);
-        atomicAdd(&counts[id], 1u);   // result unused: compiles to RED.E.ADD
-        e = id | (d < 0 ? 0x80000000u : 0u);
-      }
-      *row = e;
+      __builtin_assume(w * g.c < 252);
+      *row = digit_entry(s, w, g, carry, (uint32_t)(w - wa) * wstride, ok, counts);
     }
   }
 }
@@ -932,29 +959,53 @@ k_wsum_tree(const pt_t* __restrict__ a_in, const pt_t* __restrict__ p_in, uint32
   }
 }
 
-// Horner over window sums: Q = sum_w 2^(c w) * S_w ; W = 0 means identity.  One warp;
-// lanes work in groups of four (all groups compute the same thing, lane 0 stores).
-__global__ void __launch_bounds__(32)
-k_finish(const pt_t* __restrict__ wsums, int W, int c, uint8_t* __restrict__ out_element,
-         uint8_t* __restrict__ out_encoding) {
+// Horner over the W window sums of each of J segments: Q_j = sum_w 2^(c w) * S_jw, with
+// wsums[j W + w] = S_jw; W = 0 means identity.  One four-lane group per segment (pt_dbl4 /
+// pt_add4), eight per warp; a single result (J = 1) is one warp whose other groups compute the
+// same thing.  Stores the canonical Element (out_el + 128 j) and / or the encoding
+// (out_enc + 32 j); ok_out[j] (if wanted) is the AND of the segment's per-pair decode status
+// ok_in[offs[j] .. offs[j + 1]) (all good when ok_in is null).
+constexpr int kFinishBlk = 128;
+
+__global__ void __launch_bounds__(kFinishBlk)
+k_msm_finish(const pt_t* __restrict__ wsums, uint32_t J, int W, int c, const uint32_t* __restrict__ offs,
+             const uint8_t* __restrict__ ok_in, uint8_t* __restrict__ out_el, uint8_t* __restrict__ out_enc,
+             uint8_t* __restrict__ ok_out) {
   extern __shared__ uint32_t smem[];
   const int lane = threadIdx.x & 31, role = lane & 3, base = lane & ~3;
+  const size_t seg = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 2;
+  // groups past the end repeat the last segment: the four-lane operations shuffle with a
+  // full mask, so whole warps stay in the loop; only real segments store
+  const bool real = seg < J;
+  const size_t j = real ? seg : (size_t)J - 1;
+  const pt_t* __restrict__ ws = wsums + j * (size_t)W;
   pt_t r = pt_identity();
   if (W > 0) {
-    r = ptv_load(wsums + (W - 1));
+    r = ptv_load(ws + (W - 1));
 #pragma unroll 1
     for (int w = W - 2; w >= 0; w--) {
 #pragma unroll 1
       for (int k = 0; k < c; k++) r = pt_dbl4(r, role, base);
-      r = pt_add4(r, ptv_load(wsums + w), role, base);
+      r = pt_add4(r, ptv_load(ws + w), role, base);
     }
   }
-  if (lane == 0) D377_DBG_POINT(r);
-  if (out_element && lane == 0) pt_store_canon(out_element, r);
-  if (out_encoding) {
+  if (real && role == 0) {
+    D377_DBG_POINT(r);
+    if (out_el) pt_store_canon(out_el + 128 * seg, r);
+  }
+  if (out_enc) {
     isqrt_smem_t sm = isqrt_smem(smem);
     fq_t s = pt_compress_to_field(r, sm);
-    if (lane == 0) fq_store(out_encoding, s);
+    if (real && role == 0) fq_store(out_enc + 32 * seg, s);
+  }
+  if (ok_out) {
+    bool good = true;
+    if (ok_in) {
+#pragma unroll 4
+      for (uint32_t i = offs[j] + role; i < offs[j + 1]; i += 4) good = good && ok_in[i] != 0;
+    }
+    const uint32_t bad = __ballot_sync(0xffffffffu, !good);
+    if (real && role == 0) ok_out[seg] = ((bad >> base) & 0xfu) == 0 ? 1 : 0;
   }
 }
 
@@ -1002,17 +1053,6 @@ void launch_seg_sum(const uint8_t* prods, const uint8_t* okp, const uint32_t* of
 // Scalars are any 256-bit integers, so the recoding covers 257 bits: W = ceil(257 / c)
 // leaves no carry out of the top window.
 
-// bits [w*c, w*c + c) of the 256-bit little-endian scalar; bits at or above 256 read 0 (when
-// c divides 256 the top window starts at bit 256)
-D377_DI uint32_t scalar_window_257(const fq_raw_t& s, int w, int c) {
-  const int bit = w * c;
-  if (bit >= 256) return 0u;
-  const int limb = bit >> 5, off = bit & 31;
-  uint64_t v = s.l[limb];
-  if (limb + 1 < 8) v |= (uint64_t)s.l[limb + 1] << 32;
-  return (uint32_t)(v >> off) & ((1u << c) - 1u);
-}
-
 // One thread per pair of a chunk of J segments.  `offs` (J + 1 entries) are the chunk's
 // segment bounds as absolute pair indices; pair i of the chunk is pair offs[0] + i.  The
 // entry of window w goes to row w of `dig` (window-major, as k_msm_count) with the bucket id
@@ -1036,76 +1076,7 @@ k_msm_count_seg(const uint8_t* __restrict__ scalars, size_t n, const uint32_t* _
   uint32_t id = lo * (uint32_t)g.W * g.K;
   uint32_t* row = dig + i;
 #pragma unroll 1
-  for (int w = 0; w < g.W; w++, row += n, id += g.K) {
-    const uint32_t raw = scalar_window_257(s, w, g.c) + carry;
-    carry = raw > g.K ? 1u : 0u;
-    const int32_t d = (int32_t)raw - (int32_t)(carry << g.c);
-    uint32_t e = 0xffffffffu;
-    if (d != 0) {
-      const uint32_t mag = d < 0 ? (uint32_t)(-d) : (uint32_t)d;
-      atomicAdd(&counts[id + mag - 1], 1u);   // result unused: RED.E.ADD
-      e = (id + mag - 1) | (d < 0 ? 0x80000000u : 0u);
-    }
-    *row = e;
-  }
-}
-
-// Encodings -> affine bucket operands as k_msm_points_affine<D377_PT_ENCODING>, with the decode
-// status of every pair in ok[i] (an invalid encoding is stored as the identity).
-__global__ void __launch_bounds__(kBlk)
-k_msm_points_enc_ok(const uint8_t* __restrict__ pts, size_t n, aff4_t* __restrict__ out, uint8_t* __restrict__ ok) {
-  extern __shared__ uint32_t smem[];
-  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  pt_t p;
-  ok[i] = pt_load_fmt<D377_PT_ENCODING>(p, pts, i, isqrt_smem(smem)) ? 1 : 0;
-  aff4_store(out + i, niels_from_affine(p.x, p.y));
-}
-
-// Horner over the W window sums of every segment of a chunk: one four-lane group per segment
-// (pt_dbl4 / pt_add4 as in k_finish), eight segments per warp.  wsums[j W + w] is window w of
-// segment j.  Stores the canonical Element (out_el + 128 j) and / or the encoding
-// (out_enc + 32 j); ok_out[j] (if wanted) is the AND of the segment's per-pair decode status
-// ok_in[offs[j] .. offs[j + 1]) (all good when ok_in is null).
-constexpr int kSegFinishBlk = 128;
-
-__global__ void __launch_bounds__(kSegFinishBlk)
-k_msm_finish_seg(const pt_t* __restrict__ wsums, uint32_t J, int W, int c, const uint32_t* __restrict__ offs,
-                 const uint8_t* __restrict__ ok_in, uint8_t* __restrict__ out_el, uint8_t* __restrict__ out_enc,
-                 uint8_t* __restrict__ ok_out) {
-  extern __shared__ uint32_t smem[];
-  const int lane = threadIdx.x & 31, role = lane & 3, base = lane & ~3;
-  const size_t seg = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 2;
-  // groups past the end repeat the last segment: the four-lane operations shuffle with a
-  // full mask, so whole warps stay in the loop; only real segments store
-  const bool real = seg < J;
-  const size_t j = real ? seg : (size_t)J - 1;
-  const pt_t* __restrict__ ws = wsums + j * (size_t)W;
-  pt_t r = ptv_load(ws + (W - 1));
-#pragma unroll 1
-  for (int w = W - 2; w >= 0; w--) {
-#pragma unroll 1
-    for (int k = 0; k < c; k++) r = pt_dbl4(r, role, base);
-    r = pt_add4(r, ptv_load(ws + w), role, base);
-  }
-  if (real && role == 0) {
-    D377_DBG_POINT(r);
-    if (out_el) pt_store_canon(out_el + 128 * seg, r);
-  }
-  if (out_enc) {
-    isqrt_smem_t sm = isqrt_smem(smem);
-    fq_t s = pt_compress_to_field(r, sm);
-    if (real && role == 0) fq_store(out_enc + 32 * seg, s);
-  }
-  if (ok_out) {
-    bool good = true;
-    if (ok_in) {
-#pragma unroll 4
-      for (uint32_t i = offs[j] + role; i < offs[j + 1]; i += 4) good = good && ok_in[i] != 0;
-    }
-    const uint32_t bad = __ballot_sync(0xffffffffu, !good);
-    if (real && role == 0) ok_out[seg] = ((bad >> base) & 0xfu) == 0 ? 1 : 0;
-  }
+  for (int w = 0; w < g.W; w++, row += n, id += g.K) *row = digit_entry(s, w, g, carry, id, true, counts);
 }
 
 D377_DBG_READER(msm_debug_counts)
@@ -1199,8 +1170,10 @@ int msm_join(Engine& e) {
   return D377_OK;
 }
 
+// One result: Horner over W window sums (W = 0: the identity) on one warp.
 static int finish(cudaStream_t st, const pt_t* wsums, int W, int c, uint8_t* out_element, uint8_t* out_encoding) {
-  k_finish<<<1, 32, ISQRT_SMEM_WORDS(32) * sizeof(uint32_t), st>>>(wsums, W, c, out_element, out_encoding);
+  k_msm_finish<<<1, 32, ISQRT_SMEM_WORDS(32) * sizeof(uint32_t), st>>>(wsums, 1, W, c, nullptr, nullptr, out_element,
+                                                                       out_encoding, nullptr);
   D377_LAUNCHED();
   D377_CUDA(cudaGetLastError());
   return D377_OK;
@@ -1256,15 +1229,14 @@ int element_sum_on(Engine& e, cudaStream_t st, const uint8_t* elements, size_t n
 int msm_bases_prepare(const uint8_t* points, int point_format, size_t n, uint8_t* records) {
   Engine& e = engine();
   if (n == 0) return D377_OK;
-  aff4_t* aff = (aff4_t*)records;
   uint32_t* dflags = (uint32_t*)(e.d_small + kSmallFlags);
   uint32_t* hflags = (uint32_t*)(e.h_small + kSmallFlags);
   D377_CUDA(cudaMemsetAsync(dflags, 0, 4, e.stream));
-  if (point_format == D377_PT_ELEMENT || point_format == D377_PT_XYZ) {
+  if (projective_format(point_format)) {
     int rc = ensure(e.scratch, n * 32);
     if (rc) return rc;
   }
-  launch_points_affine(e, point_format, points, n, 1, (uint8_t*)e.scratch.p, aff, dflags, e.stream);
+  launch_operands(e, point_format, true, 1, points, n, (uint8_t*)e.scratch.p, records, dflags, nullptr, e.stream);
   D377_CUDA(cudaGetLastError());
   D377_CUDA(cudaMemcpyAsync(hflags, dflags, 4, cudaMemcpyDeviceToHost, e.stream));
   D377_CUDA(cudaStreamSynchronize(e.stream));
@@ -1345,47 +1317,177 @@ static void group_windows(int W, int ngroups, int* wlo, int* whi) {
   }
 }
 
-// Stitch the bucket pieces the accumulation left in 2 * nthreads slots (pb / part) into
-// `bsum`; the slot lists of the later levels rotate through (kbuf[0], pbuf[0]) and
-// (kbuf[1], pbuf[1]).
-static void launch_stitch(cudaStream_t ts, const int32_t* pb, const pt_t* part, size_t nthreads, pt_t* bsum,
-                          int32_t* const kbuf[2], pt_t* const pbuf[2]) {
-  const int32_t* kin = pb;
-  const pt_t* pin = part;
-  size_t nslots = 2 * nthreads;
-  for (int lvl = 0;; lvl++) {
-    size_t nt = (nslots + kSegG - 1) / kSegG;
-    int32_t* kout = kbuf[lvl & 1];
-    pt_t* pout = pbuf[lvl & 1];
-    // work-efficient serial fold while the level is large, warp scan (log depth) below
+// ---- one Pippenger pass (sort, accumulation, tail), shared by msm_once and the segmented MSM ----
+struct PassPlan {
+  int L;              // sorted entries per accumulation thread
+  int log_lseg;       // buckets per bucket-reduction thread: Lseg = 2^log_lseg
+  uint32_t Lseg, S;   // S = ceil(K / Lseg) segments per bucket set
+};
+
+// The run lengths of a pass whose sort holds at most `max_entries` entries.
+static PassPlan pass_plan(MsmGeom g, size_t max_entries) {
+  PassPlan pl;
+  // Run length per accumulate thread.  Every run boundary splits a bucket into pieces
+  // that k_msm_seg_reduce has to stitch (one extra addition each), so runs are as long
+  // as the thread count allows: >= ~2 full waves of 128-thread CTAs on 148 SMs.
+  pl.L = max_entries >= ((size_t)1 << 27) ? 128 : max_entries >= ((size_t)1 << 25) ? 64 : 32;
+  // Buckets per bucket-reduce thread.  With the weighted tree (k_wsum_tree) a segment
+  // costs no scalar multiplication, so segments can be short: many threads, short
+  // dependent chains.
+  // With the tails hidden under the next MSM's head, their pipe work matters
+  // more than their latency: longer segments (fewer doublings and tree nodes) win once a
+  // window has many buckets -- measured back to back: 2^22 7.64 / 7.49 / 7.42 ms and 2^24
+  // 27.08 / 26.97 / 27.00 ms with 16 / 32 / 64, 2^20 (c = 16) 2.43 / 2.48 / 2.64 ms.
+  pl.log_lseg = g.c >= 18 ? 6 : g.c == 17 ? 5 : 4;
+  pl.Lseg = 1u << pl.log_lseg;   // power of two: P_s = Lseg * R_s by doublings
+  pl.S = (g.K + pl.Lseg - 1) / pl.Lseg;
+  return pl;
+}
+
+// Bucket additions against affine records cost 7 M instead of 8: free when the input
+// already has Z = 1; Element inputs are normalised first when the batch is large enough
+// for the one-inversion-per-CTA trick to pay (7 M + one inversion per CTA against W
+// multiplications saved).
+// d377_msm_set_normalize: -1 never, 1 always (at least 4 points per thread), 0 from 2^20 pairs
+static bool affine_operands(const Engine& e, int fmt, size_t n) {
+  const int want = e.msm_normalize_override;
+  return !projective_format(fmt) || want > 0 || (want == 0 && (n >> 17) >= 8);
+}
+static size_t normalize_min_per(const Engine& e) { return e.msm_normalize_override > 0 ? 4 : 1; }
+
+// Cuts a workspace into 256-byte aligned arrays.  With base = 0 it only sizes them: a driver
+// lays its workspace out once to learn the bytes to ensure() and once over the buffer.
+struct Carver {
+  uintptr_t base;
+  size_t off = 0;
+  template <class T = uint8_t>
+  T* take(size_t bytes) {
+    T* p = reinterpret_cast<T*>(base + off);
+    off += align_up(bytes);
+    return p;
+  }
+};
+
+struct PassWs {
+  uint32_t *dig, *sorted;   // digit entries and sorted list, window-major
+  uint32_t *counts[kMaxGroups], *cursor[kMaxGroups], *tiles[kMaxGroups];   // per window group
+  pt_t* bsum;               // bucket sums
+  pt_t* part;               // two piece slots per accumulation thread, and their keys
+  int32_t* pb;
+  int32_t* kbuf[2];         // second and third stitch level (the levels ping-pong between them)
+  pt_t* pbuf[2];
+  pt_t *a, *p, *a2, *p2;    // segment nodes of the bucket reduction and of the weighted tree
+};
+
+static size_t scan_tiles(size_t nb) { return (nb + 1 + kScanTile - 1) / kScanTile; }
+
+// A pass over `entries` sorted entries, `ngroups` window groups of gnb[k] buckets, `nthreads`
+// accumulation threads and `rows` bucket sets of g.K buckets, each reduced in S segments.
+static PassWs carve_pass(Carver& cv, size_t entries, int ngroups, const size_t* gnb, size_t nthreads, size_t rows,
+                         MsmGeom g, uint32_t S) {
+  PassWs w;
+  w.dig = cv.take<uint32_t>(entries * 4);
+  w.sorted = cv.take<uint32_t>(entries * 4);
+  for (int k = 0; k < ngroups; k++) {
+    w.counts[k] = cv.take<uint32_t>((gnb[k] + 1) * 4);
+    w.cursor[k] = cv.take<uint32_t>((gnb[k] + 1) * 4);
+    w.tiles[k] = cv.take<uint32_t>(scan_tiles(gnb[k]) * 4 + 4);
+  }
+  w.bsum = cv.take<pt_t>(rows * g.K * sizeof(pt_t));
+  w.part = cv.take<pt_t>(2 * nthreads * sizeof(pt_t));
+  w.pb = cv.take<int32_t>(2 * nthreads * 4);
+  const size_t nthreads2 = (2 * nthreads + kSegG - 1) / kSegG;
+  const size_t nthreads3 = (2 * nthreads2 + kSegG - 1) / kSegG;
+  w.pbuf[0] = cv.take<pt_t>(2 * nthreads2 * sizeof(pt_t));
+  w.kbuf[0] = cv.take<int32_t>(2 * nthreads2 * 4);
+  w.pbuf[1] = cv.take<pt_t>(2 * nthreads3 * sizeof(pt_t));
+  w.kbuf[1] = cv.take<int32_t>(2 * nthreads3 * 4);
+  const size_t seg_n = rows * S, seg_n2 = rows * ((S + kWT - 1) / kWT);
+  w.a = cv.take<pt_t>(seg_n * sizeof(pt_t));
+  w.p = cv.take<pt_t>(seg_n * sizeof(pt_t));
+  w.a2 = cv.take<pt_t>(seg_n2 * sizeof(pt_t));
+  w.p2 = cv.take<pt_t>(seg_n2 * sizeof(pt_t));
+  return w;
+}
+
+static unsigned grid_cap(size_t want, unsigned cap) { return (unsigned)(cap ? std::min<size_t>(want, cap) : want); }
+
+// The counting sort after a count kernel has filled `counts` (nb + 1 words) and the rows x n
+// entries of `dig`: scan of the counts into bucket offsets (copied into `cursor`), then the
+// scatter into `sorted`.  `cap` (0: none) bounds the scatter's grid; n = 0 (a chunk of empty
+// segments) only computes the offsets.
+static void launch_sort(cudaStream_t s, uint32_t* counts, uint32_t* cursor, uint32_t* tiles, size_t nb,
+                        const uint32_t* dig, size_t n, uint32_t rows, uint32_t* sorted, uint32_t rec_base,
+                        uint32_t rec_stride, unsigned cap) {
+  const size_t ntiles = scan_tiles(nb);
+  k_scan_tiles<<<(unsigned)ntiles, kScanBlock, 0, s>>>(counts, nb + 1, tiles);
+  D377_LAUNCHED();
+  k_scan_sums<<<1, kScanBlock, 0, s>>>(tiles, ntiles, tiles + ntiles);
+  D377_LAUNCHED();
+  k_scan_apply<<<(unsigned)ntiles, kScanBlock, 0, s>>>(counts, nb + 1, tiles, cursor);
+  D377_LAUNCHED();
+  if (n == 0) return;
+  k_msm_scatter<<<grid_cap((size_t)grid_for(n, 256 * kScatterIlp) * rows, cap), 256, 0, s>>>(
+      dig, n, rows, cursor, sorted, rec_base, rec_stride);
+  D377_LAUNCHED();
+}
+
+// Bucket accumulation of `nthreads` runs of L sorted entries; the nb buckets start at bucket b0
+// of `bsum`.
+static void launch_accumulate(cudaStream_t s, bool affine, const void* ops, const uint32_t* sorted,
+                              const uint32_t* offsets, size_t nb, int L, size_t nthreads, pt_t* bsum, size_t b0,
+                              pt_t* part, int32_t* pb) {
+  auto k = affine ? k_msm_accumulate<true> : k_msm_accumulate<false>;
+  k<<<grid_for(nthreads, kBlk), kBlk, 0, s>>>(ops, sorted, offsets, (uint32_t)nb, L, bsum + b0, part, pb, (int32_t)b0);
+  D377_LAUNCHED();
+}
+
+// The tail of a pass on `s`: reduction of the `rows` bucket sets (their offsets in `gt`) to
+// *sums, one point per row.  `marks` (may be null): two events recorded after the stitch and
+// after the bucket reduction.
+static int launch_tail(cudaStream_t s, const PassWs& w, size_t nthreads, const GroupTab& gt, MsmGeom g, size_t rows,
+                       const PassPlan& pl, const cudaEvent_t* marks, pt_t** sums) {
+  // Stitch the bucket pieces the accumulation left in 2 * nthreads slots (none: nothing to
+  // stitch) into `bsum`; the slot lists of the later levels rotate through (kbuf, pbuf)[0]
+  // and [1].  Work-efficient serial fold while a level is large, warp scan (log depth) below.
+  const int32_t* kin = w.pb;
+  const pt_t* pin = w.part;
+  for (size_t nslots = 2 * nthreads, lvl = 0; nslots; lvl++) {
+    const size_t nt = (nslots + kSegG - 1) / kSegG;
+    int32_t* kout = w.kbuf[lvl & 1];
+    pt_t* pout = w.pbuf[lvl & 1];
     if (nslots <= kStitchWarpSlots)
-      k_msm_seg_reduce_warp<<<grid_for(nt * 32, kBlk), kBlk, 0, ts>>>(kin, pin, nslots, bsum, kout, pout, nt);
+      k_msm_seg_reduce_warp<<<grid_for(nt * 32, kBlk), kBlk, 0, s>>>(kin, pin, nslots, w.bsum, kout, pout, nt);
     else
-      k_msm_seg_reduce<<<grid_for(nt, kBlk), kBlk, 0, ts>>>(kin, pin, nslots, bsum, kout, pout, nt);
+      k_msm_seg_reduce<<<grid_for(nt, kBlk), kBlk, 0, s>>>(kin, pin, nslots, w.bsum, kout, pout, nt);
     D377_LAUNCHED();
-    if (nt == 1) break;
-    nslots = 2 * nt;
+    nslots = nt == 1 ? 0 : 2 * nt;
     kin = kout;
     pin = pout;
   }
-}
-
-// Weighted tree over `rows` rows of `len` segment nodes (a, p) -> one node per row, in (a, p)
-// on return (the buffers ping-pong with a2 / p2).  The row is gridDim.y, so a launch covers
-// at most 65 535 rows; more rows are launched in slices.
-static void launch_wsum_tree(cudaStream_t ts, pt_t*& a, pt_t*& p, pt_t*& a2, pt_t*& p2, uint32_t len, size_t rows) {
+  if (marks) D377_CUDA(cudaEventRecord(marks[0], s));
+  k_msm_bucket_reduce_ap<<<grid_for(rows * pl.S, kBlk), kBlk, 0, s>>>(w.bsum, gt, geom(g.c, (int)rows), pl.Lseg,
+                                                                       pl.log_lseg, pl.S, w.a, w.p);
+  D377_LAUNCHED();
+  D377_CUDA(cudaGetLastError());
+  if (marks) D377_CUDA(cudaEventRecord(marks[1], s));
+  // Weighted tree over the rows of S segment nodes (a, p), ping-ponging with (a2, p2).  The
+  // row is gridDim.y, so a launch covers at most 65 535 rows; more rows are launched in slices.
   constexpr size_t kMaxRows = 65535;
-  while (len > 1) {
+  pt_t *a = w.a, *p = w.p, *a2 = w.a2, *p2 = w.p2;
+  for (uint32_t len = pl.S; len > 1;) {
     const uint32_t olen = (len + kWT - 1) / kWT;
     for (size_t r0 = 0; r0 < rows; r0 += kMaxRows) {
       const unsigned nr = (unsigned)std::min(kMaxRows, rows - r0);
-      k_wsum_tree<<<dim3(olen, nr), 2 * kWT, 0, ts>>>(a + r0 * len, p + r0 * len, len, a2 + r0 * olen, p2 + r0 * olen);
+      k_wsum_tree<<<dim3(olen, nr), 2 * kWT, 0, s>>>(a + r0 * len, p + r0 * len, len, a2 + r0 * olen, p2 + r0 * olen);
       D377_LAUNCHED();
     }
     std::swap(a, a2);
     std::swap(p, p2);
     len = olen;
   }
+  *sums = a;
+  return D377_OK;
 }
 
 // One Pippenger.  Head (point conversion, sort, bucket accumulation) on the engine and sort
@@ -1413,30 +1515,10 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   if (rc) return rc;
   MsmState& ms = e.msm;
   const bool windowed = point_format == D377_PT_BASES && bases && bases->c > 0;
-  MsmGeom g;
-  if (windowed) {
-    g.c = bases->c;
-    g.W = bases->W;
-    g.K = 1u << (g.c - 1);
-  } else {
-    g = choose_geom(e, n);
-  }
+  const MsmGeom g = windowed ? geom(bases->c, bases->W) : choose_geom(e, n);
   const size_t max_entries = n * (size_t)g.W;
-  // Run length per accumulate thread.  Every run boundary splits a bucket into pieces
-  // that k_msm_seg_reduce has to stitch (one extra addition each), so runs are as long
-  // as the thread count allows: >= ~2 full waves of 128-thread CTAs on 148 SMs.
-  const int L = max_entries >= ((size_t)1 << 27) ? 128 : max_entries >= ((size_t)1 << 25) ? 64 : 32;
   if (max_entries >= 0xfffffff0ull) { set_error("msm chunk too large"); return D377_ERR_INVALID_ARG; }
-  // Buckets per bucket-reduce thread.  With the weighted tree (k_wsum_tree) a segment
-  // costs no scalar multiplication, so segments can be short: many threads, short
-  // dependent chains.
-  // With the tails hidden under the next MSM's head, their pipe work matters
-  // more than their latency: longer segments (fewer doublings and tree nodes) win once a
-  // window has many buckets -- measured back to back: 2^22 7.64 / 7.49 / 7.42 ms and 2^24
-  // 27.08 / 26.97 / 27.00 ms with 16 / 32 / 64, 2^20 (c = 16) 2.43 / 2.48 / 2.64 ms.
-  const int log_lseg = g.c >= 18 ? 6 : g.c == 17 ? 5 : 4;
-  const uint32_t Lseg = 1u << log_lseg;   // power of two: P_s = Lseg * R_s by doublings
-  const uint32_t S = (g.K + Lseg - 1) / Lseg;
+  const PassPlan pl = pass_plan(g, max_entries);
 
   // Window groups: group k+1 is sorted (sort stream) while group k is accumulated (engine
   // stream).  Small MSMs run as one group: the extra launches would cost more than the
@@ -1458,43 +1540,29 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   group_windows(g.W, ngroups, wlo, whi);
   // sort kernels beside a resident accumulation: one 256-thread CTA per SM
   const unsigned sort_cap = ngroups > 1 || may_prefetch ? (unsigned)e.sm_count : 0u;
-  auto capped = [&](size_t want) { return (unsigned)(sort_cap ? std::min<size_t>(want, sort_cap) : want); };
   // Buckets of group k: one set per window, or one merged set (windowed bases).  g_bucket[k]
-  // is the group's first bucket in `bsum`; rg is the geometry the bucket reduction sees (a
-  // merged set is reduced like one window).
-  size_t g_nthreads[kMaxGroups], g_tbase[kMaxGroups + 1], g_ntiles[kMaxGroups];
+  // is the group's first bucket in `bsum`; `rows` are the bucket sets the bucket reduction
+  // sees (a merged set is reduced like one window).
+  size_t g_nthreads[kMaxGroups], g_tbase[kMaxGroups + 1];
   size_t g_nb[kMaxGroups], g_bucket[kMaxGroups];
   g_tbase[0] = 0;
   for (int k = 0; k < ngroups; k++) {
     size_t ent_k = (size_t)(whi[k] - wlo[k]) * n;
-    g_nthreads[k] = (ent_k + L - 1) / L;
+    g_nthreads[k] = (ent_k + pl.L - 1) / pl.L;
     g_tbase[k + 1] = g_tbase[k] + g_nthreads[k];
     g_nb[k] = windowed ? (size_t)g.K : (size_t)(whi[k] - wlo[k]) * g.K;
     g_bucket[k] = windowed ? (size_t)k * g.K : (size_t)wlo[k] * g.K;
-    g_ntiles[k] = (g_nb[k] + 1 + kScanTile - 1) / kScanTile;
   }
   const size_t nthreads = g_tbase[ngroups];
-  MsmGeom rg = g;
-  if (windowed) rg.W = ngroups;
-  const size_t nb = (size_t)rg.W * g.K;
+  const size_t rows = windowed ? (size_t)ngroups : (size_t)g.W;
 
-  // Bucket additions against affine records cost 7 M instead of 8: free when the input
-  // already has Z = 1; Element inputs are normalised first when the batch is large enough
-  // for the one-inversion-per-CTA trick to pay (7 M + one inversion per CTA against W
-  // multiplications saved).
-  const bool projective = point_format == D377_PT_ELEMENT || point_format == D377_PT_XYZ;
   const bool prepared = point_format == D377_PT_BASES;   // `points` already holds the bucket operands
-  // d377_msm_set_normalize: -1 never, 1 always (at least 4 points per thread), 0 from 2^20 pairs
-  const int want_normalize = e.msm_normalize_override;
-  const bool normalize = projective && (want_normalize > 0 || (want_normalize == 0 && (n >> 17) >= 8));
-  const bool affine = !projective || normalize;
+  const bool affine = affine_operands(e, point_format, n);
 
   // ---- workspaces -----------------------------------------------------------------
   // Two complete sets (bucket operands, digits, sorted lists, offsets, bucket sums, piece
   // slots): the conversion of the points and the sort of the NEXT MSM run under this MSM's
   // bucket accumulation, and the tail of this MSM under the next MSM's accumulation.
-  size_t off = 0;
-  auto carve = [&](size_t bytes) { size_t o = off; off += align_up(bytes); return o; };
   // The other set is only needed while the previous MSM is still in flight: a caller that
   // waits for every result (d377_msm_dev, d377_msm) keeps using set 0 and pays for one.
   int set = 0;
@@ -1503,45 +1571,20 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
     set = ms.cur_set ^ 1;
   cudaGetLastError();
   ms.cur_set = set;
-  size_t o_cached = carve(prepared ? 0 : n * sizeof(cached_t));
-  size_t o_norm = carve(normalize ? n * 32 : 0);
-  size_t o_dig = carve(max_entries * 4);
-  size_t o_sorted = carve(max_entries * 4);
-  size_t o_sc = carve(sc_mont ? n * 32 : 0);
-  size_t o_counts[kMaxGroups], o_cursor[kMaxGroups], o_tiles[kMaxGroups];
-  for (int k = 0; k < ngroups; k++) {
-    o_counts[k] = carve((g_nb[k] + 1) * 4);
-    o_cursor[k] = carve((g_nb[k] + 1) * 4);
-    o_tiles[k] = carve(g_ntiles[k] * 4 + 4);
-  }
-  size_t o_bsum = carve(nb * sizeof(pt_t));
-  size_t o_part = carve(2 * nthreads * sizeof(pt_t));
-  size_t o_pb = carve(2 * nthreads * 4);
-  // second and third stitch level (the levels ping-pong between them)
-  const size_t nthreads2 = (2 * nthreads + kSegG - 1) / kSegG;
-  const size_t nthreads3 = (2 * nthreads2 + kSegG - 1) / kSegG;
-  size_t o_part2 = carve(2 * nthreads2 * sizeof(pt_t));
-  size_t o_pb2 = carve(2 * nthreads2 * 4);
-  size_t o_part3 = carve(2 * nthreads3 * sizeof(pt_t));
-  size_t o_pb3 = carve(2 * nthreads3 * 4);
-  const size_t seg_n = (size_t)rg.W * S, seg_n2 = (size_t)rg.W * ((S + kWT - 1) / kWT);
-  size_t o_seg_a = carve(seg_n * sizeof(pt_t));
-  size_t o_seg_p = carve(seg_n * sizeof(pt_t));
-  size_t o_seg_a2 = carve(seg_n2 * sizeof(pt_t));
-  size_t o_seg_p2 = carve(seg_n2 * sizeof(pt_t));
-  rc = ensure(ms.tail_ws[set], off);
+  uint8_t *ops = nullptr, *norm = nullptr, *sc = nullptr;
+  PassWs w;
+  auto layout = [&](uintptr_t base) {
+    Carver cv{base};
+    ops = cv.take(prepared ? 0 : n * sizeof(cached_t));
+    norm = cv.take(affine && projective_format(point_format) ? n * 32 : 0);
+    sc = cv.take(sc_mont ? n * 32 : 0);
+    w = carve_pass(cv, max_entries, ngroups, g_nb, nthreads, rows, g, pl.S);
+    return cv.off;
+  };
+  rc = ensure(ms.tail_ws[set], layout(0));
   if (rc) return rc;
-
-  uint8_t* tw = (uint8_t*)ms.tail_ws[set].p;
-  uint8_t* ws = tw;
-  cached_t* cached = (cached_t*)(ws + o_cached);
-  const aff4_t* aff_in = prepared ? (const aff4_t*)points : (const aff4_t*)(ws + o_cached);
-  aff4_t* aff = (aff4_t*)(ws + o_cached);
-  uint32_t* dig = (uint32_t*)(tw + o_dig);
-  uint32_t* sorted = (uint32_t*)(tw + o_sorted);
-  pt_t* bsum = (pt_t*)(tw + o_bsum);
-  pt_t* part = (pt_t*)(tw + o_part);
-  int32_t* pb = (int32_t*)(tw + o_pb);
+  layout((uintptr_t)ms.tail_ws[set].p);
+  const void* ops_in = prepared ? (const void*)points : ops;
   cudaStream_t st = e.stream, ss = ms.sort_stream;
   // point conversion / normalisation: on the engine stream, or -- when the inputs are known to
   // be ready -- on a stream of its own, so that it runs under the previous MSM's accumulation
@@ -1592,48 +1635,29 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   // scalars as the reference holds them in memory (Montgomery limbs): converted on the sort
   // stream into the workspace set before the digits are cut
   if (sc_mont) {
-    launch_fr_from_mont(scalars, n, tw + o_sc, ss);
-    scalars = tw + o_sc;
+    launch_fr_from_mont(scalars, n, sc, ss);
+    scalars = sc;
   }
 
   // ---- scalar side, all groups, on the sort stream (2, 3, 4) ----
   for (int k = 0; k < ngroups; k++) {
     const int wa = wlo[k], wb = whi[k];
-    const size_t nbk = g_nb[k];
-    uint32_t* counts = (uint32_t*)(tw + o_counts[k]);
-    uint32_t* tiles = (uint32_t*)(tw + o_tiles[k]);
-    uint32_t* cursor = (uint32_t*)(tw + o_cursor[k]);
-    D377_CUDA(cudaMemsetAsync(counts, 0, (nbk + 1) * 4, ss));
-    k_msm_count<<<capped(grid_for(n, 256)), 256, 0, ss>>>(scalars, n, g, wa, wb, windowed ? 0u : g.K, counts,
-                                                          dig + (size_t)wa * n, flags);
+    D377_CUDA(cudaMemsetAsync(w.counts[k], 0, (g_nb[k] + 1) * 4, ss));
+    k_msm_count<<<grid_cap(grid_for(n, 256), sort_cap), 256, 0, ss>>>(scalars, n, g, wa, wb, windowed ? 0u : g.K,
+                                                                      w.counts[k], w.dig + (size_t)wa * n, flags);
     D377_LAUNCHED();
-    k_scan_tiles<<<(unsigned)g_ntiles[k], kScanBlock, 0, ss>>>(counts, nbk + 1, tiles);
-    D377_LAUNCHED();
-    k_scan_sums<<<1, kScanBlock, 0, ss>>>(tiles, g_ntiles[k], tiles + g_ntiles[k]);
-    D377_LAUNCHED();
-    k_scan_apply<<<(unsigned)g_ntiles[k], kScanBlock, 0, ss>>>(counts, nbk + 1, tiles, cursor);
-    D377_LAUNCHED();
-    k_msm_scatter<<<capped((size_t)grid_for(n, 256 * kScatterIlp) * (size_t)(wb - wa)), 256, 0, ss>>>(
-        dig + (size_t)wa * n, n, (uint32_t)(wb - wa), cursor, sorted + (size_t)wa * n,
-        windowed ? (uint32_t)((size_t)wa * bases->n) : 0u, windowed ? (uint32_t)bases->n : 0u);
-    D377_LAUNCHED();
+    launch_sort(ss, w.counts[k], w.cursor[k], w.tiles[k], g_nb[k], w.dig + (size_t)wa * n, n, (uint32_t)(wb - wa),
+                w.sorted + (size_t)wa * n, windowed ? (uint32_t)((size_t)wa * bases->n) : 0u,
+                windowed ? (uint32_t)bases->n : 0u, sort_cap);
     D377_CUDA(cudaEventRecord(ms.ev_sorted[k], ss));
   }
   D377_CUDA(cudaEventRecord(ms.ev_sort1, ss));
 
   // ---- point side on the engine stream ----
-  D377_CUDA(cudaMemsetAsync(pb, 0xff, 2 * nthreads * 4, st));
+  D377_CUDA(cudaMemsetAsync(w.pb, 0xff, 2 * nthreads * 4, st));
   // 1
   if (!prepared) {
-    if (affine) {
-      launch_points_affine(e, point_format, points, n, want_normalize > 0 ? 4 : 1, ws + o_norm, aff, flags, ps);
-    } else {
-      if (point_format == D377_PT_ELEMENT)
-        k_msm_points<D377_PT_ELEMENT><<<grid_for(n, kBlk), kBlk, 0, ps>>>(points, n, cached);
-      else
-        k_msm_points<D377_PT_XYZ><<<grid_for(n, kBlk), kBlk, 0, ps>>>(points, n, cached);
-      D377_LAUNCHED();
-    }
+    launch_operands(e, point_format, affine, normalize_min_per(e), points, n, norm, ops, flags, nullptr, ps);
     if (pts_prefetch) {
       D377_CUDA(cudaEventRecord(ms.ev_points_done[set], ps));
       D377_CUDA(cudaStreamWaitEvent(st, ms.ev_points_done[set], 0));
@@ -1644,53 +1668,30 @@ static int msm_once(const uint8_t* scalars, const uint8_t* points, int point_for
   // 128 threads, ~106 registers, 4 CTAs/SM: measured flat from 4 to 7 CTAs/SM (the
   // fmaheavy pipe, not latency, is the limiter), slower at 8 (spills).
   for (int k = 0; k < ngroups; k++) {
-    const int wa = wlo[k];
-    const size_t nbk = g_nb[k], b0 = g_bucket[k];
-    const uint32_t* counts = (const uint32_t*)(tw + o_counts[k]);
     D377_CUDA(cudaStreamWaitEvent(st, ms.ev_sorted[k], 0));
     D377_CUDA(cudaEventRecord(ms.ev_acc0[k], st));
-    if (affine)
-      k_msm_accumulate<true><<<grid_for(g_nthreads[k], kBlk), kBlk, 0, st>>>(
-          aff_in, sorted + (size_t)wa * n, counts, (uint32_t)nbk, L, bsum + b0,
-          part + 2 * g_tbase[k], pb + 2 * g_tbase[k], (int32_t)b0);
-    else
-      k_msm_accumulate<false><<<grid_for(g_nthreads[k], kBlk), kBlk, 0, st>>>(
-          cached, sorted + (size_t)wa * n, counts, (uint32_t)nbk, L, bsum + b0,
-          part + 2 * g_tbase[k], pb + 2 * g_tbase[k], (int32_t)b0);
-    D377_LAUNCHED();
+    launch_accumulate(st, affine, ops_in, w.sorted + (size_t)wlo[k] * n, w.counts[k], g_nb[k], pl.L, g_nthreads[k],
+                      w.bsum, g_bucket[k], w.part + 2 * g_tbase[k], w.pb + 2 * g_tbase[k]);
     D377_CUDA(cudaEventRecord(ms.ev_acc[k], st));
   }
   D377_CUDA(stage_mark(5, st));
   // ---- tail: everything below runs on the tail stream ----
   D377_CUDA(cudaEventRecord(ms.ev_acc_done, st));
   if (ts != st) D377_CUDA(cudaStreamWaitEvent(ts, ms.ev_acc_done, 0));
-  // 6: stitch the bucket pieces of all groups
-  {
-    int32_t* kbuf[2] = {(int32_t*)(tw + o_pb2), (int32_t*)(tw + o_pb3)};
-    pt_t* pbuf[2] = {(pt_t*)(tw + o_part2), (pt_t*)(tw + o_part3)};
-    launch_stitch(ts, pb, part, nthreads, bsum, kbuf, pbuf);
+  // 6: stitch the bucket pieces of all groups (stage 6 ends), 7: bucket reduction of every
+  // window (stage 7 ends), 8: weighted tree -> one sum per window, Horner over the windows
+  GroupTab gt;
+  gt.ng = ngroups;
+  for (int k = 0; k < ngroups; k++) {
+    gt.wlo[k] = windowed ? k : wlo[k];
+    gt.whi[k] = windowed ? k + 1 : whi[k];
+    gt.offs[k] = w.counts[k];
   }
-  D377_CUDA(stage_mark(6, ts));
-  // 7: bucket reduction of every window
-  pt_t *a = (pt_t*)(tw + o_seg_a), *p = (pt_t*)(tw + o_seg_p);
-  pt_t *a2 = (pt_t*)(tw + o_seg_a2), *p2 = (pt_t*)(tw + o_seg_p2);
-  {
-    GroupTab gt;
-    gt.ng = ngroups;
-    for (int k = 0; k < ngroups; k++) {
-      gt.wlo[k] = windowed ? k : wlo[k];
-      gt.whi[k] = windowed ? k + 1 : whi[k];
-      gt.offs[k] = (const uint32_t*)(tw + o_counts[k]);
-    }
-    k_msm_bucket_reduce_ap<<<grid_for((size_t)rg.W * S, kBlk), kBlk, 0, ts>>>(bsum, gt, rg, Lseg, log_lseg, S, a, p);
-    D377_LAUNCHED();
-  }
-  D377_CUDA(cudaGetLastError());
-  D377_CUDA(stage_mark(7, ts));
-  // 8: weighted tree -> one sum per window, Horner over the windows, output
-  launch_wsum_tree(ts, a, p, a2, p2, S, (size_t)rg.W);
-  // windowed: the group sums are already weighted by 2^(c w), k_finish only adds them
-  rc = finish(ts, a, rg.W, windowed ? 0 : g.c, out_element, out_encoding);
+  pt_t* sums = nullptr;
+  rc = launch_tail(ts, w, nthreads, gt, g, rows, pl, &ms.ev_stage[6], &sums);
+  if (rc) return rc;
+  // windowed: the group sums are already weighted by 2^(c w), k_msm_finish only adds them
+  rc = finish(ts, sums, (int)rows, windowed ? 0 : g.c, out_element, out_encoding);
   if (rc) return rc;
   D377_CUDA(stage_mark(8, ts));
   D377_CUDA(cudaEventRecord(ms.ev_tail_done[set], ts));
@@ -1811,28 +1812,15 @@ int msm_dev_async(const uint8_t* scalars, const uint8_t* points, int point_forma
 constexpr size_t kSegBucketBudget = (size_t)1 << 30;
 constexpr size_t kSegMaxEntries = 0xfffffff0ull;   // entries (pairs x W) of a chunk, as msm_once
 
-static MsmGeom seg_geom(int c) {
-  MsmGeom g;
-  g.c = c;
-  g.W = (257 + c - 1) / c;   // any 256-bit scalar: no carry out of the top window
-  g.K = 1u << (c - 1);
-  return g;
-}
-
-// Bucket operands: affine records (7 M per addition) unless projective inputs are too few for
-// the batch normalisation to pay -- msm_once's rule, over all pairs of the call.
-static bool seg_normalize(const Engine& e, int fmt, size_t n) {
-  const bool projective = fmt == D377_PT_ELEMENT || fmt == D377_PT_XYZ;
-  const int want = e.msm_normalize_override;
-  return projective && (want > 0 || (want == 0 && (n >> 17) >= 8));
-}
+// any 256-bit scalar: no carry out of the top window
+static MsmGeom seg_geom(int c) { return geom(c, (257 + c - 1) / c); }
 
 int msm_segmented_width(Engine& e, int fmt, const uint32_t* offsets, size_t nmsm, int* c_out) {
   const size_t n = offsets[nmsm];
   size_t longest = 0;
   for (size_t j = 0; j < nmsm; j++) longest = std::max<size_t>(longest, offsets[j + 1] - offsets[j]);
-  const bool projective = fmt == D377_PT_ELEMENT || fmt == D377_PT_XYZ;
-  const double madd = projective && !seg_normalize(e, fmt, n) ? 8.0 : 7.0;
+  // bucket operands as msm_once's, over all pairs of the call
+  const double madd = affine_operands(e, fmt, n) ? 7.0 : 8.0;
   const int lo = e.msm_window_override ? e.msm_window_override : 4;
   const int hi = e.msm_window_override ? e.msm_window_override : 16;
   int best_c = 0;
@@ -1880,45 +1868,28 @@ int msm_segmented_enqueue(const uint8_t* scalars, const uint8_t* points, int fmt
     j0 += J;
   }
   const size_t max_entries = max_pairs * g.W;
-  const int L = max_entries >= ((size_t)1 << 27) ? 128 : max_entries >= ((size_t)1 << 25) ? 64 : 32;
-  const int log_lseg = g.c >= 18 ? 6 : g.c == 17 ? 5 : 4;
-  const uint32_t Lseg = 1u << log_lseg;
-  const uint32_t S = (g.K + Lseg - 1) / Lseg;
-  const bool normalize = seg_normalize(e, fmt, n);
-  const bool affine = !(fmt == D377_PT_ELEMENT || fmt == D377_PT_XYZ) || normalize;
+  const PassPlan pl = pass_plan(g, max_entries);
+  const bool affine = affine_operands(e, fmt, n);
 
-  // ---- workspace: the call's converted points, then one chunk's sort and tail ----
-  size_t off = 0;
-  auto carve = [&](size_t bytes) { size_t o = off; off += align_up(bytes); return o; };
-  const size_t o_offs = carve((nmsm + 1) * 4);
-  const size_t o_sc = carve(sc_mont ? n * 32 : 0);
-  const size_t o_pts = carve(n * 128);
-  const size_t o_norm = carve(normalize ? n * 32 : 0);
-  const size_t o_okp = carve(fmt == D377_PT_ENCODING ? n : 0);
-  const size_t max_nb = max_J * WK, max_threads = (max_entries + L - 1) / L;
-  const size_t max_tiles = (max_nb + 1 + kScanTile - 1) / kScanTile;
-  const size_t o_dig = carve(max_entries * 4);
-  const size_t o_sorted = carve(max_entries * 4);
-  const size_t o_counts = carve((max_nb + 1) * 4);
-  const size_t o_cursor = carve((max_nb + 1) * 4);
-  const size_t o_tiles = carve(max_tiles * 4 + 4);
-  const size_t o_bsum = carve(max_nb * sizeof(pt_t));
-  const size_t o_part = carve(2 * max_threads * sizeof(pt_t));
-  const size_t o_pb = carve(2 * max_threads * 4);
-  const size_t nthreads2 = (2 * max_threads + kSegG - 1) / kSegG;
-  const size_t nthreads3 = (2 * nthreads2 + kSegG - 1) / kSegG;
-  const size_t o_part2 = carve(2 * nthreads2 * sizeof(pt_t));
-  const size_t o_pb2 = carve(2 * nthreads2 * 4);
-  const size_t o_part3 = carve(2 * nthreads3 * sizeof(pt_t));
-  const size_t o_pb3 = carve(2 * nthreads3 * 4);
-  const size_t max_rows = max_J * g.W;
-  const size_t o_seg_a = carve(max_rows * S * sizeof(pt_t));
-  const size_t o_seg_p = carve(max_rows * S * sizeof(pt_t));
-  const size_t o_seg_a2 = carve(max_rows * ((S + kWT - 1) / kWT) * sizeof(pt_t));
-  const size_t o_seg_p2 = carve(max_rows * ((S + kWT - 1) / kWT) * sizeof(pt_t));
-  int rc = ensure(e.seg_ws, off);
+  // ---- workspace: the call's offsets, scalars, bucket operands and decode status, then one
+  // chunk's pass ----
+  uint32_t* d_offs = nullptr;
+  uint8_t *sc = nullptr, *ops = nullptr, *norm = nullptr, *okp = nullptr;
+  PassWs w;
+  const size_t max_nb = max_J * WK;
+  auto layout = [&](uintptr_t base) {
+    Carver cv{base};
+    d_offs = cv.take<uint32_t>((nmsm + 1) * 4);
+    sc = cv.take(sc_mont ? n * 32 : 0);
+    ops = cv.take(n * 128);
+    norm = cv.take(affine && projective_format(fmt) ? n * 32 : 0);
+    okp = fmt == D377_PT_ENCODING ? cv.take(n) : nullptr;
+    w = carve_pass(cv, max_entries, 1, &max_nb, (max_entries + pl.L - 1) / pl.L, max_J * g.W, g, pl.S);
+    return cv.off;
+  };
+  int rc = ensure(e.seg_ws, layout(0));
   if (rc) return rc;
-  uint8_t* ws = (uint8_t*)e.seg_ws.p;
+  layout((uintptr_t)e.seg_ws.p);
   cudaStream_t st = e.stream;
 
   // The offsets go up through a pinned staging copy, so that the caller may reuse its array
@@ -1934,95 +1905,47 @@ int msm_segmented_enqueue(const uint8_t* scalars, const uint8_t* points, int fmt
     e.seg_off_cap = off_bytes;
   }
   memcpy(e.seg_off_host, offsets, off_bytes);
-  uint32_t* d_offs = (uint32_t*)(ws + o_offs);
   D377_CUDA(cudaMemcpyAsync(d_offs, e.seg_off_host, off_bytes, cudaMemcpyHostToDevice, st));
   D377_CUDA(cudaEventRecord(e.ev_seg_off, st));
 
   // ---- once per call: canonical scalars, bucket operands (and per-pair decode status) ----
-  uint8_t* okp = fmt == D377_PT_ENCODING ? ws + o_okp : nullptr;
   if (n) {
     if (sc_mont) {
-      launch_fr_from_mont(scalars, n, ws + o_sc, st);
-      scalars = ws + o_sc;
+      launch_fr_from_mont(scalars, n, sc, st);
+      scalars = sc;
     }
-    if (fmt == D377_PT_ENCODING) {
-      k_msm_points_enc_ok<<<grid_for(n, kBlk), kBlk, ISQRT_SMEM_WORDS(kBlk) * 4, st>>>(points, n, (aff4_t*)(ws + o_pts),
-                                                                                        okp);
-      D377_LAUNCHED();
-    } else if (affine) {
-      // Affine inputs never fail to load and normalisation reports nothing: no flags word
-      launch_points_affine(e, fmt, points, n, e.msm_normalize_override > 0 ? 4 : 1, ws + o_norm,
-                           (aff4_t*)(ws + o_pts), nullptr, st);
-    } else {
-      if (fmt == D377_PT_ELEMENT)
-        k_msm_points<D377_PT_ELEMENT><<<grid_for(n, kBlk), kBlk, 0, st>>>(points, n, (cached_t*)(ws + o_pts));
-      else
-        k_msm_points<D377_PT_XYZ><<<grid_for(n, kBlk), kBlk, 0, st>>>(points, n, (cached_t*)(ws + o_pts));
-      D377_LAUNCHED();
-    }
+    // no flags word: affine inputs never fail to load, normalisation reports nothing and
+    // encodings report per pair in okp
+    launch_operands(e, fmt, affine, normalize_min_per(e), points, n, norm, ops, nullptr, okp, st);
   }
 
   // ---- chunk by chunk ----
-  uint32_t* dig = (uint32_t*)(ws + o_dig);
-  uint32_t* sorted = (uint32_t*)(ws + o_sorted);
-  uint32_t* counts = (uint32_t*)(ws + o_counts);
-  uint32_t* cursor = (uint32_t*)(ws + o_cursor);
-  uint32_t* tiles = (uint32_t*)(ws + o_tiles);
-  pt_t* bsum = (pt_t*)(ws + o_bsum);
-  pt_t* part = (pt_t*)(ws + o_part);
-  int32_t* pb = (int32_t*)(ws + o_pb);
-  int32_t* kbuf[2] = {(int32_t*)(ws + o_pb2), (int32_t*)(ws + o_pb3)};
-  pt_t* pbuf[2] = {(pt_t*)(ws + o_part2), (pt_t*)(ws + o_part3)};
   const size_t ob = out_bytes(out_format);
   for (const Chunk& ch : chunks) {
     const size_t p0 = offsets[ch.j0], np = offsets[ch.j0 + ch.J] - p0;
-    const size_t nb = ch.J * WK, nthreads = (np * g.W + L - 1) / L;
-    const size_t ntiles = (nb + 1 + kScanTile - 1) / kScanTile;
+    const size_t nb = ch.J * WK, nthreads = (np * g.W + pl.L - 1) / pl.L;
     const uint32_t* offs = d_offs + ch.j0;
-    D377_CUDA(cudaMemsetAsync(counts, 0, (nb + 1) * 4, st));
+    D377_CUDA(cudaMemsetAsync(w.counts[0], 0, (nb + 1) * 4, st));
     if (np) {
-      k_msm_count_seg<<<grid_for(np, 256), 256, 0, st>>>(scalars + 32 * p0, np, offs, (uint32_t)ch.J, g, counts, dig);
+      k_msm_count_seg<<<grid_for(np, 256), 256, 0, st>>>(scalars + 32 * p0, np, offs, (uint32_t)ch.J, g, w.counts[0],
+                                                         w.dig);
       D377_LAUNCHED();
     }
-    k_scan_tiles<<<(unsigned)ntiles, kScanBlock, 0, st>>>(counts, nb + 1, tiles);
-    D377_LAUNCHED();
-    k_scan_sums<<<1, kScanBlock, 0, st>>>(tiles, ntiles, tiles + ntiles);
-    D377_LAUNCHED();
-    k_scan_apply<<<(unsigned)ntiles, kScanBlock, 0, st>>>(counts, nb + 1, tiles, cursor);
-    D377_LAUNCHED();
+    // stored index: the pair within the chunk, whose bucket operands start at p0
+    launch_sort(st, w.counts[0], w.cursor[0], w.tiles[0], nb, w.dig, np, (uint32_t)g.W, w.sorted, 0u, 0u, 0u);
     if (np) {
-      // stored index: the pair within the chunk, whose bucket operands start at p0
-      k_msm_scatter<<<(unsigned)((size_t)grid_for(np, 256 * kScatterIlp) * g.W), 256, 0, st>>>(
-          dig, np, (uint32_t)g.W, cursor, sorted, 0u, 0u);
-      D377_LAUNCHED();
-      D377_CUDA(cudaMemsetAsync(pb, 0xff, 2 * nthreads * 4, st));
-      const uint8_t* recs = ws + o_pts + 128 * p0;
-      if (affine)
-        k_msm_accumulate<true><<<grid_for(nthreads, kBlk), kBlk, 0, st>>>(recs, sorted, counts, (uint32_t)nb, L, bsum,
-                                                                           part, pb, 0);
-      else
-        k_msm_accumulate<false><<<grid_for(nthreads, kBlk), kBlk, 0, st>>>(recs, sorted, counts, (uint32_t)nb, L, bsum,
-                                                                            part, pb, 0);
-      D377_LAUNCHED();
-      launch_stitch(st, pb, part, nthreads, bsum, kbuf, pbuf);
+      D377_CUDA(cudaMemsetAsync(w.pb, 0xff, 2 * nthreads * 4, st));
+      launch_accumulate(st, affine, ops + 128 * p0, w.sorted, w.counts[0], nb, pl.L, nthreads, w.bsum, 0, w.part, w.pb);
     }
     // bucket reduction: one group of J W virtual windows
     const size_t rows = ch.J * g.W;
-    pt_t *a = (pt_t*)(ws + o_seg_a), *p = (pt_t*)(ws + o_seg_p);
-    pt_t *a2 = (pt_t*)(ws + o_seg_a2), *p2 = (pt_t*)(ws + o_seg_p2);
-    GroupTab gt;
-    gt.ng = 1;
-    gt.wlo[0] = 0;
-    gt.whi[0] = (int)rows;
-    gt.offs[0] = counts;
-    MsmGeom rg = g;
-    rg.W = (int)rows;
-    k_msm_bucket_reduce_ap<<<grid_for(rows * S, kBlk), kBlk, 0, st>>>(bsum, gt, rg, Lseg, log_lseg, S, a, p);
-    D377_LAUNCHED();
-    launch_wsum_tree(st, a, p, a2, p2, S, rows);
-    k_msm_finish_seg<<<grid_for(ch.J * 4, kSegFinishBlk), kSegFinishBlk,
-                       out_format == D377_OUT_ENCODING ? ISQRT_SMEM_WORDS(kSegFinishBlk) * 4 : 0, st>>>(
-        a, (uint32_t)ch.J, g.W, g.c, offs, okp, out_format == D377_OUT_ELEMENT ? out + ob * ch.j0 : nullptr,
+    const GroupTab gt{1, {0}, {(int)rows}, {w.counts[0]}};
+    pt_t* sums = nullptr;
+    rc = launch_tail(st, w, nthreads, gt, g, rows, pl, nullptr, &sums);
+    if (rc) return rc;
+    k_msm_finish<<<grid_for(ch.J * 4, kFinishBlk), kFinishBlk,
+                   out_format == D377_OUT_ENCODING ? ISQRT_SMEM_WORDS(kFinishBlk) * 4 : 0, st>>>(
+        sums, (uint32_t)ch.J, g.W, g.c, offs, okp, out_format == D377_OUT_ELEMENT ? out + ob * ch.j0 : nullptr,
         out_format == D377_OUT_ENCODING ? out + ob * ch.j0 : nullptr, ok ? ok + ch.j0 : nullptr);
     D377_LAUNCHED();
     D377_CUDA(cudaGetLastError());
